@@ -2,7 +2,7 @@
 """bench.py — BASELINE.json's metric: Mpaths/s (and Mrays/s) of the path-tracing sample loop, on N B200s of one box, with
 the reference's CPU renderer beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 5N] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config 5N] [--impl reference] [--dump-outputs DIR]
 
 --config selects one of BASELINE.json's configs at its stated size and samples per pixel (SURVEY.md §8d):
     1       Ch01 motion-blur random scene, flat list as shipped, 200x100 x 100 spp
@@ -20,6 +20,9 @@ reduce (sum) of the float accumulation buffer to rank 0 — strong scaling, the 
 value  = paths per second with the scene resident in HBM (CUDA events around the step on the launching stream).
 e2e    = the same through the host-buffer C-ABI: the scene's device image copied from pinned host memory, render,
          accumulation buffer copied back to pinned host memory, every step.
+--dump-outputs DIR writes what the last timed step computed, DIR/accum.npy: the (ny, nx, 3) float32 per-pixel sums over
+the ns samples (row 0 at the bottom, after the reduce on rank 0).  Scene, camera and seed are fixed, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import hashlib
@@ -209,7 +212,12 @@ def main():
     ap.add_argument("--config", default="5N", choices=sorted(CONFIGS))
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--flags", type=int, default=0, help="extra RTNW_F_* render flags (4 = RTNW_F_FAST_BVH, the non-reference-exact fast traversal mode)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's accumulation buffer to DIR/accum.npy (not with --impl reference)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes this project's render; the reference arm keeps no image")
     if args.impl == "reference":
         return reference_main(args)
 
@@ -284,6 +292,10 @@ def main():
     barrier()
     step_ms = [a.elapsed_time(b) for a, b in ev]
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:  # before the e2e steps, which reuse `accum` when world > 1
+        import numpy as np
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "accum.npy"), accum.cpu().numpy())
     total_ms = torch.tensor([sum(step_ms)], dtype=torch.float64, device=dev)
     tot_rays = torch.tensor([float(rays)], dtype=torch.float64, device=dev)
     if dist is not None:

@@ -3,9 +3,10 @@
 (host/compat/*.h are one-line stand-ins for the reference's header names, host/rtnw/scene.hpp has the classes) and linked
 with librtnw_host.so.  The builders taken from the reference's text are then run and flattened, and the tables must be
 byte-identical to the ones the named scenes of the host library produce, i.e. what the GPU renders is the same.  Needs
-/root/reference (this container only); nothing from it is copied into the repo."""
+a checkout of the reference project named by RTNW_REFERENCE; nothing from it is copied into the repo."""
 import ctypes as C
 import importlib
+import os
 import subprocess
 import sys
 from pathlib import Path
@@ -14,7 +15,7 @@ import pytest
 
 ROOT = Path(__file__).resolve().parent.parent
 PKG = ROOT / "peter-shirley-ray-tracing-the-next-week_b200"
-REF = Path("/root/reference/Peter-Shirley-Project Code")
+REF = Path(os.environ["RTNW_REFERENCE"]) / "Peter-Shirley-Project Code" if os.environ.get("RTNW_REFERENCE") else None
 sys.path.insert(0, str(ROOT))
 rtnw = importlib.import_module("peter-shirley-ray-tracing-the-next-week_b200")
 
@@ -60,7 +61,7 @@ def _tables(d):
     return b"".join(len(p).to_bytes(8, "little") + p for p in parts)
 
 
-@pytest.mark.skipif(not (REF / "main.cpp").exists(), reason="/root/reference is not present on this box")
+@pytest.mark.skipif(REF is None or not (REF / "main.cpp").exists(), reason="RTNW_REFERENCE does not name a checkout of the reference project")
 def test_reference_main_cpp_compiles_unchanged_and_builds_the_same_scenes(tmp_path):
     (tmp_path / "driver.cpp").write_text(DRIVER)
     exe = tmp_path / "driver"

@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 
 import oracle_port as op
-from raysets import FLT_MAX, assert_hits_equal
+from raysets import FLT_MAX, assert_hits_equal, scene_with_material
 
 GOLD = Path(__file__).resolve().parent / "golden"
 TRACE = sorted(p.stem[len("trace_"):] for p in GOLD.glob("trace_*.npz"))
@@ -108,6 +108,44 @@ def test_cuda_reproduces_golden_units(rtnw, ctx):
     got = rtnw.camera_rays(ctx, cam, 200, 100, g["cam_ij"], g["cam_sample"], seed=77)
     for f in ("origin", "direction", "time", "key"):
         assert np.array_equal(got[f], g["cam_rays"][f]), f
+
+
+SCATTER_MATERIALS = ["lambertian", "metal", "dielectric", "light", "isotropic"]
+
+
+def _golden_scatter_scene(rtnw, g, name):
+    """a one-sphere scene whose material 0 is the fixture's row {kind, tex_kind, r, g, b, fuzz_or_ri, scale, 0}"""
+    row = g[f"{name}_row"]
+    return scene_with_material(rtnw, int(row[0]), tuple(float(x) for x in row[2:5]), float(row[5]), float(row[6]))
+
+
+@pytest.mark.parametrize("name", SCATTER_MATERIALS)
+def test_oracle_port_reproduces_golden_scatter(rtnw, name):
+    g = np.load(GOLD / "units.npz")
+    d, keep = _golden_scatter_scene(rtnw, g, name)
+    sc, att, em, flag = op.scatter(rtnw, d, g["sc_rays"], g["sc_hits"], seed=31)
+    for f in ("origin", "direction", "time"):
+        assert np.array_equal(sc[f], g[f"{name}_sc"][f], equal_nan=True), f
+    assert np.array_equal(att, g[f"{name}_att"]) and np.array_equal(em, g[f"{name}_em"]) and np.array_equal(flag, g[f"{name}_flag"])
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("name", SCATTER_MATERIALS)
+def test_cuda_reproduces_golden_scatter(rtnw, ctx, name):
+    """scatter() / emitted() on the GPU against the reference's values on the same stream (units.npz), with the rules of
+    test_gpu_parity.py::test_scatter_and_emitted_same_stream"""
+    g = np.load(GOLD / "units.npz")
+    d, keep = _golden_scatter_scene(rtnw, g, name)
+    ds = ctx.upload(d)
+    sc, att, em, flag = ds.scatter(g["sc_rays"], g["sc_hits"], seed=31)
+    ds.close()
+    assert np.array_equal(flag, g[f"{name}_flag"]) and np.array_equal(em, g[f"{name}_em"]) and np.array_equal(att, g[f"{name}_att"])
+    for f in ("origin", "time"):
+        assert np.array_equal(sc[f], g[f"{name}_sc"][f]), f
+    a, b = sc["direction"], g[f"{name}_sc"]["direction"]
+    same = np.all((a == b) | (np.isnan(a) & np.isnan(b)), axis=1)
+    # dielectric: schlick() goes through pow() in double on the CPU, so a draw within an ulp of reflect_prob may flip
+    assert (~same).sum() <= (1 if name == "dielectric" else 0)
 
 
 def _epilogue_cases():

@@ -8,10 +8,12 @@ reference is driven by the same Philox stream as the GPU (oracle/ref_harness.cpp
 import numpy as np
 import pytest
 
+import oracle_port as op
 import ref_oracle as ro
-from raysets import FLT_MAX, assert_hits_equal, make_rays
+from raysets import FLT_MAX, assert_hits_equal, make_rays, reference_camera_rays, reference_scene, scene_with_material
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not ro.available(), reason="oracle/_ref/libref_oracle.so not built")]
+# the reference side is the compiled reference when it is built, else the C restatement pinned bit-exact to it (raysets.py)
+pytestmark = pytest.mark.gpu
 
 TRACE_SCENES = ["ch01_random", "two_perlin", "cornell_box", "cornell_smoke", "final", "final+bvh", "final_northstar", "earth",
                 "simple_light", "cornell_smoke+bvh", "random_scene", "random_scene+bvh", "test"]
@@ -19,7 +21,7 @@ TRACE_SCENES = ["ch01_random", "two_perlin", "cornell_box", "cornell_smoke", "fi
 
 @pytest.mark.parametrize("name", TRACE_SCENES)
 def test_closest_hit_ids_bit_exact(rtnw, ctx, name):
-    rs, rays = make_rays(name)
+    rs, rays = make_rays(name, rtnw=rtnw)
     want = rs.trace(rays, 0.001, FLT_MAX, seed=11)
     hs = rtnw.HostScene(name)
     ds = ctx.upload(hs.desc_ptr)
@@ -38,7 +40,7 @@ def test_fast_bvh_mode_finds_the_same_closest_hit_with_fewer_tests(rtnw, ctx, na
     bit, and the same leaf except among candidates of EQUAL t (a documented tie: the exact mode lets the later leaf win, the
     fast mode may have culled it) - with fewer primitive tests and fewer tests in total."""
     rng = np.random.default_rng(17)
-    rs, base = make_rays(name, n_primary=3000, seed=5)
+    rs, base = make_rays(name, n_primary=3000, seed=5, rtnw=rtnw)
     reps = -(-1_000_000 // len(base))
     rays = np.tile(base, reps)
     jitter = (1.0 + 1e-3 * rng.standard_normal((len(rays), 3))).astype(np.float32)
@@ -72,7 +74,7 @@ def test_trace_t_range_and_empty_input(rtnw, ctx):
     hs = rtnw.HostScene("cornell_box")
     ds = ctx.upload(hs.desc_ptr)
     assert len(ds.trace(np.zeros(0, dtype=rtnw.RAY_DTYPE))) == 0
-    rs, rays = make_rays("cornell_box", n_primary=500)
+    rs, rays = make_rays("cornell_box", n_primary=500, rtnw=rtnw)
     for t_min, t_max in [(0.0, FLT_MAX), (0.01, 900.0), (100.0, 700.0)]:
         assert_hits_equal(ds.trace(rays, t_min, t_max, seed=2), rs.trace(rays, t_min, t_max, seed=2))
     ds.close()
@@ -81,11 +83,10 @@ def test_trace_t_range_and_empty_input(rtnw, ctx):
 def test_camera_rays_bit_exact(rtnw, ctx):
     rng = np.random.default_rng(1)
     for name, nx, ny in [("ch01_random", 200, 100), ("final", 1000, 1000), ("two_perlin", 400, 200)]:
-        v = ro.view_of(name)
         n = 4000
         ij = np.stack([rng.integers(0, nx, n), rng.integers(0, ny, n)], axis=1)
         s = rng.integers(0, 1000, n)
-        want = ro.camera_rays(v, nx, ny, ij, s, seed=99)
+        want = reference_camera_rays(rtnw, name, nx, ny, ij, s, seed=99)
         cam = rtnw.HostScene(name).camera(nx, ny)
         got = rtnw.camera_rays(ctx, cam, nx, ny, ij, s, seed=99)
         for f in ("origin", "direction", "time", "key"):
@@ -95,21 +96,26 @@ def test_camera_rays_bit_exact(rtnw, ctx):
 def test_perlin_and_textures(rtnw, ctx):
     rng = np.random.default_rng(2)
     hs = rtnw.HostScene("two_perlin")
-    ro.RefScene("two_perlin", tagged=False)  # same perlin tables in the reference's statics
+    live = ro.available()
+    if live:
+        ro.RefScene("two_perlin", tagged=False)  # same perlin tables in the reference's statics
     ds = ctx.upload(hs.desc_ptr)
     xyz = np.concatenate([rng.normal(scale=3, size=(3000, 3)), rng.normal(scale=400, size=(3000, 3)),
                           rng.integers(-5, 5, size=(500, 3)).astype(np.float64)]).astype(np.float32)
     for which in (0, 1):
-        got, want = ds.eval_perlin(which, xyz), ro.eval_perlin(which, xyz)
+        got = ds.eval_perlin(which, xyz)
+        want = ro.eval_perlin(which, xyz) if live else op.eval_perlin(rtnw, hs.desc_ptr, which, xyz)
         assert np.array_equal(got, want), f"perlin which={which}: {np.abs(got - want).max()}"
     uvp = np.concatenate([rng.random((len(xyz), 2)).astype(np.float32), xyz], axis=1)
     # textures of two_perlin: 0 = checker(even 1, odd 2), 3 = noise(4)
     d = hs.desc
     kinds = [d.textures[i].kind for i in range(d.n_textures)]
     checker, noise = kinds.index(1), kinds.index(2)
-    got, want = ds.eval_texture(checker, uvp), ro.eval_texture(1, [0.2, 0.3, 0.1, 0.9, 0.9, 0.9], uvp)
+    got = ds.eval_texture(checker, uvp)
+    want = ro.eval_texture(1, [0.2, 0.3, 0.1, 0.9, 0.9, 0.9], uvp) if live else op.eval_texture(rtnw, hs.desc_ptr, checker, uvp)
     assert (np.all(got == want, axis=1)).mean() > 0.999  # sign of a product of three sinf near zero may flip by an ulp
-    got, want = ds.eval_texture(noise, uvp), ro.eval_texture(2, [4.0], uvp)
+    got = ds.eval_texture(noise, uvp)
+    want = ro.eval_texture(2, [4.0], uvp) if live else op.eval_texture(rtnw, hs.desc_ptr, noise, uvp)
     assert np.allclose(got, want, rtol=0, atol=2e-6), np.abs(got - want).max()
     ds.close()
     hs = rtnw.HostScene("earth")
@@ -117,38 +123,8 @@ def test_perlin_and_textures(rtnw, ctx):
     d = hs.desc
     img = [d.textures[i].kind for i in range(d.n_textures)].index(3)
     uvp[:50, :2] = np.array([[0, 0], [1, 1], [0, 1], [1, 0], [0.5, 0.5]] * 10, dtype=np.float32)
-    assert np.array_equal(ds.eval_texture(img, uvp), ro.eval_texture(3, [], uvp))
+    assert np.array_equal(ds.eval_texture(img, uvp), ro.eval_texture(3, [], uvp) if live else op.eval_texture(rtnw, hs.desc_ptr, img, uvp))
     ds.close()
-
-
-def _scene_with_material(rtnw, kind, rgb, f, scale=0.0):
-    """a one-sphere scene_desc whose material 0 is the requested one (tables built by hand through the C structs)"""
-    import ctypes as C
-    hs = rtnw.HostScene("two_perlin")  # borrow perlin tables / xform identity
-    d = rtnw.SceneDesc()
-    C.memmove(C.byref(d), C.byref(hs.desc), C.sizeof(d))
-    tex = (rtnw.Texture * 1)()
-    tex[0].kind = 2 if scale else 0
-    tex[0].c[0], tex[0].c[1], tex[0].c[2] = (scale, 0, 0) if scale else rgb
-    mat = (rtnw.Material * 1)()
-    mat[0].kind = kind
-    mat[0].tex = 0
-    mat[0].f = f
-    mat[0].albedo[0], mat[0].albedo[1], mat[0].albedo[2] = rgb
-    prim = (rtnw.Prim * 1)()
-    prim[0].f[3] = 1.0
-    prim[0].kx = 0
-    prim[0].mat = 0
-    ids = (C.c_int32 * 1)(0)
-    item = (rtnw.Item * 1)()
-    item[0].kind, item[0].first, item[0].count = 0, 0, 1
-    d.n_items, d.items = 1, item
-    d.n_nodes = 0
-    d.n_prim_slots, d.prims, d.prim_ids = 1, prim, ids
-    d.n_materials, d.materials = 1, mat
-    d.n_textures, d.textures = 1, tex
-    keep = (hs, tex, mat, prim, ids, item)
-    return d, keep
 
 
 @pytest.mark.parametrize("kind,rgb,f,scale", [(0, (0.4, 0.2, 0.1), 0, 0), (0, (0, 0, 0), 0, 4.0), (1, (0.8, 0.8, 0.9), 0.3, 0),
@@ -157,8 +133,10 @@ def _scene_with_material(rtnw, kind, rgb, f, scale=0.0):
 def test_scatter_and_emitted_same_stream(rtnw, ctx, kind, rgb, f, scale):
     rng = np.random.default_rng(kind * 10 + int(f * 10))
     n = 4000
-    d, keep = _scene_with_material(rtnw, kind, rgb, f, scale)
-    ro.RefScene("two_perlin", tagged=False)
+    d, keep = scene_with_material(rtnw, kind, rgb, f, scale)
+    live = ro.available()
+    if live:
+        ro.RefScene("two_perlin", tagged=False)
     ds = ctx.upload(d)
     rays = np.zeros(n, dtype=rtnw.RAY_DTYPE)
     rays["origin"] = rng.normal(size=(n, 3))
@@ -171,7 +149,7 @@ def test_scatter_and_emitted_same_stream(rtnw, ctx, kind, rgb, f, scale):
     hits["t"] = 1.0
     hits["u"], hits["v"] = rng.random(n), rng.random(n)
     mat = np.tile(np.array([kind, 2 if scale else 0, rgb[0], rgb[1], rgb[2], f, scale, 0], dtype=np.float32), (n, 1))
-    w_sc, w_att, w_em, w_flag = ro.scatter(mat, rays, hits, seed=5)
+    w_sc, w_att, w_em, w_flag = ro.scatter(mat, rays, hits, seed=5) if live else op.scatter(rtnw, d, rays, hits, seed=5)
     g_sc, g_att, g_em, g_flag = ds.scatter(rays, hits, seed=5)
     assert np.array_equal(g_flag, w_flag)
     assert np.array_equal(g_em, w_em)
@@ -214,7 +192,7 @@ def test_render_matches_reference_sample_for_sample(rtnw, ctx, name, nx, ny, ns)
     cam = hs.camera(nx, ny)
     p = hs.params(nx=nx, ny=ny, ns=ns, seed=1234)
     got, st = ds.render(cam, p)
-    rs = ro.RefScene(name, tagged=True)
+    rs = reference_scene(rtnw, name)
     want, rst = rs.render(nx, ny, ns, seed=1234, rng_mode=1)
     assert st.paths == nx * ny * ns
     close = np.isclose(got, want, rtol=2e-5, atol=1e-6).all(axis=2)

@@ -1,7 +1,8 @@
 """Texture ingest (SURVEY §8f.3): rtnw_host_load_png replaces the reference's stbi_load("picture.png") (PSC/main.cpp:93).
 The decoder is checked against PNG files written here with zlib (every colour type, every row filter), against the
-reference's own picture.png when /root/reference is mounted, and through the "earth@<file>" scene builder."""
+reference's own picture.png when RTNW_REFERENCE names a checkout of the reference project, and through the "earth@<file>" scene builder."""
 import importlib
+import os
 import struct
 import sys
 import zlib
@@ -108,10 +109,11 @@ def test_earth_scene_takes_its_texture_from_the_file(tmp_path):
     assert np.array_equal(pool[tex[0].i0:tex[0].i0 + 32 * 16 * 3].reshape(16, 32, 3), img[:, :, :3])
 
 
-REF_PNG = Path("/root/reference/Peter-Shirley-Project Code/cmake-build-debug/picture.png")
+REF_PNG = (Path(os.environ["RTNW_REFERENCE"]) / "Peter-Shirley-Project Code" / "cmake-build-debug" / "picture.png"
+           if os.environ.get("RTNW_REFERENCE") else None)
 
 
-@pytest.mark.skipif(not REF_PNG.exists(), reason="reference tree not mounted")
+@pytest.mark.skipif(REF_PNG is None or not REF_PNG.exists(), reason="RTNW_REFERENCE does not name a checkout of the reference project")
 def test_reference_picture_png_decodes():
     """the file PSC/main.cpp:93 loads: decodes, has the IHDR size, and is an actual picture (not constant)"""
     w, h = struct.unpack(">II", REF_PNG.read_bytes()[16:24])
