@@ -299,6 +299,29 @@ int rtnw_quantize_device(rtnw_ctx* ctx, const float* accum_rgb_dev, int32_t nx, 
 int rtnw_trace(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_ray* rays, size_t n, float t_min, float t_max,
                uint32_t flags, uint64_t seed, rtnw_hit* out);
 
+/* First-hit feature buffers (AOVs) of a frame: the per-pixel inputs a denoiser takes next to the noisy colour, plus depth
+ * for compositing and a leaf id for picking.  For pixel p = j*nx + i and sample s = sample_begin + k*sample_stride,
+ * k < sample_count, the AOV ray is exactly the first ray rtnw_render traces for (p, s) with the same camera and seed: the
+ * path stream (seed, p, s), camera::get_ray with the pixel jitter, and one closest hit over [t_min, t_max] whose media draw
+ * with the key (p, s, depth 0).  So the first hit of every AOV sample is the first vertex of that render path.
+ * Per sample, in sample order k = 0, 1, ... (plain float additions, no atomics: the buffers are bit-reproducible):
+ *   albedo  (nx*ny*3 sums)  hit: the attenuation scatter() returns — lambertian / isotropic texture value, metal albedo,
+ *                           dielectric (1,1,1) — or, for diffuse_light, its emitted texture value clamped to 1 per channel;
+ *                           miss: the sky colour with RTNW_BG_SKY, 0 with a black background
+ *   normal  (nx*ny*3 sums)  hit: the hit_record normal (after the transform chain and flip_normals; (1,0,0) in a medium)
+ *   depth   (nx*ny sums)    hit: t * sqrtf(d.x*d.x + d.y*d.y + d.z*d.z) of the camera ray direction d (distance from its origin)
+ *   hits    (nx*ny int32)   number of samples that hit
+ *   prim_id (nx*ny int32)   leaf id of the hit of the call's first sample (k = 0), -1 if it missed
+ * These are sums like rtnw_render's: divide albedo by sample_count, normal and depth by hits.  Index order is rtnw_render's
+ * ((j*nx + i)*3 + c, j = 0 the bottom row).  Honours nx, ny, sample_begin/count/stride, t_min, t_max, background, seed
+ * and RTNW_F_FAST_BVH; accepts and ignores the other flags, max_depth and sample_ranges; rejects a pixel subset,
+ * RTNW_F_ACCUMULATE and RTNW_F_ROTATE_SAMPLES (RTNW_ERR_INVALID).  Host buffers; stats: paths = rays = nx*ny*sample_count. */
+typedef struct rtnw_aov {        /* host buffers, all required */
+    float* albedo; float* normal; float* depth; int32_t* hits; int32_t* prim_id;
+} rtnw_aov;
+int rtnw_render_aov(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam,
+                    const rtnw_render_params* params, const rtnw_aov* out, rtnw_stats* stats);
+
 /* texture::value(u,v,p) for n points; uvp = n x 5 floats {u,v,px,py,pz}; rgb_out = n x 3 (PSC/texture.h, surface_texture.h) */
 int rtnw_eval_texture(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t tex_id, const float* uvp, size_t n, float* rgb_out);
 /* perlin::noise (which=0) / perlin::turb depth 7 (which=1) at n points xyz (PSC/perlin.h:43-74) */

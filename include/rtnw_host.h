@@ -58,6 +58,11 @@ int rtnw_host_make_camera(const float lookfrom[3], const float lookat[3], const 
 int rtnw_host_quantize(const float* accum_sums, int32_t nx, int32_t ny, int32_t ns, int32_t clamp255, int32_t* rgb_out);
 /* PSC/main.cpp:295-334: ASCII P3 writer (binary P6 when binary != 0) */
 int rtnw_host_write_ppm(const char* path, const float* accum_sums, int32_t nx, int32_t ny, int32_t ns, int32_t clamp255, int32_t binary);
+/* Portable Float Map of an nx x ny image of `channels` floats per pixel (3: "PF" colour, 1: "Pf" greyscale; other counts are
+ * RTNW_ERR_INVALID): header "PF\n<nx> <ny>\n-1.0\n" (scale -1: little-endian), then the floats row by row in buffer order.
+ * PFM stores the bottom row first, which is row j = 0 of the library's buffers, so an rtnw_render / rtnw_render_aov buffer
+ * (after dividing the sums) is written as it is. */
+int rtnw_host_write_pfm(const char* path, const float* values, int32_t nx, int32_t ny, int32_t channels);
 
 #ifdef __cplusplus
 }

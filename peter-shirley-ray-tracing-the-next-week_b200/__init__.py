@@ -99,6 +99,11 @@ class Stats(C.Structure):
                 ("kernel_ms", C.c_float), ("total_ms", C.c_float), ("kernel_launches", C.c_int32), ("sample_ranges", C.c_int32)]
 
 
+class Aov(C.Structure):
+    """rtnw_aov: the host buffers rtnw_render_aov fills"""
+    _fields_ = [("albedo", C.c_void_p), ("normal", C.c_void_p), ("depth", C.c_void_p), ("hits", C.c_void_p), ("prim_id", C.c_void_p)]
+
+
 class HostView(C.Structure):
     _fields_ = [("nx", C.c_int32), ("ny", C.c_int32), ("ns", C.c_int32), ("t_min", C.c_float),
                 ("background", C.c_uint32), ("flags", C.c_uint32)]
@@ -116,10 +121,10 @@ DEVICE_SYMBOLS = ["rtnw_last_error", "rtnw_abi_version", "rtnw_device_count", "r
                   "rtnw_eval_texture", "rtnw_eval_perlin", "rtnw_scatter", "rtnw_camera_rays", "rtnw_camera_get_rays", "rtnw_plan_sample_ranges",
                   "rtnw_scene_inspect", "rtnw_ctx_create_multi", "rtnw_ctx_destroy_multi", "rtnw_multi_device_count",
                   "rtnw_scene_upload_multi", "rtnw_scene_free_multi", "rtnw_render_multi", "rtnw_scene_prepare", "rtnw_prepared_bytes",
-                  "rtnw_scene_upload_prepared", "rtnw_prepared_free"]
+                  "rtnw_scene_upload_prepared", "rtnw_prepared_free", "rtnw_render_aov"]
 HOST_SYMBOLS = ["rtnw_host_last_error", "rtnw_host_scene_build", "rtnw_host_scene_free", "rtnw_host_scene_desc",
                 "rtnw_host_scene_leaf_count", "rtnw_host_scene_camera", "rtnw_host_scene_view", "rtnw_host_make_camera",
-                "rtnw_host_quantize", "rtnw_host_write_ppm", "rtnw_host_load_png", "rtnw_host_free_image"]
+                "rtnw_host_quantize", "rtnw_host_write_ppm", "rtnw_host_load_png", "rtnw_host_free_image", "rtnw_host_write_pfm"]
 
 
 def build_native(device: bool = True, host: bool = True) -> None:
@@ -152,6 +157,7 @@ def host_lib() -> C.CDLL:
                                             C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.POINTER(Camera)]
         L.rtnw_host_quantize.argtypes = [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p]
         L.rtnw_host_write_ppm.argtypes = [C.c_char_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32]
+        L.rtnw_host_write_pfm.argtypes = [C.c_char_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32]
         L.rtnw_host_load_png.argtypes = [C.c_char_p, C.POINTER(C.POINTER(C.c_ubyte)), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]
         L.rtnw_host_free_image.argtypes = [C.POINTER(C.c_ubyte)]
         L.rtnw_host_free_image.restype = None
@@ -185,6 +191,8 @@ def device_lib() -> C.CDLL:
                                          C.c_void_p, C.POINTER(Stats)]
         L.rtnw_trace.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_float, C.c_float, C.c_uint32, C.c_uint64,
                                  C.c_void_p]
+        L.rtnw_render_aov.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams), C.POINTER(Aov),
+                                      C.POINTER(Stats)]
         L.rtnw_eval_texture.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]
         L.rtnw_eval_perlin.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]
         L.rtnw_scatter.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p,
@@ -291,6 +299,14 @@ def write_ppm(path: str, sums: np.ndarray, ns: int, clamp255: bool = True, binar
     ny, nx, _ = sums.shape
     sums = np.ascontiguousarray(sums, dtype=np.float32)
     _check_host(host_lib().rtnw_host_write_ppm(str(path).encode(), sums.ctypes.data, nx, ny, ns, int(clamp255), int(binary)))
+
+
+def write_pfm(path, array: np.ndarray) -> None:
+    """Write a float image as a Portable Float Map: (ny, nx, 3) as colour "PF", (ny, nx) as greyscale "Pf"; row 0 of the
+    array (the library's bottom row, j = 0) is the first row of the file, as PFM wants."""
+    a = np.ascontiguousarray(array, dtype=np.float32)
+    channels = a.shape[2] if a.ndim == 3 else 1
+    _check_host(host_lib().rtnw_host_write_pfm(str(path).encode(), a.ctypes.data, a.shape[1], a.shape[0], channels))
 
 
 def device_tables(desc_ptr) -> dict:
@@ -424,6 +440,19 @@ class DeviceScene:
         _check_dev(device_lib().rtnw_render_device(self.ctx._h, self._h, C.byref(cam), C.byref(params), C.c_void_p(dev_ptr),
                                                    C.c_void_p(stream), C.byref(st)))
         return st
+
+    def render_aov(self, cam: Camera, params: RenderParams, stats: Stats | None = None) -> dict:
+        """First-hit feature buffers of the frame rtnw_render draws for the same camera and params (include/rtnw.h:
+        rtnw_render_aov): dict of per-pixel SUMS albedo (ny,nx,3), normal (ny,nx,3), depth (ny,nx), and int32 hits (ny,nx) and
+        prim_id (ny,nx), row j = 0 at the bottom.  Divide albedo by sample_count, normal and depth by hits.  Pass a Stats to
+        receive the call's statistics."""
+        ny, nx = params.ny, params.nx
+        out = dict(albedo=np.empty((ny, nx, 3), np.float32), normal=np.empty((ny, nx, 3), np.float32),
+                   depth=np.empty((ny, nx), np.float32), hits=np.empty((ny, nx), np.int32), prim_id=np.empty((ny, nx), np.int32))
+        bufs = Aov(*(out[k].ctypes.data for k in ("albedo", "normal", "depth", "hits", "prim_id")))
+        st = Stats() if stats is None else stats
+        _check_dev(device_lib().rtnw_render_aov(self.ctx._h, self._h, C.byref(cam), C.byref(params), C.byref(bufs), C.byref(st)))
+        return out
 
     # -- one world->hit() per ray, PSC/main.cpp:27
     def trace(self, rays: np.ndarray, t_min: float = 0.001, t_max: float = FLT_MAX, flags: int = 0, seed: int = 1) -> np.ndarray:

@@ -375,6 +375,121 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_trace(const scene_view S, const 
     out[q] = o;
 }
 
+struct aov_args {
+    scene_view S;
+    rtnw_camera cam;
+    rtnw_render_params p;
+    float* albedo;                // nx*ny*3 sums
+    float* normal;                // nx*ny*3 sums
+    float* depth;                 // nx*ny sums
+    int32_t* hits;                // nx*ny counts
+    int32_t* prim_id;             // nx*ny leaf ids of sample k = 0
+    unsigned long long* ctr;      // [4] task stack overflows
+};
+
+// First-hit feature buffers (rtnw_render_aov): one thread per pixel traces, for each of its samples, exactly the first ray
+// k_render traces for that (pixel, sample) — same stream, same camera_ray, same medium key at depth 0 — and sums what the
+// hit shows.  Every pixel has sample_count samples, so every thread of the block runs the same number of cooperative rounds.
+// The running sums of a pixel live in shared memory, as k_render's work items do: in registers they would be live across
+// the media's Philox call inside the traversal, and spill.
+template <bool FAST> struct aov_smem {
+    block_smem<FAST> coop;
+    float4 acc[RTNW_BLOCK];    // albedo xyz, depth
+    float4 nrm[RTNW_BLOCK];    // normal xyz, w = hits (int bits)
+};
+
+// the first ray of the path (pix, s), as k_render starts it.  Not inlined: inside the sample loop the compiler would hoist the
+// pixel's coordinates and the shutter interval out of it, and those values, live across the traversal, would spill.
+__device__ __noinline__ ray_t aov_camera_ray(const rtnw_camera& cam, int nx, int ny, int pix, int s, uint64_t seed) {
+    rng_t g;
+    g.begin((uint32_t)seed, (uint32_t)(seed >> 32), (uint32_t)pix, (uint32_t)s);
+    ray_t r;
+    camera_ray(cam, nx, ny, pix % nx, pix / nx, g, r);
+    return r;
+}
+
+template <bool FAST>
+__global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_args P) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    typedef typename smem_of<FAST>::type SM;
+    aov_smem<FAST>& A = *reinterpret_cast<aov_smem<FAST>*>(smem_raw);
+    SM& sm = A.coop.g[threadIdx.x / RTNW_GROUP];
+    const int me = threadIdx.x;
+    const int nx = P.p.nx, ny = P.p.ny;
+    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+    const bool active = pix < nx * ny;  // idle threads of the last block still work on the block's BVH tasks (with a ray below the image)
+    const uint32_t k0 = (uint32_t)P.p.seed, k1 = (uint32_t)(P.p.seed >> 32);
+    trav_counters cnt;
+    cnt.box_tests = 0; cnt.prim_tests = 0;
+    coop_init<RTNW_GROUP, SM>(sm);
+    A.acc[me] = make_float4(0.f, 0.f, 0.f, 0.f);
+    A.nrm[me] = make_float4(0.f, 0.f, 0.f, __int_as_float(0));
+    group_sync<RTNW_GROUP>();
+#if RTNW_SMEM_NODES
+    stage_top_nodes<RTNW_GROUP, FAST, SM>(P.S, sm);
+#endif
+    int r3 = 0;
+    for (int k = 0; k < P.p.sample_count; ++k) {
+        const int s = P.p.sample_begin + k * P.p.sample_stride;
+        const ray_t r = aov_camera_ray(P.cam, nx, ny, pix, s, P.p.seed);
+        medium_key mk;
+        mk.k0 = k0; mk.k1 = k1; mk.pixel = (uint32_t)pix; mk.sample = (uint32_t)s; mk.depth = 0;
+        const hkey_t key = coop_closest_hit<RTNW_GROUP, false, FAST, SM>(P.S, sm, r, active, P.p.t_min, P.p.t_max, mk, cnt, r3);
+        if (!active) continue;
+        hit_t h;
+        key_to_hit(P.S, key, P.p.t_max, h);
+        if (h.rec < 0) {
+            if (k == 0) P.prim_id[pix] = -1;
+            if (P.p.background == RTNW_BG_SKY) {
+                const f3 c = sky_color(r.d);
+                float4 acc = A.acc[me];
+                acc.x += c.x; acc.y += c.y; acc.z += c.z;
+                A.acc[me] = acc;
+            }
+            continue;
+        }
+        if (k == 0) P.prim_id[pix] = __ldg(&P.S.rec_leaf[h.rec]);
+        // u,v only when the hit material's texture reads them: the rule of k_render
+        const int mat_id = __float_as_int(__ldg(&P.S.recs[h.rec].b).w);
+        const float4 m0 = __ldg(reinterpret_cast<const float4*>(P.S.materials + mat_id));
+        const uint32_t mkind = __float_as_uint(m0.x);
+        bool want_uv = false;
+        if (__float_as_int(m0.y) >= 0 && mkind != RTNW_MAT_METAL && mkind != RTNW_MAT_DIELECTRIC) {
+            const uint32_t tk = __float_as_uint(__ldg(reinterpret_cast<const float4*>(P.S.textures + __float_as_int(m0.y))).x);
+            want_uv = tk == RTNW_TEX_IMAGE || tk == RTNW_TEX_CHECKER;
+        }
+        surf_t sf;
+        finish_hit<FAST && RTNW_FAST_APPROX>(P.S, r, h, sf, want_uv);
+        f3 a;  // the attenuation scatter() returns; a light's emission clamped to 1
+        if (mkind == RTNW_MAT_METAL) {
+            const float4 m1 = __ldg(reinterpret_cast<const float4*>(P.S.materials + mat_id) + 1);
+            a = mk3(m1.x, m1.y, m1.z);
+        } else if (mkind == RTNW_MAT_DIELECTRIC) {
+            a = mk3(1.f, 1.f, 1.f);
+        } else {
+            a = texture_value(P.S, __float_as_int(m0.y), sf.u, sf.v, sf.p);
+            if (mkind == RTNW_MAT_DIFFUSE_LIGHT) a = mk3(fminf(a.x, 1.f), fminf(a.y, 1.f), fminf(a.z, 1.f));
+        }
+        float4 acc = A.acc[me];
+        acc.x += a.x; acc.y += a.y; acc.z += a.z;
+        acc.w += h.t * length(r.d);
+        A.acc[me] = acc;
+        float4 nrm = A.nrm[me];
+        nrm.x += sf.n.x; nrm.y += sf.n.y; nrm.z += sf.n.z;
+        nrm.w = __int_as_float(__float_as_int(nrm.w) + 1);
+        A.nrm[me] = nrm;
+    }
+    group_sync<RTNW_GROUP>();
+    if (threadIdx.x % RTNW_GROUP == 0 && sm.overflow) atomicAdd(&P.ctr[4], 1ull);
+    if (!active) return;
+    const size_t q = (size_t)pix;
+    const float4 acc = A.acc[me], nrm = A.nrm[me];
+    P.albedo[3 * q] = acc.x; P.albedo[3 * q + 1] = acc.y; P.albedo[3 * q + 2] = acc.z;
+    P.normal[3 * q] = nrm.x; P.normal[3 * q + 1] = nrm.y; P.normal[3 * q + 2] = nrm.z;
+    P.depth[q] = acc.w;
+    P.hits[q] = __float_as_int(nrm.w);
+}
+
 // the epilogue of the sample loop, PSC/main.cpp:315-325, one thread per pixel; output row 0 = top row (j = ny-1)
 __global__ void k_quantize(const float* __restrict__ sums, int nx, int ny, float inv_ns, int clamp255, int32_t* __restrict__ out) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1621,6 +1736,61 @@ int rtnw_trace(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_ray* rays, siz
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(out, d_out.p, n * sizeof(rtnw_hit), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return RTNW_OK;
+}
+
+int rtnw_render_aov(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam, const rtnw_render_params* params,
+                    const rtnw_aov* out, rtnw_stats* stats) {
+    int rc = check_ctx(ctx);
+    if (rc != RTNW_OK) return rc;
+    if (!scene || !cam || !out || !out->albedo || !out->normal || !out->depth || !out->hits || !out->prim_id)
+        return fail(RTNW_ERR_INVALID, "null argument");
+    if ((rc = validate_params(params)) != RTNW_OK) return rc;
+    if (params->pixel_count != 0 || (params->flags & (RTNW_F_ACCUMULATE | RTNW_F_ROTATE_SAMPLES)))
+        return fail(RTNW_ERR_INVALID, "rtnw_render_aov covers whole images: no pixel subset, RTNW_F_ACCUMULATE or RTNW_F_ROTATE_SAMPLES");
+    const size_t n = (size_t)params->nx * params->ny;
+    dev_buf d;  // albedo | normal | depth | hits | prim_id
+    CUDA_TRY(d.alloc(n * 9 * sizeof(float)));
+    aov_args a;
+    a.S = scene->view;
+    a.cam = *cam;
+    a.p = *params;
+    a.albedo = d.as<float>();
+    a.normal = a.albedo + 3 * n;
+    a.depth = a.normal + 3 * n;
+    a.hits = reinterpret_cast<int32_t*>(a.depth + n);
+    a.prim_id = a.hits + n;
+    a.ctr = ctx->ctr;
+    const unsigned grid = (unsigned)((n + RTNW_BLOCK - 1) / RTNW_BLOCK);
+    CUDA_TRY(cudaEventRecord(ctx->ev_t0, ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(ctx->ctr, 0, 8 * sizeof(unsigned long long), ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
+    if (params->flags & RTNW_F_FAST_BVH) {
+        CUDA_TRY(cudaFuncSetAttribute(k_aov<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(aov_smem<true>)));
+        k_aov<true><<<grid, RTNW_BLOCK, sizeof(aov_smem<true>), ctx->stream>>>(a);
+    } else {
+        CUDA_TRY(cudaFuncSetAttribute(k_aov<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(aov_smem<false>)));
+        k_aov<false><<<grid, RTNW_BLOCK, sizeof(aov_smem<false>), ctx->stream>>>(a);
+    }
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(ctx->ctr_host, ctx->ctr, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out->albedo, a.albedo, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out->normal, a.normal, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out->depth, a.depth, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out->hits, a.hits, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(out->prim_id, a.prim_id, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev_t1, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    if (ctx->ctr_host[4]) return fail(RTNW_ERR_UNSUPPORTED, "BVH task stack overflow: the tree is deeper than RTNW_QN/RTNW_BLOCK - 1 levels");
+    if (stats) {
+        std::memset(stats, 0, sizeof *stats);
+        stats->paths = stats->rays = (uint64_t)n * params->sample_count;
+        CUDA_TRY(cudaEventElapsedTime(&stats->kernel_ms, ctx->ev0, ctx->ev1));
+        CUDA_TRY(cudaEventElapsedTime(&stats->total_ms, ctx->ev_t0, ctx->ev_t1));
+        stats->kernel_launches = 1;
+        stats->sample_ranges = 1;
+    }
     return RTNW_OK;
 }
 

@@ -5,6 +5,7 @@
 #include <cstdio>
 #include <cstring>
 #include <string>
+#include <vector>
 
 #include "rtnw/flatten.hpp"
 #include "scenes/chapter_scenes.hpp"
@@ -197,6 +198,24 @@ int rtnw_host_write_ppm(const char* path, const float* sums, int32_t nx, int32_t
         }
     }
     std::fclose(f);
+    return RTNW_OK;
+}
+
+int rtnw_host_write_pfm(const char* path, const float* values, int32_t nx, int32_t ny, int32_t channels) {
+    if (!path || !values || nx <= 0 || ny <= 0) return fail(RTNW_ERR_INVALID, "bad pfm arguments");
+    if (channels != 1 && channels != 3) return fail(RTNW_ERR_INVALID, "a PFM holds 1 or 3 channels");
+    FILE* f = std::fopen(path, "wb");
+    if (!f) return fail(RTNW_ERR_INVALID, std::string("cannot open ") + path);
+    std::fprintf(f, "%s\n%d %d\n-1.0\n", channels == 3 ? "PF" : "Pf", nx, ny);
+    const size_t n = (size_t)nx * ny * channels;
+    std::vector<unsigned char> bytes(4 * n);
+    for (size_t i = 0; i < n; ++i) {  // little-endian whatever the host's byte order
+        uint32_t u;
+        std::memcpy(&u, values + i, 4);
+        for (int b = 0; b < 4; ++b) bytes[4 * i + b] = (unsigned char)(u >> (8 * b));
+    }
+    const bool ok = std::fwrite(bytes.data(), 1, bytes.size(), f) == bytes.size();
+    if (std::fclose(f) != 0 || !ok) return fail(RTNW_ERR_INVALID, std::string("cannot write ") + path);
     return RTNW_OK;
 }
 
