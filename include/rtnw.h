@@ -322,6 +322,39 @@ typedef struct rtnw_aov {        /* host buffers, all required */
 int rtnw_render_aov(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam,
                     const rtnw_render_params* params, const rtnw_aov* out, rtnw_stats* stats);
 
+/* Feature-guided denoiser of a frame: spatial-only SVGF (Schied et al. 2017 without the temporal part), i.e. the edge-avoiding
+ * a-trous wavelet filter of Dammertz et al. 2010 with a variance-guided luminance weight, on the GPU.  Inputs are the colour
+ * sums of rtnw_render and the rtnw_aov sums of rtnw_render_aov for the same params (ns = their sample_count); prim_id is not
+ * read and may be NULL.  rgb_out receives the denoised MEAN colour (nx*ny*3, not sums).  All buffers are host buffers in the
+ * library's index order ((j*nx + i)*3 + c, j = 0 the bottom row).  Every step is float32 in a fixed order: the result is
+ * bit-reproducible and equals its C restatement (tests/denoise_oracle.c).
+ *   inputs   c = colour/ns, a = albedo/ns; a pixel is a hit pixel when hits > 0, and then n = normal/hits normalised (0 if its
+ *            length is 0) and z = depth/hits.  Demodulation: a' = max(a, 1e-3) per channel, irradiance e = c / a',
+ *            luminance l = 0.2126 e.r + 0.7152 e.g + 0.0722 e.b.  (A sky miss pixel has c ~ a, e ~ 1; a black miss stays 0.)
+ *   gradient (|dz/dx|, |dz/dy|) by central differences over hit neighbours, one-sided next to a miss or the border, else 0.
+ *   weight   of tap q at offset (dx, dy) from p: 0 if exactly one of p, q is a hit pixel, else
+ *            h(dx) h(dy) w_n exp(-(d_z + d_l)) with h the B3 spline [1/16 1/4 3/8 1/4 1/16] on the pass's step,
+ *            w_n = max(0, n_p.n_q)^(2^normal_power_log2), d_z = |z_p - z_q| / (sigma_depth (|dz/dx|_p |dx| + |dz/dy|_p |dy|)
+ *            + 1e-3 z_p), d_l = |l_p - l_q| / (sigma_luminance sqrt(g(var)_p) + 1e-4); for two miss pixels w_n = 1, d_z = 0.
+ *            g is the 3x3 binomial blur of the variance over the taps p may mix with (same hit class, weights x w_n for hits).
+ *            The centre tap weighs exactly h(0)^2.  Taps outside the image are skipped; taps are summed row by row, then
+ *            left to right.  exp(-x) is the library's own: range reduction to 2^-f, f in [0, 1), a degree-6 polynomial, and
+ *            the exponent bits; within 1e-5 relative of exp, exactly 1 at 0 and 0 from 88 up.
+ *   variance of l before the first pass: over 7x7 with weights w_n exp(-d_z) (1 at the centre), max(mu2 - mu1^2, 0).
+ *   passes   i = 0 .. iterations-1 with step 2^i: e' = sum w e_q / sum w, var' = sum w^2 var_q / (sum w)^2; then out = e' a'.
+ * Rejects (RTNW_ERR_INVALID, the context stays usable) a null colour, albedo, normal, depth or hits buffer or params, nx, ny or
+ * ns <= 0, parameters outside their ranges, and a sigma that is not finite and > 0.  stats: kernel_ms = the denoise kernels,
+ * total_ms = with the copies, kernel_launches = iterations + 2; the other fields 0.  Device memory: 101 bytes per pixel. */
+typedef struct rtnw_denoise_params {
+    int32_t iterations;         /* a-trous passes, step 2^i; 1..8 (5) */
+    float sigma_luminance;      /* (4) */
+    float sigma_depth;          /* (1) */
+    int32_t normal_power_log2;  /* w_n = max(0, n_p.n_q)^(2^k); 0..10 (7 = 128) */
+} rtnw_denoise_params;
+#define RTNW_DENOISE_DEFAULTS {5, 4.0f, 1.0f, 7}
+int rtnw_denoise(rtnw_ctx* ctx, const float* color_sums, const rtnw_aov* features, int32_t nx, int32_t ny, int32_t ns,
+                 const rtnw_denoise_params* dp, float* rgb_out, rtnw_stats* stats);
+
 /* texture::value(u,v,p) for n points; uvp = n x 5 floats {u,v,px,py,pz}; rgb_out = n x 3 (PSC/texture.h, surface_texture.h) */
 int rtnw_eval_texture(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t tex_id, const float* uvp, size_t n, float* rgb_out);
 /* perlin::noise (which=0) / perlin::turb depth 7 (which=1) at n points xyz (PSC/perlin.h:43-74) */

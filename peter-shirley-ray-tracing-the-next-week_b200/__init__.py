@@ -104,6 +104,12 @@ class Aov(C.Structure):
     _fields_ = [("albedo", C.c_void_p), ("normal", C.c_void_p), ("depth", C.c_void_p), ("hits", C.c_void_p), ("prim_id", C.c_void_p)]
 
 
+class DenoiseParams(C.Structure):
+    """rtnw_denoise_params; the defaults are RTNW_DENOISE_DEFAULTS"""
+    _fields_ = [("iterations", C.c_int32), ("sigma_luminance", C.c_float), ("sigma_depth", C.c_float),
+                ("normal_power_log2", C.c_int32)]
+
+
 class HostView(C.Structure):
     _fields_ = [("nx", C.c_int32), ("ny", C.c_int32), ("ns", C.c_int32), ("t_min", C.c_float),
                 ("background", C.c_uint32), ("flags", C.c_uint32)]
@@ -121,7 +127,7 @@ DEVICE_SYMBOLS = ["rtnw_last_error", "rtnw_abi_version", "rtnw_device_count", "r
                   "rtnw_eval_texture", "rtnw_eval_perlin", "rtnw_scatter", "rtnw_camera_rays", "rtnw_camera_get_rays", "rtnw_plan_sample_ranges",
                   "rtnw_scene_inspect", "rtnw_ctx_create_multi", "rtnw_ctx_destroy_multi", "rtnw_multi_device_count",
                   "rtnw_scene_upload_multi", "rtnw_scene_free_multi", "rtnw_render_multi", "rtnw_scene_prepare", "rtnw_prepared_bytes",
-                  "rtnw_scene_upload_prepared", "rtnw_prepared_free", "rtnw_render_aov"]
+                  "rtnw_scene_upload_prepared", "rtnw_prepared_free", "rtnw_render_aov", "rtnw_denoise"]
 HOST_SYMBOLS = ["rtnw_host_last_error", "rtnw_host_scene_build", "rtnw_host_scene_free", "rtnw_host_scene_desc",
                 "rtnw_host_scene_leaf_count", "rtnw_host_scene_camera", "rtnw_host_scene_view", "rtnw_host_make_camera",
                 "rtnw_host_quantize", "rtnw_host_write_ppm", "rtnw_host_load_png", "rtnw_host_free_image", "rtnw_host_write_pfm"]
@@ -193,6 +199,8 @@ def device_lib() -> C.CDLL:
                                  C.c_void_p]
         L.rtnw_render_aov.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams), C.POINTER(Aov),
                                       C.POINTER(Stats)]
+        L.rtnw_denoise.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Aov), C.c_int32, C.c_int32, C.c_int32, C.POINTER(DenoiseParams),
+                                   C.c_void_p, C.POINTER(Stats)]
         L.rtnw_eval_texture.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]
         L.rtnw_eval_perlin.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]
         L.rtnw_scatter.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p,
@@ -364,6 +372,27 @@ class Context:
 
     def upload(self, desc) -> "DeviceScene":
         return DeviceScene(self, desc)
+
+    def denoise(self, sums: np.ndarray, aov: dict, ns: int, iterations: int = 5, sigma_luminance: float = 4.0,
+                sigma_depth: float = 1.0, normal_power_log2: int = 7, stats: Stats | None = None) -> np.ndarray:
+        """Denoise a frame on the GPU from its first-hit feature buffers (include/rtnw.h: rtnw_denoise): `sums` as
+        DeviceScene.render returns them and `aov` as DeviceScene.render_aov returns it for the same params, ns = their
+        sample_count.  Returns the denoised MEAN colour, (ny, nx, 3) float32, row j = 0 at the bottom.  Pass a Stats to
+        receive the call's statistics."""
+        ny, nx, _ = sums.shape
+        sums = np.ascontiguousarray(sums, dtype=np.float32)
+        bufs = {k: np.ascontiguousarray(aov[k], dtype=np.int32 if k == "hits" else np.float32)
+                for k in ("albedo", "normal", "depth", "hits")}
+        for k, shape in (("albedo", (ny, nx, 3)), ("normal", (ny, nx, 3)), ("depth", (ny, nx)), ("hits", (ny, nx))):
+            if bufs[k].shape != shape:
+                raise RtnwError(RTNW_ERR_INVALID, f"aov[{k!r}] has shape {bufs[k].shape}, expected {shape}")
+        feats = Aov(bufs["albedo"].ctypes.data, bufs["normal"].ctypes.data, bufs["depth"].ctypes.data, bufs["hits"].ctypes.data, None)
+        out = np.empty((ny, nx, 3), np.float32)
+        dp = DenoiseParams(iterations, sigma_luminance, sigma_depth, normal_power_log2)
+        st = Stats() if stats is None else stats
+        _check_dev(device_lib().rtnw_denoise(self._h, sums.ctypes.data, C.byref(feats), nx, ny, ns, C.byref(dp), out.ctypes.data,
+                                             C.byref(st)))
+        return out
 
     def close(self):
         if self._h:

@@ -490,6 +490,209 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_
     P.hits[q] = __float_as_int(nrm.w);
 }
 
+// ---- rtnw_denoise: spatial-only SVGF (include/rtnw.h).  One thread per pixel, 2D blocks.  Every operation is float32 in the
+// order of the C restatement tests/denoise_oracle.c (--fmad=false: no contraction), so the two agree bit for bit.
+#define DN_EPS_ALBEDO 1e-3f  // albedo floor of the demodulation
+#define DN_EPS_DEPTH 1e-3f   // depth tolerance, relative to the centre pixel's depth
+#define DN_EPS_LUM 1e-4f     // luminance tolerance where the variance is 0
+#define DN_LUM_R 0.2126f     // Rec. 709 luminance of the irradiance
+#define DN_LUM_G 0.7152f
+#define DN_LUM_B 0.0722f
+#define DN_BX 32
+#define DN_BY 8
+
+struct dn_args {
+    int nx, ny, k;           // image size, normal_power_log2
+    float fns, sigma_l, sigma_z;
+    const float* color;      // nx*ny*3 sums
+    const float* albedo;     // nx*ny*3 sums
+    const float* normal;     // nx*ny*3 sums
+    const float* depth;      // nx*ny sums
+    const int32_t* hits;     // nx*ny
+    float4* ev[2];           // irradiance xyz, variance (ping-pong)
+    float4* feat;            // normalised normal xyz, depth (0 for misses)
+    float2* grad;            // |dz/dx|, |dz/dy|
+    unsigned char* hit;      // hits > 0
+    float* out;              // nx*ny*3 denoised means (may alias color: only k_dn_prepare reads it)
+};
+
+// exp(-x) for x >= 0: 2^-y, y = x*log2(e) = n + f, f in [0, 1): a Horner polynomial for 2^-f (constant term exactly 1) times
+// 2^-n from the exponent bits; 0 for x >= 88, +inf and NaN.  Within 1e-5 relative of exp (tests/test_denoise_cpu.py).
+__device__ __forceinline__ float dn_exp_neg(float x) {
+    if (!(x < 88.f)) return 0.f;
+    const float y = x * 1.44269502f;
+    const float n = floorf(y);
+    const float f = y - n;
+    const float p = 1.f + f * (-6.93147063e-01f + f * (2.40224302e-01f + f * (-5.54905124e-02f + f * (9.57873557e-03f +
+                    f * (-1.27437152e-03f + f * 1.08902554e-04f)))));
+    return p * __uint_as_float((uint32_t)(127 - (int)n) << 23);
+}
+
+__device__ __forceinline__ float dn_lum(float4 e) { return DN_LUM_R * e.x + DN_LUM_G * e.y + DN_LUM_B * e.z; }
+
+// max(0, n_p . n_q)^(2^k)
+__device__ __forceinline__ float dn_normal_weight(float4 a, float4 b, int k) {
+    const float d = a.x * b.x + a.y * b.y + a.z * b.z;
+    float w = d > 0.f ? d : 0.f;
+    for (int s = 0; s < k; ++s) w = w * w;
+    return w;
+}
+
+// |z_p - z_q| / (sigma_z * |grad z_p . (dx, dy)| + eps * z_p), the gradient's components taken as absolute values
+__device__ __forceinline__ float dn_depth_distance(float zp, float zq, float2 g, float sigma_z, int dx, int dy) {
+    const float ox = (float)abs(dx), oy = (float)abs(dy);
+    return fabsf(zp - zq) / (sigma_z * (g.x * ox + g.y * oy) + DN_EPS_DEPTH * zp);
+}
+
+__device__ __forceinline__ float dn_albedo(const dn_args& P, int p, int c) {
+    const float a = __ldg(&P.albedo[3 * p + c]) / P.fns;
+    return a > DN_EPS_ALBEDO ? a : DN_EPS_ALBEDO;
+}
+
+__device__ __forceinline__ float dn_depth(const dn_args& P, int q) { return __ldg(&P.depth[q]) / (float)__ldg(&P.hits[q]); }
+
+// means, demodulation, normalised normal, hit flag, depth gradient
+__global__ void __launch_bounds__(DN_BX * DN_BY) k_dn_prepare(const __grid_constant__ dn_args P) {
+    const int i = blockIdx.x * DN_BX + threadIdx.x, j = blockIdx.y * DN_BY + threadIdx.y;
+    if (i >= P.nx || j >= P.ny) return;
+    const int p = j * P.nx + i;
+    const int h = __ldg(&P.hits[p]);
+    float4 e;
+    e.x = (__ldg(&P.color[3 * p]) / P.fns) / dn_albedo(P, p, 0);
+    e.y = (__ldg(&P.color[3 * p + 1]) / P.fns) / dn_albedo(P, p, 1);
+    e.z = (__ldg(&P.color[3 * p + 2]) / P.fns) / dn_albedo(P, p, 2);
+    e.w = 0.f;
+    float4 f = make_float4(0.f, 0.f, 0.f, 0.f);
+    float2 g = make_float2(0.f, 0.f);
+    if (h > 0) {
+        const float fh = (float)h;
+        const float x = __ldg(&P.normal[3 * p]) / fh, y = __ldg(&P.normal[3 * p + 1]) / fh, w = __ldg(&P.normal[3 * p + 2]) / fh;
+        const float len = sqrtf(x * x + y * y + w * w);
+        if (len > 0.f) { f.x = x / len; f.y = y / len; f.z = w / len; }
+        f.w = __ldg(&P.depth[p]) / fh;
+        for (int axis = 0; axis < 2; ++axis) {
+            const bool lo_ok = axis == 0 ? i > 0 : j > 0, hi_ok = axis == 0 ? i < P.nx - 1 : j < P.ny - 1;
+            const int lo = axis == 0 ? p - 1 : p - P.nx, hi = axis == 0 ? p + 1 : p + P.nx;
+            const bool l = lo_ok && __ldg(&P.hits[lo]) > 0, u = hi_ok && __ldg(&P.hits[hi]) > 0;
+            float d = 0.f;
+            if (l && u) d = fabsf(dn_depth(P, hi) - dn_depth(P, lo)) * 0.5f;
+            else if (u) d = fabsf(dn_depth(P, hi) - f.w);
+            else if (l) d = fabsf(f.w - dn_depth(P, lo));
+            if (axis == 0) g.x = d; else g.y = d;
+        }
+    }
+    P.ev[0][p] = e;
+    P.feat[p] = f;
+    P.grad[p] = g;
+    P.hit[p] = h > 0;
+}
+
+// variance of the luminance over 7x7, weights w_n * exp(-d_z) (1 at the centre); reads ev[0], writes ev[1] = (e, var)
+__global__ void __launch_bounds__(DN_BX * DN_BY) k_dn_variance(const __grid_constant__ dn_args P) {
+    const int i = blockIdx.x * DN_BX + threadIdx.x, j = blockIdx.y * DN_BY + threadIdx.y;
+    if (i >= P.nx || j >= P.ny) return;
+    const int p = j * P.nx + i;
+    const bool hp = P.hit[p];
+    const float4 fp = P.feat[p];
+    const float2 gp = P.grad[p];
+    float sw = 0.f, s1 = 0.f, s2 = 0.f;
+    for (int dy = -3; dy <= 3; ++dy) {
+        const int qj = j + dy;
+        if (qj < 0 || qj >= P.ny) continue;
+        for (int dx = -3; dx <= 3; ++dx) {
+            const int qi = i + dx;
+            if (qi < 0 || qi >= P.nx) continue;
+            const int q = qj * P.nx + qi;
+            if ((bool)__ldg(&P.hit[q]) != hp) continue;
+            float w = 1.f;
+            if (q != p && hp) {
+                const float4 fq = __ldg(&P.feat[q]);
+                w = dn_normal_weight(fp, fq, P.k) * dn_exp_neg(dn_depth_distance(fp.w, fq.w, gp, P.sigma_z, dx, dy));
+            }
+            const float l = dn_lum(__ldg(&P.ev[0][q]));
+            sw = sw + w;
+            s1 = s1 + w * l;
+            s2 = s2 + w * l * l;
+        }
+    }
+    const float m1 = s1 / sw, m2 = s2 / sw;
+    const float v = m2 - m1 * m1;
+    float4 e = P.ev[0][p];
+    e.w = v > 0.f ? v : 0.f;
+    P.ev[1][p] = e;
+}
+
+// one a-trous pass with step 2^it: reads ev[src], writes ev[1 - src]; the last pass remodulates into out instead
+__global__ void __launch_bounds__(DN_BX * DN_BY) k_dn_atrous(const __grid_constant__ dn_args P, int it, int src, int last) {
+    const int i = blockIdx.x * DN_BX + threadIdx.x, j = blockIdx.y * DN_BY + threadIdx.y;
+    if (i >= P.nx || j >= P.ny) return;
+    const float4* __restrict__ ev = P.ev[src];
+    const int p = j * P.nx + i;
+    const bool hp = P.hit[p];
+    const float4 fp = P.feat[p];
+    const float4 ep = ev[p];
+    // 3x3 binomial blur of the variance over the neighbours p may mix with: same hit class, weights w_n for hits
+    float gs = 0.f, gw = 0.f;
+    for (int dy = -1; dy <= 1; ++dy) {
+        const int qj = j + dy;
+        if (qj < 0 || qj >= P.ny) continue;
+        for (int dx = -1; dx <= 1; ++dx) {
+            const int qi = i + dx;
+            if (qi < 0 || qi >= P.nx) continue;
+            const int q = qj * P.nx + qi;
+            if ((bool)__ldg(&P.hit[q]) != hp) continue;
+            float w = (float)((2 - abs(dx)) * (2 - abs(dy)));
+            if (q != p && hp) w = w * dn_normal_weight(fp, __ldg(&P.feat[q]), P.k);
+            gs = gs + w * __ldg(&ev[q].w);
+            gw = gw + w;
+        }
+    }
+    const float2 gp = P.grad[p];
+    const float lp = dn_lum(ep);
+    const float dl_den = P.sigma_l * sqrtf(gs / gw) + DN_EPS_LUM;
+    const float H[5] = {1.f / 16.f, 1.f / 4.f, 3.f / 8.f, 1.f / 4.f, 1.f / 16.f};
+    const int step = 1 << it;
+    float sw = 0.f, sv = 0.f, sx = 0.f, sy = 0.f, sz = 0.f;
+#pragma unroll
+    for (int b = -2; b <= 2; ++b) {
+        const int dy = b * step, qj = j + dy;
+        if (qj < 0 || qj >= P.ny) continue;
+#pragma unroll
+        for (int a = -2; a <= 2; ++a) {
+            const int dx = a * step, qi = i + dx;
+            if (qi < 0 || qi >= P.nx) continue;
+            const int q = qj * P.nx + qi;
+            if ((bool)__ldg(&P.hit[q]) != hp) continue;
+            const float4 eq = __ldg(&ev[q]);
+            float w;
+            if (a == 0 && b == 0) {
+                w = H[2] * H[2];
+            } else {
+                const float dl = fabsf(lp - dn_lum(eq)) / dl_den;
+                if (hp) {
+                    const float4 fq = __ldg(&P.feat[q]);
+                    const float dz = dn_depth_distance(fp.w, fq.w, gp, P.sigma_z, dx, dy);
+                    w = H[a + 2] * H[b + 2] * dn_normal_weight(fp, fq, P.k) * dn_exp_neg(dz + dl);
+                } else {
+                    w = H[a + 2] * H[b + 2] * dn_exp_neg(dl);
+                }
+            }
+            sw = sw + w;
+            sx = sx + w * eq.x;
+            sy = sy + w * eq.y;
+            sz = sz + w * eq.z;
+            sv = sv + w * w * eq.w;
+        }
+    }
+    if (last) {
+        P.out[3 * p] = (sx / sw) * dn_albedo(P, p, 0);
+        P.out[3 * p + 1] = (sy / sw) * dn_albedo(P, p, 1);
+        P.out[3 * p + 2] = (sz / sw) * dn_albedo(P, p, 2);
+    } else {
+        P.ev[1 - src][p] = make_float4(sx / sw, sy / sw, sz / sw, sv / (sw * sw));
+    }
+}
+
 // the epilogue of the sample loop, PSC/main.cpp:315-325, one thread per pixel; output row 0 = top row (j = ny-1)
 __global__ void k_quantize(const float* __restrict__ sums, int nx, int ny, float inv_ns, int clamp255, int32_t* __restrict__ out) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1808,6 +2011,66 @@ int rtnw_eval_texture(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t tex_id, co
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(rgb_out, d_out.p, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    return RTNW_OK;
+}
+
+int rtnw_denoise(rtnw_ctx* ctx, const float* color_sums, const rtnw_aov* features, int32_t nx, int32_t ny, int32_t ns,
+                 const rtnw_denoise_params* dp, float* rgb_out, rtnw_stats* stats) {
+    int rc = check_ctx(ctx);
+    if (rc != RTNW_OK) return rc;
+    if (!color_sums || !features || !features->albedo || !features->normal || !features->depth || !features->hits || !dp || !rgb_out)
+        return fail(RTNW_ERR_INVALID, "null argument");
+    if (nx <= 0 || ny <= 0 || (long long)nx * ny > 0x7fffffffLL / 4 || ns <= 0) return fail(RTNW_ERR_INVALID, "bad image size or sample count");
+    if (dp->iterations < 1 || dp->iterations > 8) return fail(RTNW_ERR_INVALID, "iterations must be 1..8");
+    if (dp->normal_power_log2 < 0 || dp->normal_power_log2 > 10) return fail(RTNW_ERR_INVALID, "normal_power_log2 must be 0..10");
+    if (!(dp->sigma_luminance > 0.f) || !std::isfinite(dp->sigma_luminance) || !(dp->sigma_depth > 0.f) || !std::isfinite(dp->sigma_depth))
+        return fail(RTNW_ERR_INVALID, "sigmas must be finite and > 0");
+    const size_t n = (size_t)nx * ny;
+    // color (the output after k_dn_prepare) | albedo | normal | depth | hits | ev[0] | ev[1] | feat | grad | hit, 256-B aligned
+    const size_t sz[10] = {12 * n, 12 * n, 12 * n, 4 * n, 4 * n, 16 * n, 16 * n, 16 * n, 8 * n, n};
+    size_t off[10], total = 0;
+    for (int b = 0; b < 10; ++b) { off[b] = total; total += align256(sz[b]); }
+    dev_buf d;
+    CUDA_TRY(d.alloc(total));
+    unsigned char* base = d.as<unsigned char>();
+    dn_args a;
+    a.nx = nx; a.ny = ny; a.k = dp->normal_power_log2;
+    a.fns = (float)ns; a.sigma_l = dp->sigma_luminance; a.sigma_z = dp->sigma_depth;
+    float* color = reinterpret_cast<float*>(base + off[0]);
+    a.color = color;
+    a.albedo = reinterpret_cast<float*>(base + off[1]);
+    a.normal = reinterpret_cast<float*>(base + off[2]);
+    a.depth = reinterpret_cast<float*>(base + off[3]);
+    a.hits = reinterpret_cast<int32_t*>(base + off[4]);
+    a.ev[0] = reinterpret_cast<float4*>(base + off[5]);
+    a.ev[1] = reinterpret_cast<float4*>(base + off[6]);
+    a.feat = reinterpret_cast<float4*>(base + off[7]);
+    a.grad = reinterpret_cast<float2*>(base + off[8]);
+    a.hit = base + off[9];
+    a.out = color;
+    CUDA_TRY(cudaEventRecord(ctx->ev_t0, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(color, color_sums, sz[0], cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(base + off[1], features->albedo, sz[1], cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(base + off[2], features->normal, sz[2], cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(base + off[3], features->depth, sz[3], cudaMemcpyHostToDevice, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(base + off[4], features->hits, sz[4], cudaMemcpyHostToDevice, ctx->stream));
+    const dim3 block(DN_BX, DN_BY), grid((unsigned)((nx + DN_BX - 1) / DN_BX), (unsigned)((ny + DN_BY - 1) / DN_BY));
+    CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
+    k_dn_prepare<<<grid, block, 0, ctx->stream>>>(a);
+    k_dn_variance<<<grid, block, 0, ctx->stream>>>(a);
+    for (int it = 0; it < dp->iterations; ++it)  // k_dn_variance left (e, var) in ev[1]
+        k_dn_atrous<<<grid, block, 0, ctx->stream>>>(a, it, it % 2 == 0 ? 1 : 0, it == dp->iterations - 1);
+    CUDA_TRY(cudaGetLastError());
+    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
+    CUDA_TRY(cudaMemcpyAsync(rgb_out, color, sz[0], cudaMemcpyDeviceToHost, ctx->stream));
+    CUDA_TRY(cudaEventRecord(ctx->ev_t1, ctx->stream));
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    if (stats) {
+        std::memset(stats, 0, sizeof *stats);
+        CUDA_TRY(cudaEventElapsedTime(&stats->kernel_ms, ctx->ev0, ctx->ev1));
+        CUDA_TRY(cudaEventElapsedTime(&stats->total_ms, ctx->ev_t0, ctx->ev_t1));
+        stats->kernel_launches = dp->iterations + 2;
+    }
     return RTNW_OK;
 }
 
