@@ -17,17 +17,9 @@
 
 using namespace rtnw_dev;
 
-#ifndef RTNW_BLOCK
-#define RTNW_BLOCK 320      // x 2 blocks per SM at 96 registers: 640 rays in flight per SM (measured against 256 x 2 at 124
-#endif                      // registers, 192 x 3, 288 x 2, 352 x 2, 384 x 2 and 256 x 3 at 80: DESIGN.md §6)
 #ifndef RTNW_MIN_BLOCKS
-#define RTNW_MIN_BLOCKS 2   // resident blocks per SM the register allocation is sized for
+#define RTNW_MIN_BLOCKS 2   // resident blocks per SM the register allocation is sized for (block size: RTNW_BLOCK, rtnw_device.cuh)
 #endif
-#ifndef RTNW_GROUP
-#define RTNW_GROUP RTNW_BLOCK  // threads that traverse BVH items cooperatively: the whole block, or 32 = one warp
-#endif
-static_assert(RTNW_GROUP == RTNW_BLOCK || RTNW_GROUP == 32,
-              "cooperating group = the whole block (__syncthreads) or one warp (__syncwarp); other sizes would need named barriers");
 
 #define RTNW_MAX_CHUNKS 64
 #define RTNW_MAX_DEVICES 16
@@ -64,11 +56,8 @@ __device__ __forceinline__ float from_fixed(unsigned long long u) {
     return (float)((double)(long long)u * (1.0 / 2199023255552.0));  // 2^-41, one rounding
 }
 
-typedef coop_smem<RTNW_GROUP, 1> group_smem;   // reference-exact kernels: one BVH item at a time
-typedef coop_smem<RTNW_GROUP, 2> group_smem2;  // RTNW_F_FAST_BVH kernels: two BVH items traversed together (two ray frames)
-template <bool FAST> struct smem_of { typedef group_smem type; };
-template <> struct smem_of<true> { typedef group_smem2 type; };
-template <bool FAST> struct block_smem { typename smem_of<FAST>::type g[RTNW_BLOCK / RTNW_GROUP]; };
+// the reference-exact kernels traverse one BVH item at a time; the RTNW_F_FAST_BVH kernels two together (two ray frames)
+template <bool FAST> using block_smem = coop_smem<FAST ? 2 : 1>;
 
 // The sample loop of PSC/main.cpp:299-313 as ONE persistent megakernel.
 //
@@ -85,8 +74,8 @@ template <bool FAST> struct block_smem { typename smem_of<FAST>::type g[RTNW_BLO
 template <bool COUNT, bool FAST>
 __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const render_args P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    typedef typename smem_of<FAST>::type SM;
-    SM& sm = reinterpret_cast<block_smem<FAST>*>(smem_raw)->g[threadIdx.x / RTNW_GROUP];
+    typedef block_smem<FAST> SM;
+    SM& sm = *reinterpret_cast<SM*>(smem_raw);
     constexpr unsigned FULL = 0xffffffffu;
     const unsigned lane = threadIdx.x & 31u;
     const int nx = P.p.nx, ny = P.p.ny;
@@ -98,18 +87,15 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
     const bool denan = (P.p.flags & RTNW_F_DE_NAN) != 0;
     const bool sky = P.p.background == RTNW_BG_SKY;
 
-    coop_init<RTNW_GROUP, SM>(sm);
-    group_sync<RTNW_GROUP>();
-#if RTNW_SMEM_NODES
-    stage_top_nodes<RTNW_GROUP, FAST, SM>(P.S, sm);
-#endif
+    coop_init<SM>(sm);
+    __syncthreads();
     int r3 = 0;  // index of the cooperative traversal's next round, mod 3 (coop_bvh_item)
 #ifdef RTNW_ROUND_STATS
     const long long t_start = clock64();
 #endif
     // The work item of a thread (pixel, sample range, running sum) lives in shared memory: it is touched when a path
     // ends, i.e. once every few rounds, and would otherwise occupy eight registers across every round.
-    int me = threadIdx.x % RTNW_GROUP;  // index of this thread's work item in sm.acc / sm.span (RTNW_MIGRATE: travels with the ray)
+    int me = threadIdx.x % RTNW_BLOCK;  // index of this thread's work item in sm.acc / sm.span
     bool alive = true, need = true, has_item = false;
     int depth = 0;
     f3 T = mk3(0.f, 0.f, 0.f);
@@ -168,7 +154,7 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
                 }
             }
         }
-        if (RTNW_GROUP == 32 ? __ballot_sync(FULL, alive) == 0 : __syncthreads_count(alive) == 0) break;  // the group is done
+        if (__syncthreads_count(alive) == 0) break;  // the block is done
         if (alive && need && has_item) {
             const int k = __float_as_int(sm.acc[me].w);
             const int4 sp = sm.span[me];
@@ -190,69 +176,10 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
 #ifdef RTNW_ROUND_STATS
         const long long c0 = clock64();
 #endif
-        const hkey_t key = coop_closest_hit<RTNW_GROUP, COUNT, FAST, SM>(P.S, sm, wr, tracing, P.p.t_min, P.p.t_max, mk, cnt, r3);
+        const hkey_t key = coop_closest_hit<COUNT, FAST, SM>(P.S, sm, wr, tracing, P.p.t_min, P.p.t_max, mk, cnt, r3);
 #ifdef RTNW_ROUND_STATS
         if (threadIdx.x == 0) { RTNW_STAT(10, 1); RTNW_STAT(11, clock64() - c0); }
         const long long c1 = clock64();
-#endif
-#if RTNW_MIGRATE
-        // ---- rays change threads so that a warp shades rays of ONE kind: the next step of a ray (miss / light: the path ends
-        // and a new one starts; lambertian; metal; dielectric; isotropic) is known from its hit.  Each ray's state (20 words)
-        // is written to shared memory at its rank in a counting sort by that class and read back by the thread of that rank;
-        // the work item stays where it is (sm.acc / sm.span[me], `me` travels with the ray).  What a ray computes does not
-        // depend on the thread that runs it, so results are unchanged.
-        bool tracing_ = tracing;
-        hkey_t key_ = key;
-        {
-            static_assert(RTNW_GROUP == RTNW_BLOCK, "ray migration uses block barriers");
-            int cls = 0;
-            if (tracing) {
-                cls = 1;
-                if (key != RTNW_KEY_NONE) {
-                    const int mat_id = __float_as_int(__ldg(&P.S.recs[key_rec(key)].b).w);
-                    const float4 m0 = __ldg(reinterpret_cast<const float4*>(P.S.materials + mat_id));
-                    const uint32_t mkind = __float_as_uint(m0.x);
-                    cls = mkind == RTNW_MAT_DIFFUSE_LIGHT ? 2 : mkind == RTNW_MAT_METAL ? 5 : mkind == RTNW_MAT_DIELECTRIC ? 6 : mkind == RTNW_MAT_ISOTROPIC ? 7 : 3;
-                    if (cls == 3 && __float_as_uint(__ldg(reinterpret_cast<const float4*>(P.S.textures + __float_as_int(m0.y))).x) != RTNW_TEX_CONSTANT) cls = 4;
-                }
-            }
-            const unsigned same = __match_any_sync(FULL, cls);
-            const int leader = __ffs(same) - 1;
-            int base = 0;
-            if ((int)lane == leader) base = atomicAdd(&sm.bins[cls], __popc(same));
-            base = __shfl_sync(FULL, base, leader);
-            const int off = base + __popc(same & ((1u << lane) - 1u));
-            __syncthreads();
-            const int4 b0 = *reinterpret_cast<const int4*>(&sm.bins[0]), b1 = *reinterpret_cast<const int4*>(&sm.bins[4]);
-            const int cnt8[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
-            int pos = off;
-#pragma unroll
-            for (int c = 0; c < 7; ++c) pos += c < cls ? cnt8[c] : 0;
-            float4* xch = reinterpret_cast<float4*>(sm.q);  // both queues are empty between closest-hit queries
-            const unsigned flags = (alive ? 1u : 0u) | (need ? 2u : 0u) | (has_item ? 4u : 0u) | (tracing ? 8u : 0u);
-            xch[5 * pos + 0] = make_float4(wr.o.x, wr.o.y, wr.o.z, wr.time);
-            xch[5 * pos + 1] = make_float4(wr.d.x, wr.d.y, wr.d.z, T.x);
-            xch[5 * pos + 2] = make_float4(T.y, T.z, __uint_as_float((uint32_t)g.x), __uint_as_float((uint32_t)(g.x >> 32)));
-            xch[5 * pos + 3] = make_float4(__uint_as_float(g.sample), __int_as_float(depth), __uint_as_float(flags), __int_as_float(me));
-            xch[5 * pos + 4] = make_float4(__uint_as_float((uint32_t)key), __uint_as_float((uint32_t)(key >> 32)), 0.f, 0.f);
-            __syncthreads();
-            if (threadIdx.x < 8) sm.bins[threadIdx.x] = 0;
-            const float4 x0 = xch[5 * threadIdx.x + 0], x1 = xch[5 * threadIdx.x + 1], x2 = xch[5 * threadIdx.x + 2],
-                         x3 = xch[5 * threadIdx.x + 3], x4 = xch[5 * threadIdx.x + 4];
-            wr.o = mk3(x0.x, x0.y, x0.z); wr.time = x0.w;
-            wr.d = mk3(x1.x, x1.y, x1.z);
-            T = mk3(x1.w, x2.x, x2.y);
-            g.x = (unsigned long long)__float_as_uint(x2.z) | ((unsigned long long)__float_as_uint(x2.w) << 32);
-            g.sample = __float_as_uint(x3.x);
-            depth = __float_as_int(x3.y);
-            const unsigned fl = __float_as_uint(x3.z);
-            alive = fl & 1u; need = (fl & 2u) != 0; has_item = (fl & 4u) != 0; tracing_ = (fl & 8u) != 0;
-            me = __float_as_int(x3.w);
-            key_ = (hkey_t)__float_as_uint(x4.x) | ((hkey_t)__float_as_uint(x4.y) << 32);
-            __syncthreads();  // the queues are used again by the next closest-hit query
-        }
-#define tracing tracing_
-#define key key_
 #endif
         // ---- one level of color(), PSC/main.cpp:25-46, in iterative form (DESIGN.md §5)
         if (tracing) {
@@ -272,7 +199,7 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
                     const uint32_t tk = __float_as_uint(__ldg(reinterpret_cast<const float4*>(P.S.textures + __float_as_int(m0.y))).x);
                     want_uv = tk == RTNW_TEX_IMAGE || tk == RTNW_TEX_CHECKER;
                 }
-                finish_hit<FAST && RTNW_FAST_APPROX>(P.S, wr, h, s, want_uv);
+                finish_hit(P.S, wr, h, s, want_uv);
                 if (__float_as_uint(m0.x) == RTNW_MAT_DIFFUSE_LIGHT) {  // the only material that emits; it never scatters
                     if (emit) L = L + T * texture_value(P.S, __float_as_int(m0.y), s.u, s.v, s.p);
                 } else if (depth < P.p.max_depth) {
@@ -299,10 +226,6 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
                 sm.acc[me] = acc;
             }
         }
-#if RTNW_MIGRATE
-#undef tracing
-#undef key
-#endif
 #ifdef RTNW_ROUND_STATS
         if (threadIdx.x == 0) RTNW_STAT(13, clock64() - c1);
 #endif
@@ -310,8 +233,8 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
 #ifdef RTNW_ROUND_STATS
     if (threadIdx.x == 0) RTNW_STAT(12, clock64() - t_start);
 #endif
-    group_sync<RTNW_GROUP>();
-    if (threadIdx.x % RTNW_GROUP == 0 && sm.overflow) atomicAdd(&P.ctr[4], 1ull);
+    __syncthreads();
+    if (threadIdx.x % RTNW_BLOCK == 0 && sm.overflow) atomicAdd(&P.ctr[4], 1ull);
     // work counters: one atomic per warp
     if (COUNT) { box_total = cnt.box_tests; prim_total = cnt.prim_tests; }
     unsigned long long rays_total = n_rays;
@@ -331,8 +254,8 @@ template <bool FAST>
 __global__ void __launch_bounds__(RTNW_BLOCK) k_trace(const scene_view S, const rtnw_ray* __restrict__ rays, size_t n, float t_min,
                                                       float t_max, uint64_t seed, rtnw_hit* __restrict__ out) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    typedef typename smem_of<FAST>::type SM;
-    SM& sm = reinterpret_cast<block_smem<FAST>*>(smem_raw)->g[threadIdx.x / RTNW_GROUP];
+    typedef block_smem<FAST> SM;
+    SM& sm = *reinterpret_cast<SM*>(smem_raw);
     const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool active = q < n;  // idle threads of the last block still work on the block's BVH tasks
     rtnw_ray in;
@@ -347,13 +270,10 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_trace(const scene_view S, const 
     mk.k0 = (uint32_t)seed; mk.k1 = (uint32_t)(seed >> 32); mk.pixel = in.key; mk.sample = 0; mk.depth = 0;
     trav_counters cnt;
     cnt.box_tests = 0; cnt.prim_tests = 0;
-    coop_init<RTNW_GROUP, SM>(sm);
-    group_sync<RTNW_GROUP>();
-#if RTNW_SMEM_NODES
-    stage_top_nodes<RTNW_GROUP, FAST, SM>(S, sm);
-#endif
+    coop_init<SM>(sm);
+    __syncthreads();
     int r3 = 0;
-    const hkey_t key = coop_closest_hit<RTNW_GROUP, false, FAST, SM>(S, sm, r, active, t_min, t_max, mk, cnt, r3);
+    const hkey_t key = coop_closest_hit<false, FAST, SM>(S, sm, r, active, t_min, t_max, mk, cnt, r3);
     if (!active) return;
     hit_t h;
     key_to_hit(S, key, t_max, h);
@@ -363,7 +283,7 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_trace(const scene_view S, const 
     o.mat_id = -1;
     if (h.rec >= 0) {
         surf_t s;
-        finish_hit<FAST && RTNW_FAST_APPROX>(S, r, h, s);
+        finish_hit(S, r, h, s);
         o.prim_id = S.rec_leaf[h.rec];
         o.sub_id = h.face;
         o.t = h.t;
@@ -411,9 +331,9 @@ __device__ __noinline__ ray_t aov_camera_ray(const rtnw_camera& cam, int nx, int
 template <bool FAST>
 __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_args P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    typedef typename smem_of<FAST>::type SM;
+    typedef block_smem<FAST> SM;
     aov_smem<FAST>& A = *reinterpret_cast<aov_smem<FAST>*>(smem_raw);
-    SM& sm = A.coop.g[threadIdx.x / RTNW_GROUP];
+    SM& sm = A.coop;
     const int me = threadIdx.x;
     const int nx = P.p.nx, ny = P.p.ny;
     const int pix = blockIdx.x * blockDim.x + threadIdx.x;
@@ -421,20 +341,17 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_
     const uint32_t k0 = (uint32_t)P.p.seed, k1 = (uint32_t)(P.p.seed >> 32);
     trav_counters cnt;
     cnt.box_tests = 0; cnt.prim_tests = 0;
-    coop_init<RTNW_GROUP, SM>(sm);
+    coop_init<SM>(sm);
     A.acc[me] = make_float4(0.f, 0.f, 0.f, 0.f);
     A.nrm[me] = make_float4(0.f, 0.f, 0.f, __int_as_float(0));
-    group_sync<RTNW_GROUP>();
-#if RTNW_SMEM_NODES
-    stage_top_nodes<RTNW_GROUP, FAST, SM>(P.S, sm);
-#endif
+    __syncthreads();
     int r3 = 0;
     for (int k = 0; k < P.p.sample_count; ++k) {
         const int s = P.p.sample_begin + k * P.p.sample_stride;
         const ray_t r = aov_camera_ray(P.cam, nx, ny, pix, s, P.p.seed);
         medium_key mk;
         mk.k0 = k0; mk.k1 = k1; mk.pixel = (uint32_t)pix; mk.sample = (uint32_t)s; mk.depth = 0;
-        const hkey_t key = coop_closest_hit<RTNW_GROUP, false, FAST, SM>(P.S, sm, r, active, P.p.t_min, P.p.t_max, mk, cnt, r3);
+        const hkey_t key = coop_closest_hit<false, FAST, SM>(P.S, sm, r, active, P.p.t_min, P.p.t_max, mk, cnt, r3);
         if (!active) continue;
         hit_t h;
         key_to_hit(P.S, key, P.p.t_max, h);
@@ -459,7 +376,7 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_
             want_uv = tk == RTNW_TEX_IMAGE || tk == RTNW_TEX_CHECKER;
         }
         surf_t sf;
-        finish_hit<FAST && RTNW_FAST_APPROX>(P.S, r, h, sf, want_uv);
+        finish_hit(P.S, r, h, sf, want_uv);
         f3 a;  // the attenuation scatter() returns; a light's emission clamped to 1
         if (mkind == RTNW_MAT_METAL) {
             const float4 m1 = __ldg(reinterpret_cast<const float4*>(P.S.materials + mat_id) + 1);
@@ -479,8 +396,8 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_
         nrm.w = __int_as_float(__float_as_int(nrm.w) + 1);
         A.nrm[me] = nrm;
     }
-    group_sync<RTNW_GROUP>();
-    if (threadIdx.x % RTNW_GROUP == 0 && sm.overflow) atomicAdd(&P.ctr[4], 1ull);
+    __syncthreads();
+    if (threadIdx.x % RTNW_BLOCK == 0 && sm.overflow) atomicAdd(&P.ctr[4], 1ull);
     if (!active) return;
     const size_t q = (size_t)pix;
     const float4 acc = A.acc[me], nrm = A.nrm[me];
@@ -1223,7 +1140,7 @@ struct stream_builder {
     }
     // Collapse binary trees into 4-wide nodes (repeatedly open the child with the largest box) and number the nodes of a
     // whole FOREST level by level: all roots first, then every tree's second level, and so on — so that the first M nodes of
-    // the forest are the top levels of every tree (what k_render can keep in shared memory, RTNW_SMEM_NODES).
+    // the forest are the top levels of every tree (DESIGN.md §6 measured keeping those in shared memory).
     struct tree_t { std::vector<bin_node> bt; int broot = 0; size_t item_rec = 0; int root = 0, depth = 0; };
     void emit_forest(std::vector<tree_t>& forest) {
         struct pend { int tree, bnode, depth; size_t parent; int slot; };
@@ -1297,7 +1214,7 @@ struct stream_builder {
         emit_forest(fast_forest);
         for (size_t t = 0; t < exact_forest.size(); ++t) {
             const tree_t &E = exact_forest[t], &F = fast_forest[t];
-            if (2 * RTNW_GROUP + 3 * std::max(E.depth, F.depth) + 8 > group_smem::QN) return bad("gate tree deeper than the cooperative task stack can reserve for");
+            if (2 * RTNW_BLOCK + 3 * std::max(E.depth, F.depth) + 8 > coop_smem<>::QN) return bad("gate tree deeper than the cooperative task stack can reserve for");
             recs[E.item_rec].a.y = bits(E.root);
             recs[E.item_rec].a.z = bits(E.depth);
             recs[E.item_rec].a.w = bits(F.root);   // RTNW_F_FAST_BVH: tree over the leaves' own boxes

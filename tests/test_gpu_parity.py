@@ -308,7 +308,7 @@ def test_render_is_bitwise_deterministic(rtnw, ctx, name, n, ns, reps):
     order the block's threads happened to take the shared-memory tasks in (stands in for racecheck, closed on this pool).
     The full-size soak is the regression test of a real race: the children a round pushes reuse the stack slots the round
     pops, and about once in 10^8 warp-rounds a starved warp read its task after another warp's push had overwritten it — one
-    wrong path in ~7 % of 1000x1000 frames, invisible at small sizes (fixed by the node-warp barrier RTNW_POP_FENCE)."""
+    wrong path in ~7 % of 1000x1000 frames, invisible at small sizes (fixed by the node-warp barrier)."""
     hs = rtnw.HostScene(name)
     ds = ctx.upload(hs.desc_ptr)
     nx = ny = n
