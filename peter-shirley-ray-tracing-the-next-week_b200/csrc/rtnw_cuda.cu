@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "rtnw.h"
@@ -859,6 +860,88 @@ struct dev_buf {  // RAII device allocation for the query entry points
     template <class T> T* as() { return static_cast<T*>(p); }
 };
 
+// Lays out n tables of sz[i] bytes back to back, each at a 256-byte aligned offset off[i]; returns the total size.
+size_t layout256(const size_t* sz, int n, size_t* off) {
+    size_t total = 0;
+    for (int i = 0; i < n; ++i) {
+        off[i] = total;
+        total += (sz[i] + 255) & ~(size_t)255;
+    }
+    return total;
+}
+
+// The device buffers of one query call in one allocation.  add() declares a span of `bytes` with a host source (copied
+// in), a host destination (copied out), both, or neither (device scratch) and returns its index.  copy_in allocates every
+// span (layout256) and copies the sources in; copy_out copies the destinations out and waits for the stream.  The
+// optional events are recorded before the copies in and after the copies out (the total_ms of rtnw_stats).
+struct staging {
+    static constexpr int MAX_SPANS = 10;
+    size_t bytes[MAX_SPANS], off[MAX_SPANS];
+    const void* src[MAX_SPANS];
+    void* dst[MAX_SPANS];
+    int n = 0;
+    dev_buf d;
+
+    int add(size_t size, const void* from = nullptr, void* to = nullptr) {
+        bytes[n] = size;
+        src[n] = from;
+        dst[n] = to;
+        return n++;
+    }
+    template <class T> T* at(int i) { return reinterpret_cast<T*>(d.as<unsigned char>() + off[i]); }
+    cudaError_t copy_in(cudaStream_t st, cudaEvent_t start = nullptr) {
+        cudaError_t e = d.alloc(layout256(bytes, n, off));
+        if (e == cudaSuccess && start) e = cudaEventRecord(start, st);
+        for (int i = 0; i < n && e == cudaSuccess; ++i)
+            if (src[i]) e = cudaMemcpyAsync(at<void>(i), src[i], bytes[i], cudaMemcpyHostToDevice, st);
+        return e;
+    }
+    cudaError_t copy_out(cudaStream_t st, cudaEvent_t done = nullptr) {
+        cudaError_t e = cudaSuccess;
+        for (int i = 0; i < n && e == cudaSuccess; ++i)
+            if (dst[i]) e = cudaMemcpyAsync(dst[i], at<void>(i), bytes[i], cudaMemcpyDeviceToHost, st);
+        if (e == cudaSuccess && done) e = cudaEventRecord(done, st);
+        return e == cudaSuccess ? cudaStreamSynchronize(st) : e;
+    }
+};
+
+// Makes *buf hold at least `count` elements of device memory: a smaller buffer is freed and replaced, its contents are
+// not kept.  On failure *buf is null, *cap is 0 and the call fails with RTNW_ERR_NOMEM and `what`.
+template <class T>
+int grow(T** buf, size_t* cap, size_t count, const char* what) {
+    if (*cap >= count) return RTNW_OK;
+    if (*buf) cudaFree(*buf);
+    *buf = nullptr;
+    *cap = 0;
+    if (cudaMalloc(buf, count * sizeof(T)) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(RTNW_ERR_NOMEM, what);
+    }
+    *cap = count;
+    return RTNW_OK;
+}
+
+// Launches a block-cooperative kernel whose dynamic shared memory is one SMEM.  That is more than the 48 KB a kernel gets
+// by default, so the kernel opts in first.
+template <class SMEM, class... P, class... A>
+int launch_coop(void (*k)(P...), unsigned grid, cudaStream_t st, const A&... args) {
+    CUDA_TRY(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SMEM)));
+    k<<<grid, RTNW_BLOCK, sizeof(SMEM), st>>>(args...);
+    CUDA_TRY(cudaGetLastError());
+    return RTNW_OK;
+}
+
+// Calls f(count, fast) with the flags that select a traversal kernel's instantiation, RTNW_F_COUNTERS and RTNW_F_FAST_BVH,
+// as std::bool_constant values, so that f can name the instantiation with decltype(count)::value.
+template <class F>
+int by_variant(uint32_t flags, F&& f) {
+    using T = std::true_type;
+    using N = std::false_type;
+    const bool count = (flags & RTNW_F_COUNTERS) != 0;
+    if (flags & RTNW_F_FAST_BVH) return count ? f(T(), T()) : f(N(), T());
+    return count ? f(T(), N()) : f(N(), N());
+}
+
 }  // namespace
 
 struct rtnw_ctx {
@@ -884,7 +967,6 @@ struct rtnw_scene {
     scene_view view;
     void* slab = nullptr;  // one allocation holding every table
     size_t slab_bytes = 0;
-    int32_t n_leaf_ids = 0;
 };
 
 namespace {
@@ -1139,8 +1221,8 @@ struct stream_builder {
         return me;
     }
     // Collapse binary trees into 4-wide nodes (repeatedly open the child with the largest box) and number the nodes of a
-    // whole FOREST level by level: all roots first, then every tree's second level, and so on — so that the first M nodes of
-    // the forest are the top levels of every tree (DESIGN.md §6 measured keeping those in shared memory).
+    // whole FOREST level by level: all roots first, then every tree's second level, and so on.  The traversal needs no
+    // particular order; this one stays because every render measurement of the project was taken on the layout it gives.
     struct tree_t { std::vector<bin_node> bt; int broot = 0; size_t item_rec = 0; int root = 0, depth = 0; };
     void emit_forest(std::vector<tree_t>& forest) {
         struct pend { int tree, bnode, depth; size_t parent; int slot; };
@@ -1169,21 +1251,19 @@ struct stream_builder {
                 else (&wnodes[8 * p.parent + 6].x)[p.slot] = bits((int32_t)me);
                 forest[p.tree].depth = std::max(forest[p.tree].depth, p.depth + 1);
                 float v[6][4];
-                int32_t ref[4], lrec[4];
+                int32_t ref[4];
                 for (int q = 0; q < 4; ++q) {
                     ref[q] = RTNW_REF_NONE;
-                    lrec[q] = -1;
                     for (int a = 0; a < 6; ++a) v[a][q] = 0.f;
                 }
                 for (int q = 0; q < nk; ++q) {
                     const bin_node& c = bt[kids[q]];
                     for (int a = 0; a < 3; ++a) { v[a][q] = c.bmin[a]; v[3 + a][q] = c.bmax[a]; }
-                    if (c.gate >= 0) { ref[q] = ~c.gate; lrec[q] = gate_leaves[c.gate].x; }  // lrec: first record of the gate's first leaf (prefetch hint)
+                    if (c.gate >= 0) ref[q] = ~c.gate;
                     else { ref[q] = 0; next.push_back(pend{p.tree, kids[q], p.depth + 1, me, q}); }  // patched when the child is numbered
                 }
                 for (int a = 0; a < 6; ++a) wnodes[8 * me + a] = make_float4(v[a][0], v[a][1], v[a][2], v[a][3]);
-                wnodes[8 * me + 6] = make_float4(bits(ref[0]), bits(ref[1]), bits(ref[2]), bits(ref[3]));
-                wnodes[8 * me + 7] = make_float4(bits(lrec[0]), bits(lrec[1]), bits(lrec[2]), bits(lrec[3]));
+                wnodes[8 * me + 6] = make_float4(bits(ref[0]), bits(ref[1]), bits(ref[2]), bits(ref[3]));  // row 7 stays zero
             }
             level.swap(next);
         }
@@ -1279,11 +1359,24 @@ struct stream_builder {
     }
 };
 
-size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-
 int check_ctx(rtnw_ctx* ctx) {
     if (!ctx) return fail(RTNW_ERR_INVALID, "null context");
     CUDA_TRY(cudaSetDevice(ctx->device));
+    return RTNW_OK;
+}
+
+// k_render and k_aov set counter 4 when a block's traversal task stack overflowed: the frame is then incomplete
+int check_task_stack(const rtnw_ctx* ctx) {
+    if (ctx->ctr_host[4]) return fail(RTNW_ERR_UNSUPPORTED, "BVH task stack overflow: the tree is deeper than RTNW_QN/RTNW_BLOCK - 1 levels");
+    return RTNW_OK;
+}
+
+// *stats (when given) = s, with kernel_ms between ctx->ev0 and ev1 and, when `total`, total_ms between ev_t0 and ev_t1
+int report_stats(rtnw_ctx* ctx, rtnw_stats* stats, rtnw_stats s, bool total) {
+    if (!stats) return RTNW_OK;
+    CUDA_TRY(cudaEventElapsedTime(&s.kernel_ms, ctx->ev0, ctx->ev1));
+    if (total) CUDA_TRY(cudaEventElapsedTime(&s.total_ms, ctx->ev_t0, ctx->ev_t1));
+    *stats = s;
     return RTNW_OK;
 }
 
@@ -1386,22 +1479,15 @@ int render_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam
     if (a.chunks > 1) {
         if (ctx->fixed_words < plane) {
             CUDA_TRY(cudaStreamSynchronize(st));
-            if (ctx->fixed) cudaFree(ctx->fixed);
-            ctx->fixed = nullptr;
-            ctx->fixed_words = 0;
-            if (cudaMalloc(&ctx->fixed, plane * sizeof(unsigned long long)) != cudaSuccess) {
-                cudaGetLastError();
-                return fail(RTNW_ERR_NOMEM, "cudaMalloc of the sample-range accumulation plane failed");
-            }
-            ctx->fixed_words = plane;
+            rc = grow(&ctx->fixed, &ctx->fixed_words, plane, "cudaMalloc of the sample-range accumulation plane failed");
+            if (rc != RTNW_OK) return rc;
             CUDA_TRY(cudaMemsetAsync(ctx->fixed, 0, plane * sizeof(unsigned long long), st));  // k_finish_fixed keeps it zero afterwards
         }
         a.fixed = ctx->fixed;
     }
     CUDA_TRY(cudaMemsetAsync(ctx->ctr, 0, 8 * sizeof(unsigned long long), st));
     CUDA_TRY(cudaEventRecord(ctx->ev0, st));
-    if (p->flags & RTNW_F_FAST_BVH) rc = (p->flags & RTNW_F_COUNTERS) ? launch_render<true, true>(ctx, a, st) : launch_render<false, true>(ctx, a, st);
-    else rc = (p->flags & RTNW_F_COUNTERS) ? launch_render<true, false>(ctx, a, st) : launch_render<false, false>(ctx, a, st);
+    rc = by_variant(p->flags, [&](auto count, auto fast) { return launch_render<decltype(count)::value, decltype(fast)::value>(ctx, a, st); });
     if (rc != RTNW_OK) return rc;
     if (a.chunks > 1) {
         k_finish_fixed<<<(a.p.pixel_count + 255) / 256, 256, 0, st>>>(a.fixed, a.p.pixel_begin, a.p.pixel_stride, a.p.pixel_count,
@@ -1454,19 +1540,17 @@ int render_finish(rtnw_ctx* ctx, const render_ticket& t, rtnw_stats* stats) {
         cudaMemcpyToSymbol(g_round_stats, z, sizeof z);
     }
 #endif
+    const int rc = check_task_stack(ctx);
+    if (rc != RTNW_OK || !stats) return rc;
     const unsigned long long* h = ctx->ctr_host;
-    if (h[4]) return fail(RTNW_ERR_UNSUPPORTED, "BVH task stack overflow: the tree is deeper than RTNW_QN/RTNW_BLOCK - 1 levels");
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        stats->paths = paths_of(t.p);
-        stats->rays = h[1];
-        stats->box_tests = h[2];
-        stats->prim_tests = h[3];
-        CUDA_TRY(cudaEventElapsedTime(&stats->kernel_ms, ctx->ev0, ctx->ev1));
-        stats->kernel_launches = t.chunks > 1 ? 2 : 1;
-        stats->sample_ranges = t.chunks;
-    }
-    return RTNW_OK;
+    rtnw_stats s = {};
+    s.paths = paths_of(t.p);
+    s.rays = h[1];
+    s.box_tests = h[2];
+    s.prim_tests = h[3];
+    s.kernel_launches = t.chunks > 1 ? 2 : 1;
+    s.sample_ranges = t.chunks;
+    return report_stats(ctx, stats, s, false);
 }
 
 // render into a device buffer on stream st, synchronously
@@ -1562,13 +1646,14 @@ int rtnw_measure_fp32_peak(rtnw_ctx* ctx, float* tflops) {
     int rc = check_ctx(ctx);
     if (rc != RTNW_OK) return rc;
     if (!tflops) return fail(RTNW_ERR_INVALID, "null argument");
-    dev_buf d;
-    CUDA_TRY(d.alloc(sizeof(float)));
+    staging g;
+    const int sink = g.add(sizeof(float));
+    CUDA_TRY(g.copy_in(ctx->stream));
     const int iters = 1 << 14, blocks = ctx->sm_count * 32;
     float best = 0.f;
     for (int rep = 0; rep < 4; ++rep) {  // first repetition warms the clocks up
         CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
-        k_fma_peak<<<blocks, 256, 0, ctx->stream>>>(d.as<float>(), iters);
+        k_fma_peak<<<blocks, 256, 0, ctx->stream>>>(g.at<float>(sink), iters);
         CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));
         float ms = 0.f;
@@ -1584,13 +1669,13 @@ int rtnw_selftest_recip(rtnw_ctx* ctx, uint64_t n, uint32_t seed, uint64_t out[6
     int rc = check_ctx(ctx);
     if (rc != RTNW_OK) return rc;
     if (!out) return fail(RTNW_ERR_INVALID, "null argument");
-    dev_buf d;
-    CUDA_TRY(d.alloc(6 * sizeof(unsigned long long)));
-    CUDA_TRY(cudaMemsetAsync(d.p, 0, 6 * sizeof(unsigned long long), ctx->stream));
-    k_selftest_recip<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(n, seed, d.as<unsigned long long>());
+    staging g;
+    const int counts = g.add(6 * sizeof(unsigned long long), nullptr, out);
+    CUDA_TRY(g.copy_in(ctx->stream));
+    CUDA_TRY(cudaMemsetAsync(g.at<void>(counts), 0, 6 * sizeof(unsigned long long), ctx->stream));
+    k_selftest_recip<<<ctx->sm_count * 8, 256, 0, ctx->stream>>>(n, seed, g.at<unsigned long long>(counts));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(out, d.p, 6 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -1613,11 +1698,12 @@ int64_t rtnw_scene_inspect(const rtnw_scene_desc* desc, int32_t table, void* buf
 
 // The device image of a scene, built once on the host (no device needed): one slab with every table at a 256-byte
 // aligned offset, in pinned memory when a CUDA driver is present (so an upload is a single asynchronous DMA).
+enum prepared_table { T_RECS, T_LEAF, T_RXF, T_NODES, T_GATES, T_XF, T_MAT, T_TEX, T_RV, T_PERM, T_IMG, N_TABLES };
 struct rtnw_prepared {
     uint8_t* host = nullptr;
     bool pinned = false;
     size_t bytes = 0;
-    size_t o_recs = 0, o_leaf = 0, o_rxf = 0, o_nodes = 0, o_gates = 0, o_xf = 0, o_mat = 0, o_tex = 0, o_rv = 0, o_perm = 0, o_img = 0;
+    size_t off[N_TABLES] = {};  // byte offset of each table in the slab
     int32_t n_recs = 0, n_materials = 0, n_textures = 0, n_wnodes = 0, fast_node_base = 0;
 };
 
@@ -1645,42 +1731,24 @@ int rtnw_scene_prepare(const rtnw_scene_desc* desc, rtnw_prepared** out) {
         perm[i] = (uint8_t)px; perm[256 + i] = (uint8_t)py; perm[512 + i] = (uint8_t)pz;
     }
 
-    // one slab, every table 256-byte aligned
+    // one slab, every table 256-byte aligned; the image table has 16 bytes of slack after the pool
+    const void* src[N_TABLES] = {sb.recs.data(), sb.leaf.data(), sb.rec_xf.data(), sb.wnodes.data(), sb.gate_leaves.data(),
+                                 desc->xforms, desc->materials, desc->textures, ranvec.data(), perm.data(), desc->images};
+    const size_t sz[N_TABLES] = {sb.recs.size() * sizeof(rec), sb.leaf.size() * sizeof(int32_t), sb.rec_xf.size() * sizeof(uint32_t),
+                                 sb.wnodes.size() * sizeof(float4), sb.gate_leaves.size() * sizeof(int2),
+                                 (size_t)desc->n_xform_ops * sizeof(rtnw_xform_op), (size_t)desc->n_materials * sizeof(rtnw_material),
+                                 (size_t)desc->n_textures * sizeof(rtnw_texture), 256 * sizeof(float4), 768, (size_t)desc->image_bytes + 16};
     rtnw_prepared* P = new rtnw_prepared();
-    const size_t sz_recs = sb.recs.size() * sizeof(rec), sz_leaf = sb.leaf.size() * sizeof(int32_t);
-    const size_t sz_xf = (size_t)desc->n_xform_ops * sizeof(rtnw_xform_op);
-    const size_t sz_mat = (size_t)desc->n_materials * sizeof(rtnw_material), sz_tex = (size_t)desc->n_textures * sizeof(rtnw_texture);
-    const size_t sz_img = (size_t)desc->image_bytes, sz_rv = 256 * sizeof(float4), sz_perm = 768;
-    const size_t sz_nodes = sb.wnodes.size() * sizeof(float4), sz_gates = sb.gate_leaves.size() * sizeof(int2);
-    size_t off = 0;
-    P->o_recs = off; off += align256(sz_recs);
-    P->o_leaf = off; off += align256(sz_leaf);
-    P->o_rxf = off; off += align256(sz_leaf);
-    P->o_nodes = off; off += align256(sz_nodes);
-    P->o_gates = off; off += align256(sz_gates);
-    P->o_xf = off; off += align256(sz_xf);
-    P->o_mat = off; off += align256(sz_mat);
-    P->o_tex = off; off += align256(sz_tex);
-    P->o_rv = off; off += align256(sz_rv);
-    P->o_perm = off; off += align256(sz_perm);
-    P->o_img = off; off += align256(sz_img + 16);
-    P->bytes = off;
+    P->bytes = layout256(sz, N_TABLES, P->off);
     void* pin = nullptr;
-    if (cudaHostAlloc(&pin, off, cudaHostAllocDefault) == cudaSuccess) { P->host = static_cast<uint8_t*>(pin); P->pinned = true; }
-    else { cudaGetLastError(); P->host = static_cast<uint8_t*>(std::malloc(off)); }
+    if (cudaHostAlloc(&pin, P->bytes, cudaHostAllocDefault) == cudaSuccess) { P->host = static_cast<uint8_t*>(pin); P->pinned = true; }
+    else { cudaGetLastError(); P->host = static_cast<uint8_t*>(std::malloc(P->bytes)); }
     if (!P->host) { delete P; return fail(RTNW_ERR_NOMEM, "cannot allocate the host image of the scene"); }
-    std::memset(P->host, 0, off);
-    std::memcpy(P->host + P->o_recs, sb.recs.data(), sz_recs);
-    std::memcpy(P->host + P->o_leaf, sb.leaf.data(), sz_leaf);
-    std::memcpy(P->host + P->o_rxf, sb.rec_xf.data(), sz_leaf);
-    std::memcpy(P->host + P->o_nodes, sb.wnodes.data(), sz_nodes);
-    std::memcpy(P->host + P->o_gates, sb.gate_leaves.data(), sz_gates);
-    std::memcpy(P->host + P->o_xf, desc->xforms, sz_xf);
-    if (sz_mat) std::memcpy(P->host + P->o_mat, desc->materials, sz_mat);
-    if (sz_tex) std::memcpy(P->host + P->o_tex, desc->textures, sz_tex);
-    std::memcpy(P->host + P->o_rv, ranvec.data(), sz_rv);
-    std::memcpy(P->host + P->o_perm, perm.data(), sz_perm);
-    if (sz_img) std::memcpy(P->host + P->o_img, desc->images, sz_img);
+    std::memset(P->host, 0, P->bytes);
+    for (int t = 0; t < N_TABLES; ++t) {
+        const size_t bytes = t == T_IMG ? (size_t)desc->image_bytes : sz[t];
+        if (bytes) std::memcpy(P->host + P->off[t], src[t], bytes);
+    }
     P->n_recs = (int32_t)sb.recs.size();
     P->n_wnodes = (int32_t)(sb.wnodes.size() / 8);
     P->fast_node_base = sb.fast_base;
@@ -1721,17 +1789,18 @@ int rtnw_scene_upload_prepared(rtnw_ctx* ctx, const rtnw_prepared* P, rtnw_scene
         return fail(e == cudaErrorMemoryAllocation ? RTNW_ERR_NOMEM : RTNW_ERR_CUDA, std::string("scene upload: ") + cudaGetErrorString(e));
     }
     uint8_t* base = static_cast<uint8_t*>(s->slab);
-    s->view.recs = reinterpret_cast<const rec*>(base + P->o_recs);
-    s->view.rec_leaf = reinterpret_cast<const int32_t*>(base + P->o_leaf);
-    s->view.rec_xf = reinterpret_cast<const uint32_t*>(base + P->o_rxf);
-    s->view.wnodes = reinterpret_cast<const float4*>(base + P->o_nodes);
-    s->view.gates = reinterpret_cast<const int2*>(base + P->o_gates);
-    s->view.xforms = reinterpret_cast<const rtnw_xform_op*>(base + P->o_xf);
-    s->view.materials = reinterpret_cast<const rtnw_material*>(base + P->o_mat);
-    s->view.textures = reinterpret_cast<const rtnw_texture*>(base + P->o_tex);
-    s->view.ranvec = reinterpret_cast<const float4*>(base + P->o_rv);
-    s->view.perm = base + P->o_perm;
-    s->view.images = base + P->o_img;
+    const size_t* o = P->off;
+    s->view.recs = reinterpret_cast<const rec*>(base + o[T_RECS]);
+    s->view.rec_leaf = reinterpret_cast<const int32_t*>(base + o[T_LEAF]);
+    s->view.rec_xf = reinterpret_cast<const uint32_t*>(base + o[T_RXF]);
+    s->view.wnodes = reinterpret_cast<const float4*>(base + o[T_NODES]);
+    s->view.gates = reinterpret_cast<const int2*>(base + o[T_GATES]);
+    s->view.xforms = reinterpret_cast<const rtnw_xform_op*>(base + o[T_XF]);
+    s->view.materials = reinterpret_cast<const rtnw_material*>(base + o[T_MAT]);
+    s->view.textures = reinterpret_cast<const rtnw_texture*>(base + o[T_TEX]);
+    s->view.ranvec = reinterpret_cast<const float4*>(base + o[T_RV]);
+    s->view.perm = base + o[T_PERM];
+    s->view.images = base + o[T_IMG];
     s->view.n_recs = P->n_recs;
     s->view.n_wnodes = P->n_wnodes;
     s->view.fast_node_base = P->fast_node_base;
@@ -1789,16 +1858,7 @@ int rtnw_render(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam, 
     if (params->pixel_count != 0 || (params->flags & RTNW_F_ACCUMULATE))
         return fail(RTNW_ERR_INVALID, "pixel subsets / RTNW_F_ACCUMULATE need rtnw_render_device (the host entry point returns whole images)");
     const size_t floats = (size_t)params->nx * params->ny * 3;
-    if (ctx->accum_floats < floats) {
-        if (ctx->accum) cudaFree(ctx->accum);
-        ctx->accum = nullptr;
-        ctx->accum_floats = 0;
-        if (cudaMalloc(&ctx->accum, floats * sizeof(float)) != cudaSuccess) {
-            cudaGetLastError();
-            return fail(RTNW_ERR_NOMEM, "cannot allocate the accumulation buffer");
-        }
-        ctx->accum_floats = floats;
-    }
+    if ((rc = grow(&ctx->accum, &ctx->accum_floats, floats, "cannot allocate the accumulation buffer")) != RTNW_OK) return rc;
     CUDA_TRY(cudaEventRecord(ctx->ev_t0, ctx->stream));
     rc = render_core(ctx, scene, cam, params, ctx->accum, ctx->stream, stats);
     if (rc != RTNW_OK) return rc;
@@ -1825,13 +1885,13 @@ int rtnw_quantize_device(rtnw_ctx* ctx, const float* accum_rgb_dev, int32_t nx, 
     if (rc != RTNW_OK) return rc;
     if (!accum_rgb_dev || !rgb_out || nx <= 0 || ny <= 0 || ns <= 0) return fail(RTNW_ERR_INVALID, "bad quantize arguments");
     const size_t n = (size_t)nx * ny;
-    dev_buf d_out;
-    CUDA_TRY(d_out.alloc(n * 3 * sizeof(int32_t)));
+    staging g;  // the input is the caller's device buffer
+    const int rgb = g.add(n * 3 * sizeof(int32_t), nullptr, rgb_out);
+    CUDA_TRY(g.copy_in(ctx->stream));
     const float inv_ns = (float)(1.0 / (double)(float)ns);
-    k_quantize<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(accum_rgb_dev, nx, ny, inv_ns, clamp255, d_out.as<int32_t>());
+    k_quantize<<<(unsigned)((n + 255) / 256), 256, 0, ctx->stream>>>(accum_rgb_dev, nx, ny, inv_ns, clamp255, g.at<int32_t>(rgb));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(rgb_out, d_out.p, n * 3 * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -1841,21 +1901,17 @@ int rtnw_trace(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_ray* rays, siz
     if (rc != RTNW_OK) return rc;
     if (!scene || (n && (!rays || !out))) return fail(RTNW_ERR_INVALID, "null argument");
     if (n == 0) return RTNW_OK;
-    dev_buf d_rays, d_out;
-    CUDA_TRY(d_rays.alloc(n * sizeof(rtnw_ray)));
-    CUDA_TRY(d_out.alloc(n * sizeof(rtnw_hit)));
-    CUDA_TRY(cudaMemcpyAsync(d_rays.p, rays, n * sizeof(rtnw_ray), cudaMemcpyHostToDevice, ctx->stream));
+    staging g;
+    const int in = g.add(n * sizeof(rtnw_ray), rays), hit = g.add(n * sizeof(rtnw_hit), nullptr, out);
+    CUDA_TRY(g.copy_in(ctx->stream));
     const unsigned grid = (unsigned)((n + RTNW_BLOCK - 1) / RTNW_BLOCK);
-    if (flags & RTNW_F_FAST_BVH) {
-        CUDA_TRY(cudaFuncSetAttribute(k_trace<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(block_smem<true>)));
-        k_trace<true><<<grid, RTNW_BLOCK, sizeof(block_smem<true>), ctx->stream>>>(scene->view, d_rays.as<rtnw_ray>(), n, t_min, t_max, seed, d_out.as<rtnw_hit>());
-    } else {
-        CUDA_TRY(cudaFuncSetAttribute(k_trace<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(block_smem<false>)));
-        k_trace<false><<<grid, RTNW_BLOCK, sizeof(block_smem<false>), ctx->stream>>>(scene->view, d_rays.as<rtnw_ray>(), n, t_min, t_max, seed, d_out.as<rtnw_hit>());
-    }
-    CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(out, d_out.p, n * sizeof(rtnw_hit), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    rc = by_variant(flags, [&](auto, auto fast) {
+        constexpr bool FAST = decltype(fast)::value;
+        return launch_coop<block_smem<FAST>>(k_trace<FAST>, grid, ctx->stream, scene->view, g.at<const rtnw_ray>(in), n, t_min, t_max,
+                                             seed, g.at<rtnw_hit>(hit));
+    });
+    if (rc != RTNW_OK) return rc;
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -1869,49 +1925,38 @@ int rtnw_render_aov(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* c
     if (params->pixel_count != 0 || (params->flags & (RTNW_F_ACCUMULATE | RTNW_F_ROTATE_SAMPLES)))
         return fail(RTNW_ERR_INVALID, "rtnw_render_aov covers whole images: no pixel subset, RTNW_F_ACCUMULATE or RTNW_F_ROTATE_SAMPLES");
     const size_t n = (size_t)params->nx * params->ny;
-    dev_buf d;  // albedo | normal | depth | hits | prim_id
-    CUDA_TRY(d.alloc(n * 9 * sizeof(float)));
+    staging g;
+    const int albedo = g.add(n * 3 * sizeof(float), nullptr, out->albedo), normal = g.add(n * 3 * sizeof(float), nullptr, out->normal);
+    const int depth = g.add(n * sizeof(float), nullptr, out->depth), hits = g.add(n * sizeof(int32_t), nullptr, out->hits);
+    const int prim_id = g.add(n * sizeof(int32_t), nullptr, out->prim_id);
+    CUDA_TRY(g.copy_in(ctx->stream, ctx->ev_t0));
     aov_args a;
     a.S = scene->view;
     a.cam = *cam;
     a.p = *params;
-    a.albedo = d.as<float>();
-    a.normal = a.albedo + 3 * n;
-    a.depth = a.normal + 3 * n;
-    a.hits = reinterpret_cast<int32_t*>(a.depth + n);
-    a.prim_id = a.hits + n;
+    a.albedo = g.at<float>(albedo);
+    a.normal = g.at<float>(normal);
+    a.depth = g.at<float>(depth);
+    a.hits = g.at<int32_t>(hits);
+    a.prim_id = g.at<int32_t>(prim_id);
     a.ctr = ctx->ctr;
     const unsigned grid = (unsigned)((n + RTNW_BLOCK - 1) / RTNW_BLOCK);
-    CUDA_TRY(cudaEventRecord(ctx->ev_t0, ctx->stream));
     CUDA_TRY(cudaMemsetAsync(ctx->ctr, 0, 8 * sizeof(unsigned long long), ctx->stream));
     CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
-    if (params->flags & RTNW_F_FAST_BVH) {
-        CUDA_TRY(cudaFuncSetAttribute(k_aov<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(aov_smem<true>)));
-        k_aov<true><<<grid, RTNW_BLOCK, sizeof(aov_smem<true>), ctx->stream>>>(a);
-    } else {
-        CUDA_TRY(cudaFuncSetAttribute(k_aov<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(aov_smem<false>)));
-        k_aov<false><<<grid, RTNW_BLOCK, sizeof(aov_smem<false>), ctx->stream>>>(a);
-    }
-    CUDA_TRY(cudaGetLastError());
+    rc = by_variant(params->flags, [&](auto, auto fast) {
+        constexpr bool FAST = decltype(fast)::value;
+        return launch_coop<aov_smem<FAST>>(k_aov<FAST>, grid, ctx->stream, a);
+    });
+    if (rc != RTNW_OK) return rc;
     CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
     CUDA_TRY(cudaMemcpyAsync(ctx->ctr_host, ctx->ctr, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out->albedo, a.albedo, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out->normal, a.normal, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out->depth, a.depth, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out->hits, a.hits, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out->prim_id, a.prim_id, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev_t1, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    if (ctx->ctr_host[4]) return fail(RTNW_ERR_UNSUPPORTED, "BVH task stack overflow: the tree is deeper than RTNW_QN/RTNW_BLOCK - 1 levels");
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        stats->paths = stats->rays = (uint64_t)n * params->sample_count;
-        CUDA_TRY(cudaEventElapsedTime(&stats->kernel_ms, ctx->ev0, ctx->ev1));
-        CUDA_TRY(cudaEventElapsedTime(&stats->total_ms, ctx->ev_t0, ctx->ev_t1));
-        stats->kernel_launches = 1;
-        stats->sample_ranges = 1;
-    }
-    return RTNW_OK;
+    CUDA_TRY(g.copy_out(ctx->stream, ctx->ev_t1));
+    if ((rc = check_task_stack(ctx)) != RTNW_OK) return rc;
+    rtnw_stats s = {};
+    s.paths = s.rays = (uint64_t)n * params->sample_count;
+    s.kernel_launches = 1;
+    s.sample_ranges = 1;
+    return report_stats(ctx, stats, s, true);
 }
 
 int rtnw_eval_texture(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t tex_id, const float* uvp, size_t n, float* rgb_out) {
@@ -1920,14 +1965,12 @@ int rtnw_eval_texture(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t tex_id, co
     if (!scene || (n && (!uvp || !rgb_out))) return fail(RTNW_ERR_INVALID, "null argument");
     if (tex_id < 0 || tex_id >= scene->view.n_textures) return fail(RTNW_ERR_INVALID, "texture index out of range");
     if (n == 0) return RTNW_OK;
-    dev_buf d_in, d_out;
-    CUDA_TRY(d_in.alloc(n * 5 * sizeof(float)));
-    CUDA_TRY(d_out.alloc(n * 3 * sizeof(float)));
-    CUDA_TRY(cudaMemcpyAsync(d_in.p, uvp, n * 5 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    k_eval_texture<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(scene->view, tex_id, d_in.as<float>(), n, d_out.as<float>());
+    staging g;
+    const int in = g.add(n * 5 * sizeof(float), uvp), rgb = g.add(n * 3 * sizeof(float), nullptr, rgb_out);
+    CUDA_TRY(g.copy_in(ctx->stream));
+    k_eval_texture<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(scene->view, tex_id, g.at<float>(in), n, g.at<float>(rgb));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(rgb_out, d_out.p, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -1943,34 +1986,24 @@ int rtnw_denoise(rtnw_ctx* ctx, const float* color_sums, const rtnw_aov* feature
     if (!(dp->sigma_luminance > 0.f) || !std::isfinite(dp->sigma_luminance) || !(dp->sigma_depth > 0.f) || !std::isfinite(dp->sigma_depth))
         return fail(RTNW_ERR_INVALID, "sigmas must be finite and > 0");
     const size_t n = (size_t)nx * ny;
-    // color (the output after k_dn_prepare) | albedo | normal | depth | hits | ev[0] | ev[1] | feat | grad | hit, 256-B aligned
-    const size_t sz[10] = {12 * n, 12 * n, 12 * n, 4 * n, 4 * n, 16 * n, 16 * n, 16 * n, 8 * n, n};
-    size_t off[10], total = 0;
-    for (int b = 0; b < 10; ++b) { off[b] = total; total += align256(sz[b]); }
-    dev_buf d;
-    CUDA_TRY(d.alloc(total));
-    unsigned char* base = d.as<unsigned char>();
+    staging g;  // 101 bytes per pixel; the colour span is overwritten with the output
+    const int color = g.add(12 * n, color_sums, rgb_out), albedo = g.add(12 * n, features->albedo), normal = g.add(12 * n, features->normal);
+    const int depth = g.add(4 * n, features->depth), hits = g.add(4 * n, features->hits);
+    const int ev0 = g.add(16 * n), ev1 = g.add(16 * n), feat = g.add(16 * n), grad = g.add(8 * n), hit = g.add(n);
+    CUDA_TRY(g.copy_in(ctx->stream, ctx->ev_t0));
     dn_args a;
     a.nx = nx; a.ny = ny; a.k = dp->normal_power_log2;
     a.fns = (float)ns; a.sigma_l = dp->sigma_luminance; a.sigma_z = dp->sigma_depth;
-    float* color = reinterpret_cast<float*>(base + off[0]);
-    a.color = color;
-    a.albedo = reinterpret_cast<float*>(base + off[1]);
-    a.normal = reinterpret_cast<float*>(base + off[2]);
-    a.depth = reinterpret_cast<float*>(base + off[3]);
-    a.hits = reinterpret_cast<int32_t*>(base + off[4]);
-    a.ev[0] = reinterpret_cast<float4*>(base + off[5]);
-    a.ev[1] = reinterpret_cast<float4*>(base + off[6]);
-    a.feat = reinterpret_cast<float4*>(base + off[7]);
-    a.grad = reinterpret_cast<float2*>(base + off[8]);
-    a.hit = base + off[9];
-    a.out = color;
-    CUDA_TRY(cudaEventRecord(ctx->ev_t0, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(color, color_sums, sz[0], cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(base + off[1], features->albedo, sz[1], cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(base + off[2], features->normal, sz[2], cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(base + off[3], features->depth, sz[3], cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(base + off[4], features->hits, sz[4], cudaMemcpyHostToDevice, ctx->stream));
+    a.color = a.out = g.at<float>(color);
+    a.albedo = g.at<float>(albedo);
+    a.normal = g.at<float>(normal);
+    a.depth = g.at<float>(depth);
+    a.hits = g.at<int32_t>(hits);
+    a.ev[0] = g.at<float4>(ev0);
+    a.ev[1] = g.at<float4>(ev1);
+    a.feat = g.at<float4>(feat);
+    a.grad = g.at<float2>(grad);
+    a.hit = g.at<unsigned char>(hit);
     const dim3 block(DN_BX, DN_BY), grid((unsigned)((nx + DN_BX - 1) / DN_BX), (unsigned)((ny + DN_BY - 1) / DN_BY));
     CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
     k_dn_prepare<<<grid, block, 0, ctx->stream>>>(a);
@@ -1979,16 +2012,10 @@ int rtnw_denoise(rtnw_ctx* ctx, const float* color_sums, const rtnw_aov* feature
         k_dn_atrous<<<grid, block, 0, ctx->stream>>>(a, it, it % 2 == 0 ? 1 : 0, it == dp->iterations - 1);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(rgb_out, color, sz[0], cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev_t1, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
-    if (stats) {
-        std::memset(stats, 0, sizeof *stats);
-        CUDA_TRY(cudaEventElapsedTime(&stats->kernel_ms, ctx->ev0, ctx->ev1));
-        CUDA_TRY(cudaEventElapsedTime(&stats->total_ms, ctx->ev_t0, ctx->ev_t1));
-        stats->kernel_launches = dp->iterations + 2;
-    }
-    return RTNW_OK;
+    CUDA_TRY(g.copy_out(ctx->stream, ctx->ev_t1));
+    rtnw_stats s = {};
+    s.kernel_launches = dp->iterations + 2;
+    return report_stats(ctx, stats, s, true);
 }
 
 int rtnw_eval_perlin(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t which, const float* xyz, size_t n, float* out) {
@@ -1997,14 +2024,12 @@ int rtnw_eval_perlin(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t which, cons
     if (!scene || (n && (!xyz || !out))) return fail(RTNW_ERR_INVALID, "null argument");
     if (which != 0 && which != 1) return fail(RTNW_ERR_INVALID, "which must be 0 (noise) or 1 (turb)");
     if (n == 0) return RTNW_OK;
-    dev_buf d_in, d_out;
-    CUDA_TRY(d_in.alloc(n * 3 * sizeof(float)));
-    CUDA_TRY(d_out.alloc(n * sizeof(float)));
-    CUDA_TRY(cudaMemcpyAsync(d_in.p, xyz, n * 3 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    k_eval_perlin<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(scene->view, which, d_in.as<float>(), n, d_out.as<float>());
+    staging g;
+    const int in = g.add(n * 3 * sizeof(float), xyz), val = g.add(n * sizeof(float), nullptr, out);
+    CUDA_TRY(g.copy_in(ctx->stream));
+    k_eval_perlin<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(scene->view, which, g.at<float>(in), n, g.at<float>(val));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(out, d_out.p, n * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -2017,24 +2042,16 @@ int rtnw_scatter(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_ray* rays_in
     for (size_t i = 0; i < n; ++i)
         if (hits[i].mat_id < 0 || hits[i].mat_id >= scene->view.n_materials) return fail(RTNW_ERR_INVALID, "hit.mat_id out of range");
     if (n == 0) return RTNW_OK;
-    dev_buf d_rays, d_hits, d_sc, d_att, d_em, d_flag;
-    CUDA_TRY(d_rays.alloc(n * sizeof(rtnw_ray)));
-    CUDA_TRY(d_hits.alloc(n * sizeof(rtnw_hit)));
-    CUDA_TRY(d_sc.alloc(n * sizeof(rtnw_ray)));
-    CUDA_TRY(d_att.alloc(n * 3 * sizeof(float)));
-    CUDA_TRY(d_em.alloc(n * 3 * sizeof(float)));
-    CUDA_TRY(d_flag.alloc(n * sizeof(int32_t)));
-    CUDA_TRY(cudaMemcpyAsync(d_rays.p, rays_in, n * sizeof(rtnw_ray), cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(d_hits.p, hits, n * sizeof(rtnw_hit), cudaMemcpyHostToDevice, ctx->stream));
-    k_scatter<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(scene->view, d_rays.as<rtnw_ray>(), d_hits.as<rtnw_hit>(), n, seed,
-                                                                    d_sc.as<rtnw_ray>(), d_att.as<float>(), d_em.as<float>(),
-                                                                    d_flag.as<int32_t>());
+    staging g;
+    const int rays = g.add(n * sizeof(rtnw_ray), rays_in), hit = g.add(n * sizeof(rtnw_hit), hits);
+    const int sc = g.add(n * sizeof(rtnw_ray), nullptr, out_scattered), att = g.add(n * 3 * sizeof(float), nullptr, out_atten);
+    const int em = g.add(n * 3 * sizeof(float), nullptr, out_emitted), flag = g.add(n * sizeof(int32_t), nullptr, out_flag);
+    CUDA_TRY(g.copy_in(ctx->stream));
+    k_scatter<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(scene->view, g.at<rtnw_ray>(rays), g.at<rtnw_hit>(hit), n, seed,
+                                                                    g.at<rtnw_ray>(sc), g.at<float>(att), g.at<float>(em),
+                                                                    g.at<int32_t>(flag));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(out_scattered, d_sc.p, n * sizeof(rtnw_ray), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_atten, d_att.p, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_emitted, d_em.p, n * 3 * sizeof(float), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(out_flag, d_flag.p, n * sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -2044,17 +2061,13 @@ int rtnw_camera_rays(rtnw_ctx* ctx, const rtnw_camera* cam, int32_t nx, int32_t 
     if (rc != RTNW_OK) return rc;
     if (!cam || nx <= 0 || ny <= 0 || (n && (!ij || !sample || !rays_out))) return fail(RTNW_ERR_INVALID, "bad argument");
     if (n == 0) return RTNW_OK;
-    dev_buf d_ij, d_s, d_out;
-    CUDA_TRY(d_ij.alloc(n * 2 * sizeof(int32_t)));
-    CUDA_TRY(d_s.alloc(n * sizeof(int32_t)));
-    CUDA_TRY(d_out.alloc(n * sizeof(rtnw_ray)));
-    CUDA_TRY(cudaMemcpyAsync(d_ij.p, ij, n * 2 * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(d_s.p, sample, n * sizeof(int32_t), cudaMemcpyHostToDevice, ctx->stream));
-    k_camera_rays<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(*cam, nx, ny, d_ij.as<int32_t>(), d_s.as<int32_t>(), n, seed,
-                                                                        d_out.as<rtnw_ray>());
+    staging g;
+    const int pix = g.add(n * 2 * sizeof(int32_t), ij), smp = g.add(n * sizeof(int32_t), sample), ray = g.add(n * sizeof(rtnw_ray), nullptr, rays_out);
+    CUDA_TRY(g.copy_in(ctx->stream));
+    k_camera_rays<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(*cam, nx, ny, g.at<int32_t>(pix), g.at<int32_t>(smp), n, seed,
+                                                                        g.at<rtnw_ray>(ray));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(rays_out, d_out.p, n * sizeof(rtnw_ray), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -2064,14 +2077,12 @@ int rtnw_camera_get_rays(rtnw_ctx* ctx, const rtnw_camera* cam, const float* st,
     if (rc != RTNW_OK) return rc;
     if (!cam || (n && (!st || !rays_out))) return fail(RTNW_ERR_INVALID, "bad argument");
     if (n == 0) return RTNW_OK;
-    dev_buf d_st, d_out;
-    CUDA_TRY(d_st.alloc(n * 2 * sizeof(float)));
-    CUDA_TRY(d_out.alloc(n * sizeof(rtnw_ray)));
-    CUDA_TRY(cudaMemcpyAsync(d_st.p, st, n * 2 * sizeof(float), cudaMemcpyHostToDevice, ctx->stream));
-    k_camera_get_rays<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(*cam, d_st.as<float>(), n, seed, key_base, d_out.as<rtnw_ray>());
+    staging g;
+    const int in = g.add(n * 2 * sizeof(float), st), ray = g.add(n * sizeof(rtnw_ray), nullptr, rays_out);
+    CUDA_TRY(g.copy_in(ctx->stream));
+    k_camera_get_rays<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(*cam, g.at<float>(in), n, seed, key_base, g.at<rtnw_ray>(ray));
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(rays_out, d_out.p, n * sizeof(rtnw_ray), cudaMemcpyDeviceToHost, ctx->stream));
-    CUDA_TRY(cudaStreamSynchronize(ctx->stream));
+    CUDA_TRY(g.copy_out(ctx->stream));
     return RTNW_OK;
 }
 
@@ -2080,7 +2091,7 @@ struct rtnw_multi {
     int n = 0;
     rtnw_ctx* ctx[RTNW_MAX_DEVICES] = {};
     float* accum[RTNW_MAX_DEVICES] = {};   // per device: nx*ny*3 sums of its share of the samples
-    size_t accum_floats = 0;
+    size_t accum_floats[RTNW_MAX_DEVICES] = {};
     cudaEvent_t done[RTNW_MAX_DEVICES] = {};
     bool peer[RTNW_MAX_DEVICES] = {};      // device 0 reads this rank's buffer directly (same device, or P2P over NVLink)
     float* stage = nullptr;                // device 0: copies of the buffers it cannot read directly
@@ -2175,21 +2186,14 @@ int rtnw_render_multi(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_came
     const size_t floats = (size_t)params->nx * params->ny * 3;
     int need_stage = 0;
     for (int d = 1; d < n; ++d) need_stage += m->peer[d] ? 0 : 1;
-    if (m->accum_floats < floats || (need_stage && m->stage_floats < floats * need_stage)) {
-        for (int d = 0; d < n; ++d) {
-            CUDA_TRY(cudaSetDevice(m->ctx[d]->device));
-            if (m->accum[d]) cudaFree(m->accum[d]);
-            m->accum[d] = nullptr;
-            if (cudaMalloc(&m->accum[d], floats * sizeof(float)) != cudaSuccess) { cudaGetLastError(); m->accum_floats = 0; return fail(RTNW_ERR_NOMEM, "cannot allocate the per-device accumulation buffers"); }
-        }
-        m->accum_floats = floats;
-        if (need_stage) {
-            CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
-            if (m->stage) cudaFree(m->stage);
-            m->stage = nullptr;
-            if (cudaMalloc(&m->stage, floats * need_stage * sizeof(float)) != cudaSuccess) { cudaGetLastError(); m->stage_floats = 0; return fail(RTNW_ERR_NOMEM, "cannot allocate the staging planes"); }
-            m->stage_floats = floats * need_stage;
-        }
+    for (int d = 0; d < n; ++d) {
+        CUDA_TRY(cudaSetDevice(m->ctx[d]->device));
+        rc = grow(&m->accum[d], &m->accum_floats[d], floats, "cannot allocate the per-device accumulation buffers");
+        if (rc != RTNW_OK) return rc;
+    }
+    if (need_stage) {
+        CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
+        if ((rc = grow(&m->stage, &m->stage_floats, floats * need_stage, "cannot allocate the staging planes")) != RTNW_OK) return rc;
     }
     // every device renders its share of every pixel's samples (ownership rotates with the pixel index: even for any ns)
     render_ticket ticket[RTNW_MAX_DEVICES];
