@@ -322,6 +322,16 @@ typedef struct rtnw_aov {        /* host buffers, all required */
 int rtnw_render_aov(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam,
                     const rtnw_render_params* params, const rtnw_aov* out, rtnw_stats* stats);
 
+/* rtnw_render_aov into caller-owned DEVICE buffers (an rtnw_aov holding device pointers, all required, overwritten),
+ * stream-ordered on cuda_stream (NULL = the legacy default stream) and synchronous on return, like rtnw_render_device.
+ * Honours RTNW_F_ROTATE_SAMPLES with rtnw_render's meaning: sample_count is the frame's total ns, and pixel p sums its samples
+ * s = (sample_begin - p) mod sample_stride + k*sample_stride < ns in that order; prim_id is the leaf id of the first of them,
+ * -1 on a miss or when the pixel has no sample in this call (ns < sample_stride).  Rank g of G (sample_begin g, sample_stride
+ * G) holds sample 0 of the pixels p = g mod G, so its prim_id there is the whole frame's.  Still rejects a pixel subset and
+ * RTNW_F_ACCUMULATE.  stats: paths = rays = the samples traced, kernel_ms = total_ms = k_aov, kernel_launches = 1. */
+int rtnw_render_aov_device(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam, const rtnw_render_params* params,
+                           const rtnw_aov* out_dev, void* cuda_stream, rtnw_stats* stats);
+
 /* Feature-guided denoiser of a frame: spatial-only SVGF (Schied et al. 2017 without the temporal part), i.e. the edge-avoiding
  * a-trous wavelet filter of Dammertz et al. 2010 with a variance-guided luminance weight, on the GPU.  Inputs are the colour
  * sums of rtnw_render and the rtnw_aov sums of rtnw_render_aov for the same params (ns = their sample_count); prim_id is not
@@ -354,6 +364,13 @@ typedef struct rtnw_denoise_params {
 #define RTNW_DENOISE_DEFAULTS {5, 4.0f, 1.0f, 7}
 int rtnw_denoise(rtnw_ctx* ctx, const float* color_sums, const rtnw_aov* features, int32_t nx, int32_t ny, int32_t ns,
                  const rtnw_denoise_params* dp, float* rgb_out, rtnw_stats* stats);
+
+/* rtnw_denoise on DEVICE buffers (e.g. the ones rtnw_render_device and rtnw_render_aov_device filled): the same definition and
+ * the same bits, without the host copies.  Stream-ordered on cuda_stream (NULL = the legacy default stream), synchronous on
+ * return.  The scratch planes (57 bytes per pixel) belong to the context and grow on demand.  rgb_out_dev (nx*ny*3 floats)
+ * must not overlap an input (RTNW_ERR_INVALID).  stats as rtnw_denoise's, with total_ms = kernel_ms. */
+int rtnw_denoise_device(rtnw_ctx* ctx, const float* color_sums_dev, const rtnw_aov* features_dev, int32_t nx, int32_t ny,
+                        int32_t ns, const rtnw_denoise_params* dp, float* rgb_out_dev, void* cuda_stream, rtnw_stats* stats);
 
 /* texture::value(u,v,p) for n points; uvp = n x 5 floats {u,v,px,py,pz}; rgb_out = n x 3 (PSC/texture.h, surface_texture.h) */
 int rtnw_eval_texture(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t tex_id, const float* uvp, size_t n, float* rgb_out);
@@ -394,6 +411,20 @@ int rtnw_scene_free_multi(rtnw_multi* m, rtnw_multi_scene* scene);
  * stats: paths / rays / tests summed over the devices, kernel_ms = the slowest device, total_ms = launch to frame on the host. */
 int rtnw_render_multi(rtnw_multi* m, const rtnw_multi_scene* scene, const rtnw_camera* cam, const rtnw_render_params* params,
                       float* accum_rgb, rtnw_stats* stats);
+/* One frame with its first-hit feature buffers on the N GPUs of m.  Each device renders its colour share (as rtnw_render_multi)
+ * and then the AOVs of the same share (rtnw_render_aov_device with RTNW_F_ROTATE_SAMPLES, sample_begin = rank,
+ * sample_stride = N) on its stream.  Device 0 adds both in rank order: albedo, normal and depth as floats, hits as integers,
+ * prim_id taken from rank p mod N.  So hits and prim_id equal rtnw_render_aov's on one GPU, and the float planes differ from
+ * it by summation order only, as the colour does.  With dp != NULL device 0 then denoises the summed frame (rtnw_denoise).
+ * Host outputs, each optional (NULL = not copied), at least one given: accum_rgb (colour sums), aov (all five buffers),
+ * denoised_rgb (mean colour); denoised_rgb requires dp and dp requires denoised_rgb.  params restrictions as
+ * rtnw_render_multi.  Per device: 36 bytes per pixel of AOV planes, and on device 0 the denoiser's 57 bytes per pixel.
+ * stats: paths, rays, box_tests, prim_tests, kernel_ms and sample_ranges are the colour render's (as rtnw_render_multi);
+ * kernel_launches counts every launch (render, k_aov on each device, the two rank sums when N > 1, the denoiser's);
+ * total_ms runs from the first launch to the end of the last host copy. */
+int rtnw_render_aov_multi(rtnw_multi* m, const rtnw_multi_scene* scene, const rtnw_camera* cam, const rtnw_render_params* params,
+                          float* accum_rgb, const rtnw_aov* aov, const rtnw_denoise_params* dp, float* denoised_rgb,
+                          rtnw_stats* stats);
 
 #ifdef __cplusplus
 }

@@ -127,7 +127,8 @@ DEVICE_SYMBOLS = ["rtnw_last_error", "rtnw_abi_version", "rtnw_device_count", "r
                   "rtnw_eval_texture", "rtnw_eval_perlin", "rtnw_scatter", "rtnw_camera_rays", "rtnw_camera_get_rays", "rtnw_plan_sample_ranges",
                   "rtnw_scene_inspect", "rtnw_ctx_create_multi", "rtnw_ctx_destroy_multi", "rtnw_multi_device_count",
                   "rtnw_scene_upload_multi", "rtnw_scene_free_multi", "rtnw_render_multi", "rtnw_scene_prepare", "rtnw_prepared_bytes",
-                  "rtnw_scene_upload_prepared", "rtnw_prepared_free", "rtnw_render_aov", "rtnw_denoise"]
+                  "rtnw_scene_upload_prepared", "rtnw_prepared_free", "rtnw_render_aov", "rtnw_denoise", "rtnw_render_aov_device",
+                  "rtnw_denoise_device", "rtnw_render_aov_multi"]
 HOST_SYMBOLS = ["rtnw_host_last_error", "rtnw_host_scene_build", "rtnw_host_scene_free", "rtnw_host_scene_desc",
                 "rtnw_host_scene_leaf_count", "rtnw_host_scene_camera", "rtnw_host_scene_view", "rtnw_host_make_camera",
                 "rtnw_host_quantize", "rtnw_host_write_ppm", "rtnw_host_load_png", "rtnw_host_free_image", "rtnw_host_write_pfm"]
@@ -201,6 +202,10 @@ def device_lib() -> C.CDLL:
                                       C.POINTER(Stats)]
         L.rtnw_denoise.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Aov), C.c_int32, C.c_int32, C.c_int32, C.POINTER(DenoiseParams),
                                    C.c_void_p, C.POINTER(Stats)]
+        L.rtnw_render_aov_device.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams), C.POINTER(Aov),
+                                             C.c_void_p, C.POINTER(Stats)]
+        L.rtnw_denoise_device.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Aov), C.c_int32, C.c_int32, C.c_int32,
+                                          C.POINTER(DenoiseParams), C.c_void_p, C.c_void_p, C.POINTER(Stats)]
         L.rtnw_eval_texture.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]
         L.rtnw_eval_perlin.argtypes = [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_size_t, C.c_void_p]
         L.rtnw_scatter.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_uint64, C.c_void_p,
@@ -219,6 +224,8 @@ def device_lib() -> C.CDLL:
         L.rtnw_scene_upload_multi.argtypes = [C.c_void_p, C.POINTER(SceneDesc), C.POINTER(C.c_void_p)]
         L.rtnw_scene_free_multi.argtypes = [C.c_void_p, C.c_void_p]
         L.rtnw_render_multi.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams), C.c_void_p, C.POINTER(Stats)]
+        L.rtnw_render_aov_multi.argtypes = [C.c_void_p, C.c_void_p, C.POINTER(Camera), C.POINTER(RenderParams), C.c_void_p,
+                                            C.POINTER(Aov), C.POINTER(DenoiseParams), C.c_void_p, C.POINTER(Stats)]
         _dev = L
     return _dev
 
@@ -339,6 +346,17 @@ def plan_sample_ranges(params) -> np.ndarray:
     return np.array(cum[:n + 1], dtype=np.int64)
 
 
+AOV_KEYS = ("albedo", "normal", "depth", "hits", "prim_id")
+
+
+def _aov_arrays(params):
+    """host arrays for the five AOV buffers of a frame, and the rtnw_aov pointing at them"""
+    ny, nx = params.ny, params.nx
+    out = dict(albedo=np.empty((ny, nx, 3), np.float32), normal=np.empty((ny, nx, 3), np.float32),
+               depth=np.empty((ny, nx), np.float32), hits=np.empty((ny, nx), np.int32), prim_id=np.empty((ny, nx), np.int32))
+    return out, Aov(*(out[k].ctypes.data for k in AOV_KEYS))
+
+
 # ------------------------------------------------------------------------------------------------ device
 class Context:
     """One GPU + its stream (rtnw_ctx)."""
@@ -393,6 +411,20 @@ class Context:
         _check_dev(device_lib().rtnw_denoise(self._h, sums.ctypes.data, C.byref(feats), nx, ny, ns, C.byref(dp), out.ctypes.data,
                                              C.byref(st)))
         return out
+
+    def denoise_device(self, color_ptr: int, aov_ptrs: dict, nx: int, ny: int, ns: int, out_ptr: int, stream: int = 0,
+                       iterations: int = 5, sigma_luminance: float = 4.0, sigma_depth: float = 1.0, normal_power_log2: int = 7,
+                       stats: Stats | None = None) -> Stats:
+        """Context.denoise on device buffers (include/rtnw.h: rtnw_denoise_device), e.g. torch tensors' data_ptr(): the colour
+        sums at color_ptr, aov_ptrs["albedo" | "normal" | "depth" | "hits"] (a "prim_id" entry is ignored), the denoised mean
+        colour written to out_ptr (nx*ny*3 floats, not overlapping an input).  Ordered on `stream` (0 = the legacy default
+        stream); returns the call's Stats."""
+        feats = Aov(*(aov_ptrs[k] for k in ("albedo", "normal", "depth", "hits")), None)
+        dp = DenoiseParams(iterations, sigma_luminance, sigma_depth, normal_power_log2)
+        st = Stats() if stats is None else stats
+        _check_dev(device_lib().rtnw_denoise_device(self._h, C.c_void_p(color_ptr), C.byref(feats), nx, ny, ns, C.byref(dp),
+                                                    C.c_void_p(out_ptr), C.c_void_p(stream), C.byref(st)))
+        return st
 
     def close(self):
         if self._h:
@@ -475,13 +507,21 @@ class DeviceScene:
         rtnw_render_aov): dict of per-pixel SUMS albedo (ny,nx,3), normal (ny,nx,3), depth (ny,nx), and int32 hits (ny,nx) and
         prim_id (ny,nx), row j = 0 at the bottom.  Divide albedo by sample_count, normal and depth by hits.  Pass a Stats to
         receive the call's statistics."""
-        ny, nx = params.ny, params.nx
-        out = dict(albedo=np.empty((ny, nx, 3), np.float32), normal=np.empty((ny, nx, 3), np.float32),
-                   depth=np.empty((ny, nx), np.float32), hits=np.empty((ny, nx), np.int32), prim_id=np.empty((ny, nx), np.int32))
-        bufs = Aov(*(out[k].ctypes.data for k in ("albedo", "normal", "depth", "hits", "prim_id")))
+        out, bufs = _aov_arrays(params)
         st = Stats() if stats is None else stats
         _check_dev(device_lib().rtnw_render_aov(self.ctx._h, self._h, C.byref(cam), C.byref(params), C.byref(bufs), C.byref(st)))
         return out
+
+    def render_aov_device(self, cam: Camera, params: RenderParams, bufs: dict, stream: int = 0, stats: Stats | None = None) -> Stats:
+        """render_aov into caller-owned device memory (include/rtnw.h: rtnw_render_aov_device): bufs maps "albedo", "normal",
+        "depth", "hits" and "prim_id" to device pointers (e.g. torch tensors' data_ptr()) of the shapes render_aov returns.
+        Ordered on `stream` (0 = the legacy default stream).  Takes params.flags | F_ROTATE_SAMPLES for one rank's share of
+        a multi-GPU frame.  Returns the call's Stats."""
+        aov = Aov(*(bufs[k] for k in AOV_KEYS))
+        st = Stats() if stats is None else stats
+        _check_dev(device_lib().rtnw_render_aov_device(self.ctx._h, self._h, C.byref(cam), C.byref(params), C.byref(aov),
+                                                       C.c_void_p(stream), C.byref(st)))
+        return st
 
     # -- one world->hit() per ray, PSC/main.cpp:27
     def trace(self, rays: np.ndarray, t_min: float = 0.001, t_max: float = FLT_MAX, flags: int = 0, seed: int = 1) -> np.ndarray:
@@ -554,6 +594,19 @@ class MultiScene:
         st = Stats()
         _check_dev(device_lib().rtnw_render_multi(self.mctx._h, self._h, C.byref(cam), C.byref(params), out.ctypes.data, C.byref(st)))
         return out, st
+
+    def render_aov(self, cam: Camera, params: RenderParams, denoise: DenoiseParams | None = None):
+        """One frame and its first-hit feature buffers on every device of the handle (include/rtnw.h: rtnw_render_aov_multi),
+        denoised on the first device when `denoise` is given.  Returns (sums, aov, denoised or None, Stats) in the shapes of
+        DeviceScene.render, DeviceScene.render_aov and Context.denoise."""
+        sums = np.empty((params.ny, params.nx, 3), dtype=np.float32)
+        aov, bufs = _aov_arrays(params)
+        den = None if denoise is None else np.empty((params.ny, params.nx, 3), dtype=np.float32)
+        st = Stats()
+        _check_dev(device_lib().rtnw_render_aov_multi(self.mctx._h, self._h, C.byref(cam), C.byref(params), sums.ctypes.data,
+                                                      C.byref(bufs), None if denoise is None else C.byref(denoise),
+                                                      None if den is None else den.ctypes.data, C.byref(st)))
+        return sums, aov, den, st
 
     def close(self):
         if self._h and self.mctx._h:

@@ -311,6 +311,9 @@ struct aov_args {
 // First-hit feature buffers (rtnw_render_aov): one thread per pixel traces, for each of its samples, exactly the first ray
 // k_render traces for that (pixel, sample) — same stream, same camera_ray, same medium key at depth 0 — and sums what the
 // hit shows.  Every pixel has sample_count samples, so every thread of the block runs the same number of cooperative rounds.
+// ROT (RTNW_F_ROTATE_SAMPLES, a rank's share of a multi-GPU frame): pixel p has the samples (sample_begin - p) mod G + k*G
+// below sample_count, G = sample_stride, i.e. floor or ceil(sample_count / G) of them; every thread runs the ceil rounds and
+// sits out, still cooperating in the traversal, the rounds its pixel has no sample for.
 // The running sums of a pixel live in shared memory, as k_render's work items do: in registers they would be live across
 // the media's Philox call inside the traversal, and spill.
 template <bool FAST> struct aov_smem {
@@ -329,7 +332,7 @@ __device__ __noinline__ ray_t aov_camera_ray(const rtnw_camera& cam, int nx, int
     return r;
 }
 
-template <bool FAST>
+template <bool FAST, bool ROT>
 __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_args P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     typedef block_smem<FAST> SM;
@@ -340,6 +343,12 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_
     const int pix = blockIdx.x * blockDim.x + threadIdx.x;
     const bool active = pix < nx * ny;  // idle threads of the last block still work on the block's BVH tasks (with a ray below the image)
     const uint32_t k0 = (uint32_t)P.p.seed, k1 = (uint32_t)(P.p.seed >> 32);
+    int rounds = 0, s_begin = P.p.sample_begin;
+    if (ROT) {
+        const int g = P.p.sample_stride;
+        rounds = (P.p.sample_count + g - 1) / g;
+        s_begin = ((P.p.sample_begin - pix) % g + g) % g;
+    }
     trav_counters cnt;
     cnt.box_tests = 0; cnt.prim_tests = 0;
     coop_init<SM>(sm);
@@ -347,13 +356,17 @@ __global__ void __launch_bounds__(RTNW_BLOCK) k_aov(const __grid_constant__ aov_
     A.nrm[me] = make_float4(0.f, 0.f, 0.f, __int_as_float(0));
     __syncthreads();
     int r3 = 0;
-    for (int k = 0; k < P.p.sample_count; ++k) {
-        const int s = P.p.sample_begin + k * P.p.sample_stride;
+    for (int k = 0; k < (ROT ? rounds : P.p.sample_count); ++k) {
+        const int s = s_begin + k * P.p.sample_stride;
+        const bool on = ROT ? active && s < P.p.sample_count : active;
         const ray_t r = aov_camera_ray(P.cam, nx, ny, pix, s, P.p.seed);
         medium_key mk;
         mk.k0 = k0; mk.k1 = k1; mk.pixel = (uint32_t)pix; mk.sample = (uint32_t)s; mk.depth = 0;
-        const hkey_t key = coop_closest_hit<false, FAST, SM>(P.S, sm, r, active, P.p.t_min, P.p.t_max, mk, cnt, r3);
-        if (!active) continue;
+        const hkey_t key = coop_closest_hit<false, FAST, SM>(P.S, sm, r, on, P.p.t_min, P.p.t_max, mk, cnt, r3);
+        if (!on) {
+            if (ROT && active && k == 0) P.prim_id[pix] = -1;  // a pixel without a sample in this share (sample_count < G)
+            continue;
+        }
         hit_t h;
         key_to_hit(P.S, key, P.p.t_max, h);
         if (h.rec < 0) {
@@ -838,6 +851,30 @@ __global__ void k_sum_ranks(float* __restrict__ dst, const rank_planes P, size_t
     }
 }
 
+// rtnw_render_aov_multi: the ranks' AOV planes added into rank 0's on device 0, one thread per pixel.  Each rank's planes are
+// one buffer of 9 words per pixel (aov_planes): albedo and normal sums (3n each), depth sums (n), hits and prim_id (n int32
+// each).  The float sums are added in rank order, the hit counts as integers, and prim_id is rank p mod G's: the rank whose
+// share holds sample 0 of pixel p (RTNW_F_ROTATE_SAMPLES), so it is the one-GPU prim_id.  src[0] is dst and is not read.
+__global__ void k_sum_aov_ranks(float* __restrict__ dst, const rank_planes P, size_t pixels) {
+    const size_t stride = (size_t)gridDim.x * blockDim.x;
+    for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < pixels; q += stride) {
+        const size_t at[7] = {3 * q, 3 * q + 1, 3 * q + 2, 3 * pixels + 3 * q, 3 * pixels + 3 * q + 1, 3 * pixels + 3 * q + 2,
+                              6 * pixels + q};
+#pragma unroll
+        for (int c = 0; c < 7; ++c) {
+            float v = dst[at[c]];
+            for (int r = 1; r < P.n; ++r) v += P.src[r][at[c]];
+            dst[at[c]] = v;
+        }
+        const size_t hq = 7 * pixels + q, pq = 8 * pixels + q;
+        int h = __float_as_int(dst[hq]);
+        for (int r = 1; r < P.n; ++r) h += __float_as_int(P.src[r][hq]);
+        dst[hq] = __int_as_float(h);
+        const int owner = (int)(q % (size_t)P.n);
+        if (owner != 0) dst[pq] = P.src[owner][pq];
+    }
+}
+
 // ================================================================================================ host side
 namespace {
 
@@ -955,6 +992,8 @@ struct rtnw_ctx {
     size_t fixed_words = 0;
     unsigned long long* ctr = nullptr;       // 8 device counters
     unsigned long long* ctr_host = nullptr;  // their pinned host copy (filled asynchronously after every render)
+    unsigned char* dn_scratch = nullptr;     // the denoiser's planes for rtnw_denoise_device and rtnw_render_aov_multi
+    size_t dn_scratch_bytes = 0;
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;  // rtnw_render's total_ms
     int blocks_per_sm[4] = {0, 0, 0, 0};
     // freed scene slabs are kept for the next upload (cudaMalloc/cudaFree synchronise the device and can take
@@ -1365,9 +1404,10 @@ int check_ctx(rtnw_ctx* ctx) {
     return RTNW_OK;
 }
 
-// k_render and k_aov set counter 4 when a block's traversal task stack overflowed: the frame is then incomplete
-int check_task_stack(const rtnw_ctx* ctx) {
-    if (ctx->ctr_host[4]) return fail(RTNW_ERR_UNSUPPORTED, "BVH task stack overflow: the tree is deeper than RTNW_QN/RTNW_BLOCK - 1 levels");
+// k_render and k_aov set counter 4 when a block's traversal task stack overflowed: the frame is then incomplete.  `slot` is
+// where its host copy landed (aov_launch).
+int check_task_stack(const rtnw_ctx* ctx, int slot = 4) {
+    if (ctx->ctr_host[slot]) return fail(RTNW_ERR_UNSUPPORTED, "BVH task stack overflow: the tree is deeper than RTNW_QN/RTNW_BLOCK - 1 levels");
     return RTNW_OK;
 }
 
@@ -1562,6 +1602,111 @@ int render_core(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam, 
     return render_finish(ctx, t, stats);
 }
 
+// The AOV calls' restrictions on validated params: whole images, no RTNW_F_ACCUMULATE; RTNW_F_ROTATE_SAMPLES only if `rotate`
+int validate_aov_params(const rtnw_render_params* p, bool rotate, const char* msg) {
+    const uint32_t rejected = RTNW_F_ACCUMULATE | (rotate ? 0u : RTNW_F_ROTATE_SAMPLES);
+    if (p->pixel_count != 0 || (p->flags & rejected)) return fail(RTNW_ERR_INVALID, msg);
+    return RTNW_OK;
+}
+
+bool aov_complete(const rtnw_aov* a) { return a && a->albedo && a->normal && a->depth && a->hits && a->prim_id; }
+
+// The five planes of an rtnw_aov in one device buffer of 9 words per pixel (the per-device planes of rtnw_render_aov_multi)
+rtnw_aov aov_planes(float* base, size_t pixels) {
+    rtnw_aov v;
+    v.albedo = base;
+    v.normal = base + 3 * pixels;
+    v.depth = base + 6 * pixels;
+    v.hits = reinterpret_cast<int32_t*>(base + 7 * pixels);
+    v.prim_id = reinterpret_cast<int32_t*>(base + 8 * pixels);
+    return v;
+}
+
+// Queues k_aov for params p into the device planes `out` on stream st, between ctx->ev0 and ev1 when `timed`.  Its task-stack
+// overflow count reaches ctx->ctr_host[slot] when st gets there: slot 4 (check_task_stack's default) in the one-device calls,
+// 5 in rtnw_render_aov_multi, where the colour render queued before it on the same stream reports in slot 4 and owns the events.
+int aov_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam, const rtnw_render_params* p, const rtnw_aov& out,
+               cudaStream_t st, int slot, bool timed) {
+    aov_args a;
+    a.S = scene->view;
+    a.cam = *cam;
+    a.p = *p;
+    a.albedo = out.albedo;
+    a.normal = out.normal;
+    a.depth = out.depth;
+    a.hits = out.hits;
+    a.prim_id = out.prim_id;
+    a.ctr = ctx->ctr;
+    const unsigned grid = (unsigned)(((size_t)p->nx * p->ny + RTNW_BLOCK - 1) / RTNW_BLOCK);
+    CUDA_TRY(cudaMemsetAsync(ctx->ctr + 4, 0, sizeof(unsigned long long), st));
+    if (timed) CUDA_TRY(cudaEventRecord(ctx->ev0, st));
+    const bool rot = (p->flags & RTNW_F_ROTATE_SAMPLES) != 0;
+    const int rc = by_variant(p->flags, [&](auto, auto fast) {
+        constexpr bool FAST = decltype(fast)::value;
+        return rot ? launch_coop<aov_smem<FAST>>(k_aov<FAST, true>, grid, st, a) : launch_coop<aov_smem<FAST>>(k_aov<FAST, false>, grid, st, a);
+    });
+    if (rc != RTNW_OK) return rc;
+    if (timed) CUDA_TRY(cudaEventRecord(ctx->ev1, st));
+    CUDA_TRY(cudaMemcpyAsync(ctx->ctr_host + slot, ctx->ctr + 4, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    return RTNW_OK;
+}
+
+// paths = rays of an AOV call on the whole image (with RTNW_F_ROTATE_SAMPLES, the pixels' shares)
+uint64_t aov_rays(const rtnw_render_params& p) {
+    rtnw_render_params q = p;
+    q.pixel_begin = 0; q.pixel_stride = 1; q.pixel_count = p.nx * p.ny;
+    return paths_of(q);
+}
+
+int validate_denoise(int32_t nx, int32_t ny, int32_t ns, const rtnw_denoise_params* dp) {
+    if (nx <= 0 || ny <= 0 || (long long)nx * ny > 0x7fffffffLL / 4 || ns <= 0) return fail(RTNW_ERR_INVALID, "bad image size or sample count");
+    if (dp->iterations < 1 || dp->iterations > 8) return fail(RTNW_ERR_INVALID, "iterations must be 1..8");
+    if (dp->normal_power_log2 < 0 || dp->normal_power_log2 > 10) return fail(RTNW_ERR_INVALID, "normal_power_log2 must be 0..10");
+    if (!(dp->sigma_luminance > 0.f) || !std::isfinite(dp->sigma_luminance) || !(dp->sigma_depth > 0.f) || !std::isfinite(dp->sigma_depth))
+        return fail(RTNW_ERR_INVALID, "sigmas must be finite and > 0");
+    return RTNW_OK;
+}
+
+// dn_args for device inputs; the scratch planes are set by the caller (denoise_scratch or rtnw_denoise's staging)
+dn_args dn_inputs(const float* color, const rtnw_aov& f, int32_t nx, int32_t ny, int32_t ns, const rtnw_denoise_params* dp, float* out) {
+    dn_args a;
+    a.nx = nx; a.ny = ny; a.k = dp->normal_power_log2;
+    a.fns = (float)ns; a.sigma_l = dp->sigma_luminance; a.sigma_z = dp->sigma_depth;
+    a.color = color;
+    a.albedo = f.albedo;
+    a.normal = f.normal;
+    a.depth = f.depth;
+    a.hits = f.hits;
+    a.out = out;
+    return a;
+}
+
+// Points the denoiser's scratch planes of `a` (57 bytes per pixel, rtnw_denoise's order) into ctx->dn_scratch, grown on demand
+int denoise_scratch(rtnw_ctx* ctx, dn_args& a) {
+    const size_t n = (size_t)a.nx * a.ny;
+    const size_t sz[5] = {16 * n, 16 * n, 16 * n, 8 * n, n};
+    size_t off[5];
+    const int rc = grow(&ctx->dn_scratch, &ctx->dn_scratch_bytes, layout256(sz, 5, off), "cannot allocate the denoiser's scratch planes");
+    if (rc != RTNW_OK) return rc;
+    a.ev[0] = reinterpret_cast<float4*>(ctx->dn_scratch + off[0]);
+    a.ev[1] = reinterpret_cast<float4*>(ctx->dn_scratch + off[1]);
+    a.feat = reinterpret_cast<float4*>(ctx->dn_scratch + off[2]);
+    a.grad = reinterpret_cast<float2*>(ctx->dn_scratch + off[3]);
+    a.hit = ctx->dn_scratch + off[4];
+    return RTNW_OK;
+}
+
+// the denoiser's iterations + 2 launches on st (k_dn_variance leaves (e, var) in ev[1] for the first pass)
+int denoise_launch(const dn_args& a, int iterations, cudaStream_t st) {
+    const dim3 block(DN_BX, DN_BY), grid((unsigned)((a.nx + DN_BX - 1) / DN_BX), (unsigned)((a.ny + DN_BY - 1) / DN_BY));
+    k_dn_prepare<<<grid, block, 0, st>>>(a);
+    k_dn_variance<<<grid, block, 0, st>>>(a);
+    for (int it = 0; it < iterations; ++it)
+        k_dn_atrous<<<grid, block, 0, st>>>(a, it, it % 2 == 0 ? 1 : 0, it == iterations - 1);
+    CUDA_TRY(cudaGetLastError());
+    return RTNW_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1621,6 +1766,7 @@ int rtnw_ctx_destroy(rtnw_ctx* c) {
     cudaSetDevice(c->device);
     if (c->accum) cudaFree(c->accum);
     if (c->fixed) cudaFree(c->fixed);
+    if (c->dn_scratch) cudaFree(c->dn_scratch);
     for (int q = 0; q < 2; ++q) if (c->spare_slab[q]) cudaFree(c->spare_slab[q]);
     if (c->ctr) cudaFree(c->ctr);
     if (c->ctr_host) cudaFreeHost(c->ctr_host);
@@ -1919,37 +2065,23 @@ int rtnw_render_aov(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* c
                     const rtnw_aov* out, rtnw_stats* stats) {
     int rc = check_ctx(ctx);
     if (rc != RTNW_OK) return rc;
-    if (!scene || !cam || !out || !out->albedo || !out->normal || !out->depth || !out->hits || !out->prim_id)
-        return fail(RTNW_ERR_INVALID, "null argument");
+    if (!scene || !cam || !aov_complete(out)) return fail(RTNW_ERR_INVALID, "null argument");
     if ((rc = validate_params(params)) != RTNW_OK) return rc;
-    if (params->pixel_count != 0 || (params->flags & (RTNW_F_ACCUMULATE | RTNW_F_ROTATE_SAMPLES)))
-        return fail(RTNW_ERR_INVALID, "rtnw_render_aov covers whole images: no pixel subset, RTNW_F_ACCUMULATE or RTNW_F_ROTATE_SAMPLES");
+    if ((rc = validate_aov_params(params, false, "rtnw_render_aov covers whole images: no pixel subset, RTNW_F_ACCUMULATE or RTNW_F_ROTATE_SAMPLES")) != RTNW_OK)
+        return rc;
     const size_t n = (size_t)params->nx * params->ny;
     staging g;
     const int albedo = g.add(n * 3 * sizeof(float), nullptr, out->albedo), normal = g.add(n * 3 * sizeof(float), nullptr, out->normal);
     const int depth = g.add(n * sizeof(float), nullptr, out->depth), hits = g.add(n * sizeof(int32_t), nullptr, out->hits);
     const int prim_id = g.add(n * sizeof(int32_t), nullptr, out->prim_id);
     CUDA_TRY(g.copy_in(ctx->stream, ctx->ev_t0));
-    aov_args a;
-    a.S = scene->view;
-    a.cam = *cam;
-    a.p = *params;
-    a.albedo = g.at<float>(albedo);
-    a.normal = g.at<float>(normal);
-    a.depth = g.at<float>(depth);
-    a.hits = g.at<int32_t>(hits);
-    a.prim_id = g.at<int32_t>(prim_id);
-    a.ctr = ctx->ctr;
-    const unsigned grid = (unsigned)((n + RTNW_BLOCK - 1) / RTNW_BLOCK);
-    CUDA_TRY(cudaMemsetAsync(ctx->ctr, 0, 8 * sizeof(unsigned long long), ctx->stream));
-    CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
-    rc = by_variant(params->flags, [&](auto, auto fast) {
-        constexpr bool FAST = decltype(fast)::value;
-        return launch_coop<aov_smem<FAST>>(k_aov<FAST>, grid, ctx->stream, a);
-    });
-    if (rc != RTNW_OK) return rc;
-    CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
-    CUDA_TRY(cudaMemcpyAsync(ctx->ctr_host, ctx->ctr, 8 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    rtnw_aov planes;
+    planes.albedo = g.at<float>(albedo);
+    planes.normal = g.at<float>(normal);
+    planes.depth = g.at<float>(depth);
+    planes.hits = g.at<int32_t>(hits);
+    planes.prim_id = g.at<int32_t>(prim_id);
+    if ((rc = aov_launch(ctx, scene, cam, params, planes, ctx->stream, 4, true)) != RTNW_OK) return rc;
     CUDA_TRY(g.copy_out(ctx->stream, ctx->ev_t1));
     if ((rc = check_task_stack(ctx)) != RTNW_OK) return rc;
     rtnw_stats s = {};
@@ -1957,6 +2089,27 @@ int rtnw_render_aov(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* c
     s.kernel_launches = 1;
     s.sample_ranges = 1;
     return report_stats(ctx, stats, s, true);
+}
+
+int rtnw_render_aov_device(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam, const rtnw_render_params* params,
+                           const rtnw_aov* out_dev, void* cuda_stream, rtnw_stats* stats) {
+    int rc = check_ctx(ctx);
+    if (rc != RTNW_OK) return rc;
+    if (!scene || !cam || !aov_complete(out_dev)) return fail(RTNW_ERR_INVALID, "null argument");
+    if ((rc = validate_params(params)) != RTNW_OK) return rc;
+    if ((rc = validate_aov_params(params, true, "rtnw_render_aov_device covers whole images: no pixel subset or RTNW_F_ACCUMULATE")) != RTNW_OK)
+        return rc;
+    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : cudaStreamLegacy;  // NULL = the legacy default stream
+    if ((rc = aov_launch(ctx, scene, cam, params, *out_dev, st, 4, true)) != RTNW_OK) return rc;
+    CUDA_TRY(cudaStreamSynchronize(st));
+    if ((rc = check_task_stack(ctx)) != RTNW_OK) return rc;
+    rtnw_stats s = {};
+    s.paths = s.rays = aov_rays(*params);
+    s.kernel_launches = 1;
+    s.sample_ranges = 1;
+    if ((rc = report_stats(ctx, stats, s, false)) != RTNW_OK) return rc;
+    if (stats) stats->total_ms = stats->kernel_ms;  // no copies
+    return RTNW_OK;
 }
 
 int rtnw_eval_texture(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t tex_id, const float* uvp, size_t n, float* rgb_out) {
@@ -1980,42 +2133,60 @@ int rtnw_denoise(rtnw_ctx* ctx, const float* color_sums, const rtnw_aov* feature
     if (rc != RTNW_OK) return rc;
     if (!color_sums || !features || !features->albedo || !features->normal || !features->depth || !features->hits || !dp || !rgb_out)
         return fail(RTNW_ERR_INVALID, "null argument");
-    if (nx <= 0 || ny <= 0 || (long long)nx * ny > 0x7fffffffLL / 4 || ns <= 0) return fail(RTNW_ERR_INVALID, "bad image size or sample count");
-    if (dp->iterations < 1 || dp->iterations > 8) return fail(RTNW_ERR_INVALID, "iterations must be 1..8");
-    if (dp->normal_power_log2 < 0 || dp->normal_power_log2 > 10) return fail(RTNW_ERR_INVALID, "normal_power_log2 must be 0..10");
-    if (!(dp->sigma_luminance > 0.f) || !std::isfinite(dp->sigma_luminance) || !(dp->sigma_depth > 0.f) || !std::isfinite(dp->sigma_depth))
-        return fail(RTNW_ERR_INVALID, "sigmas must be finite and > 0");
+    if ((rc = validate_denoise(nx, ny, ns, dp)) != RTNW_OK) return rc;
     const size_t n = (size_t)nx * ny;
     staging g;  // 101 bytes per pixel; the colour span is overwritten with the output
     const int color = g.add(12 * n, color_sums, rgb_out), albedo = g.add(12 * n, features->albedo), normal = g.add(12 * n, features->normal);
     const int depth = g.add(4 * n, features->depth), hits = g.add(4 * n, features->hits);
     const int ev0 = g.add(16 * n), ev1 = g.add(16 * n), feat = g.add(16 * n), grad = g.add(8 * n), hit = g.add(n);
     CUDA_TRY(g.copy_in(ctx->stream, ctx->ev_t0));
-    dn_args a;
-    a.nx = nx; a.ny = ny; a.k = dp->normal_power_log2;
-    a.fns = (float)ns; a.sigma_l = dp->sigma_luminance; a.sigma_z = dp->sigma_depth;
-    a.color = a.out = g.at<float>(color);
-    a.albedo = g.at<float>(albedo);
-    a.normal = g.at<float>(normal);
-    a.depth = g.at<float>(depth);
-    a.hits = g.at<int32_t>(hits);
+    rtnw_aov f = {};
+    f.albedo = g.at<float>(albedo);
+    f.normal = g.at<float>(normal);
+    f.depth = g.at<float>(depth);
+    f.hits = g.at<int32_t>(hits);
+    dn_args a = dn_inputs(g.at<float>(color), f, nx, ny, ns, dp, g.at<float>(color));
     a.ev[0] = g.at<float4>(ev0);
     a.ev[1] = g.at<float4>(ev1);
     a.feat = g.at<float4>(feat);
     a.grad = g.at<float2>(grad);
     a.hit = g.at<unsigned char>(hit);
-    const dim3 block(DN_BX, DN_BY), grid((unsigned)((nx + DN_BX - 1) / DN_BX), (unsigned)((ny + DN_BY - 1) / DN_BY));
     CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
-    k_dn_prepare<<<grid, block, 0, ctx->stream>>>(a);
-    k_dn_variance<<<grid, block, 0, ctx->stream>>>(a);
-    for (int it = 0; it < dp->iterations; ++it)  // k_dn_variance left (e, var) in ev[1]
-        k_dn_atrous<<<grid, block, 0, ctx->stream>>>(a, it, it % 2 == 0 ? 1 : 0, it == dp->iterations - 1);
-    CUDA_TRY(cudaGetLastError());
+    if ((rc = denoise_launch(a, dp->iterations, ctx->stream)) != RTNW_OK) return rc;
     CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
     CUDA_TRY(g.copy_out(ctx->stream, ctx->ev_t1));
     rtnw_stats s = {};
     s.kernel_launches = dp->iterations + 2;
     return report_stats(ctx, stats, s, true);
+}
+
+int rtnw_denoise_device(rtnw_ctx* ctx, const float* color_sums_dev, const rtnw_aov* features_dev, int32_t nx, int32_t ny, int32_t ns,
+                        const rtnw_denoise_params* dp, float* rgb_out_dev, void* cuda_stream, rtnw_stats* stats) {
+    int rc = check_ctx(ctx);
+    if (rc != RTNW_OK) return rc;
+    const rtnw_aov* f = features_dev;
+    if (!color_sums_dev || !f || !f->albedo || !f->normal || !f->depth || !f->hits || !dp || !rgb_out_dev)
+        return fail(RTNW_ERR_INVALID, "null argument");
+    if ((rc = validate_denoise(nx, ny, ns, dp)) != RTNW_OK) return rc;
+    // the output must not overlap an input: the last pass writes it while it still reads other pixels' albedo
+    const size_t n = (size_t)nx * ny;
+    const uintptr_t o = (uintptr_t)rgb_out_dev, o_end = o + 12 * n;
+    const struct { const void* p; size_t bytes; } in[5] = {{color_sums_dev, 12 * n}, {f->albedo, 12 * n}, {f->normal, 12 * n},
+                                                           {f->depth, 4 * n}, {f->hits, 4 * n}};
+    for (const auto& b : in)
+        if ((uintptr_t)b.p < o_end && o < (uintptr_t)b.p + b.bytes) return fail(RTNW_ERR_INVALID, "rgb_out_dev overlaps an input");
+    dn_args a = dn_inputs(color_sums_dev, *f, nx, ny, ns, dp, rgb_out_dev);
+    if ((rc = denoise_scratch(ctx, a)) != RTNW_OK) return rc;
+    cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : cudaStreamLegacy;  // NULL = the legacy default stream
+    CUDA_TRY(cudaEventRecord(ctx->ev0, st));
+    if ((rc = denoise_launch(a, dp->iterations, st)) != RTNW_OK) return rc;
+    CUDA_TRY(cudaEventRecord(ctx->ev1, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    rtnw_stats s = {};
+    s.kernel_launches = dp->iterations + 2;
+    if ((rc = report_stats(ctx, stats, s, false)) != RTNW_OK) return rc;
+    if (stats) stats->total_ms = stats->kernel_ms;  // no copies
+    return RTNW_OK;
 }
 
 int rtnw_eval_perlin(rtnw_ctx* ctx, const rtnw_scene* scene, int32_t which, const float* xyz, size_t n, float* out) {
@@ -2093,6 +2264,8 @@ struct rtnw_multi {
     float* accum[RTNW_MAX_DEVICES] = {};   // per device: nx*ny*3 sums of its share of the samples
     size_t accum_floats[RTNW_MAX_DEVICES] = {};
     cudaEvent_t done[RTNW_MAX_DEVICES] = {};
+    float* aov[RTNW_MAX_DEVICES] = {};     // per device: rtnw_render_aov_multi's planes of its share, 9 words per pixel (aov_planes)
+    size_t aov_words[RTNW_MAX_DEVICES] = {};
     bool peer[RTNW_MAX_DEVICES] = {};      // device 0 reads this rank's buffer directly (same device, or P2P over NVLink)
     float* stage = nullptr;                // device 0: copies of the buffers it cannot read directly
     size_t stage_floats = 0;
@@ -2108,6 +2281,7 @@ int rtnw_ctx_destroy_multi(rtnw_multi* m) {
         if (!m->ctx[d]) continue;
         cudaSetDevice(m->ctx[d]->device);
         if (m->accum[d]) cudaFree(m->accum[d]);
+        if (m->aov[d]) cudaFree(m->aov[d]);
         if (m->done[d]) cudaEventDestroy(m->done[d]);
         if (d == 0 && m->stage) cudaFree(m->stage);
         rtnw_ctx_destroy(m->ctx[d]);
@@ -2174,31 +2348,43 @@ int rtnw_scene_upload_multi(rtnw_multi* m, const rtnw_scene_desc* desc, rtnw_mul
     return RTNW_OK;
 }
 
-int rtnw_render_multi(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_camera* cam, const rtnw_render_params* params,
-                      float* accum_rgb, rtnw_stats* stats) {
-    if (!m || !ms || ms->n != m->n || !cam || !accum_rgb) return fail(RTNW_ERR_INVALID, "null argument");
+// rtnw_render_multi and rtnw_render_aov_multi accept whole frames only
+static int validate_multi_params(const rtnw_render_params* params, const char* who) {
     int rc = validate_params(params);
     if (rc != RTNW_OK) return rc;
     if (params->pixel_count != 0 || params->sample_begin != 0 || params->sample_stride != 1 ||
         (params->flags & (RTNW_F_ACCUMULATE | RTNW_F_ROTATE_SAMPLES)))
-        return fail(RTNW_ERR_INVALID, "rtnw_render_multi renders whole frames: sample_begin 0, sample_stride 1, no pixel subset, no ACCUMULATE / ROTATE flags");
+        return fail(RTNW_ERR_INVALID, std::string(who) + " renders whole frames: sample_begin 0, sample_stride 1, no pixel subset, no ACCUMULATE / ROTATE flags");
+    return RTNW_OK;
+}
+
+// One frame on the devices of m.  Every device renders its share of every pixel's samples (ownership rotates with the pixel
+// index: even for any ns) and, with `aovs`, the AOVs of the same share right after it on its stream.  Device 0 adds the shares
+// in rank order (deterministic), copies the outputs that are given to the host and, with dp, denoises the summed frame there.
+static int multi_frame(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_camera* cam, const rtnw_render_params* params, bool aovs,
+                       float* accum_rgb, const rtnw_aov* aov, const rtnw_denoise_params* dp, float* denoised_rgb, rtnw_stats* stats) {
     const int n = m->n;
-    const size_t floats = (size_t)params->nx * params->ny * 3;
-    int need_stage = 0;
+    const size_t pixels = (size_t)params->nx * params->ny, floats = pixels * 3, words = aovs ? pixels * 9 : 0;
+    int rc = RTNW_OK, need_stage = 0;
     for (int d = 1; d < n; ++d) need_stage += m->peer[d] ? 0 : 1;
     for (int d = 0; d < n; ++d) {
         CUDA_TRY(cudaSetDevice(m->ctx[d]->device));
         rc = grow(&m->accum[d], &m->accum_floats[d], floats, "cannot allocate the per-device accumulation buffers");
         if (rc != RTNW_OK) return rc;
+        if (aovs && (rc = grow(&m->aov[d], &m->aov_words[d], words, "cannot allocate the per-device AOV planes")) != RTNW_OK) return rc;
     }
-    if (need_stage) {
-        CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
-        if ((rc = grow(&m->stage, &m->stage_floats, floats * need_stage, "cannot allocate the staging planes")) != RTNW_OK) return rc;
+    rtnw_ctx* c0 = m->ctx[0];
+    CUDA_TRY(cudaSetDevice(c0->device));
+    if (need_stage) {  // per staged rank: its colour plane, then (after all colour planes) its AOV planes
+        if ((rc = grow(&m->stage, &m->stage_floats, (floats + words) * need_stage, "cannot allocate the staging planes")) != RTNW_OK) return rc;
     }
-    // every device renders its share of every pixel's samples (ownership rotates with the pixel index: even for any ns)
+    dn_args dn = {};
+    if (dp) {  // the denoised frame overwrites the colour sums of device 0 after their host copy: only k_dn_prepare reads them
+        dn = dn_inputs(m->accum[0], aov_planes(m->aov[0], pixels), params->nx, params->ny, params->sample_count, dp, m->accum[0]);
+        if ((rc = denoise_scratch(c0, dn)) != RTNW_OK) return rc;
+    }
     render_ticket ticket[RTNW_MAX_DEVICES];
-    CUDA_TRY(cudaSetDevice(m->ctx[0]->device));
-    CUDA_TRY(cudaEventRecord(m->ctx[0]->ev_t0, m->ctx[0]->stream));
+    CUDA_TRY(cudaEventRecord(c0->ev_t0, c0->stream));
     for (int d = 0; d < n; ++d) {
         rtnw_ctx* c = m->ctx[d];
         CUDA_TRY(cudaSetDevice(c->device));
@@ -2206,29 +2392,50 @@ int rtnw_render_multi(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_came
         if (n > 1) { p.flags |= RTNW_F_ROTATE_SAMPLES; p.sample_begin = d; p.sample_stride = n; }
         rc = render_launch(c, ms->scene[d], cam, &p, m->accum[d], c->stream, &ticket[d]);
         if (rc != RTNW_OK) return rc;
+        if (aovs && (rc = aov_launch(c, ms->scene[d], cam, &p, aov_planes(m->aov[d], pixels), c->stream, 5, false)) != RTNW_OK) return rc;
         CUDA_TRY(cudaEventRecord(m->done[d], c->stream));
     }
-    // one sum on device 0, in rank order (deterministic), then the frame goes to the host
-    rtnw_ctx* c0 = m->ctx[0];
     CUDA_TRY(cudaSetDevice(c0->device));
     if (n > 1) {
-        rank_planes P;
-        P.n = n;
+        rank_planes P, A;  // colour, AOV planes
+        P.n = A.n = n;
         int staged = 0;
         for (int d = 1; d < n; ++d) {
             CUDA_TRY(cudaStreamWaitEvent(c0->stream, m->done[d], 0));
-            if (m->peer[d]) P.src[d] = m->accum[d];
-            else {
-                float* dst = m->stage + floats * (size_t)staged++;
-                CUDA_TRY(cudaMemcpyPeerAsync(dst, c0->device, m->accum[d], m->ctx[d]->device, floats * sizeof(float), c0->stream));
-                P.src[d] = dst;
+            if (m->peer[d]) {
+                P.src[d] = m->accum[d];
+                A.src[d] = m->aov[d];
+                continue;
             }
+            float* dst = m->stage + floats * (size_t)staged;
+            CUDA_TRY(cudaMemcpyPeerAsync(dst, c0->device, m->accum[d], m->ctx[d]->device, floats * sizeof(float), c0->stream));
+            P.src[d] = dst;
+            if (aovs) {
+                dst = m->stage + floats * (size_t)need_stage + words * (size_t)staged;
+                CUDA_TRY(cudaMemcpyPeerAsync(dst, c0->device, m->aov[d], m->ctx[d]->device, words * sizeof(float), c0->stream));
+                A.src[d] = dst;
+            }
+            ++staged;
         }
         P.src[0] = m->accum[0];
+        A.src[0] = m->aov[0];
         k_sum_ranks<<<c0->sm_count * 8, 256, 0, c0->stream>>>(m->accum[0], P, floats);
+        if (aovs) k_sum_aov_ranks<<<c0->sm_count * 8, 256, 0, c0->stream>>>(m->aov[0], A, pixels);
         CUDA_TRY(cudaGetLastError());
     }
-    CUDA_TRY(cudaMemcpyAsync(accum_rgb, m->accum[0], floats * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
+    if (accum_rgb) CUDA_TRY(cudaMemcpyAsync(accum_rgb, m->accum[0], floats * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
+    if (aov) {
+        const rtnw_aov v = aov_planes(m->aov[0], pixels);
+        CUDA_TRY(cudaMemcpyAsync(aov->albedo, v.albedo, floats * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
+        CUDA_TRY(cudaMemcpyAsync(aov->normal, v.normal, floats * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
+        CUDA_TRY(cudaMemcpyAsync(aov->depth, v.depth, pixels * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
+        CUDA_TRY(cudaMemcpyAsync(aov->hits, v.hits, pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, c0->stream));
+        CUDA_TRY(cudaMemcpyAsync(aov->prim_id, v.prim_id, pixels * sizeof(int32_t), cudaMemcpyDeviceToHost, c0->stream));
+    }
+    if (dp) {
+        if ((rc = denoise_launch(dn, dp->iterations, c0->stream)) != RTNW_OK) return rc;
+        CUDA_TRY(cudaMemcpyAsync(denoised_rgb, dn.out, floats * sizeof(float), cudaMemcpyDeviceToHost, c0->stream));
+    }
     CUDA_TRY(cudaEventRecord(c0->ev_t1, c0->stream));
     rtnw_stats total;
     std::memset(&total, 0, sizeof total);
@@ -2237,6 +2444,7 @@ int rtnw_render_multi(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_came
         rtnw_stats st;
         rc = render_finish(m->ctx[d], ticket[d], &st);
         if (rc != RTNW_OK) return rc;
+        if (aovs && (rc = check_task_stack(m->ctx[d], 5)) != RTNW_OK) return rc;
         total.paths += st.paths; total.rays += st.rays; total.box_tests += st.box_tests; total.prim_tests += st.prim_tests;
         total.kernel_ms = std::max(total.kernel_ms, st.kernel_ms);
         total.kernel_launches += st.kernel_launches;
@@ -2245,9 +2453,30 @@ int rtnw_render_multi(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_came
     CUDA_TRY(cudaSetDevice(c0->device));
     CUDA_TRY(cudaStreamSynchronize(c0->stream));
     CUDA_TRY(cudaEventElapsedTime(&total.total_ms, c0->ev_t0, c0->ev_t1));
-    if (n > 1) total.kernel_launches += 1;
+    if (n > 1) total.kernel_launches += aovs ? 2 : 1;  // k_sum_ranks, k_sum_aov_ranks
+    if (aovs) total.kernel_launches += n;             // k_aov
+    if (dp) total.kernel_launches += dp->iterations + 2;
     if (stats) *stats = total;
     return RTNW_OK;
+}
+
+int rtnw_render_multi(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_camera* cam, const rtnw_render_params* params,
+                      float* accum_rgb, rtnw_stats* stats) {
+    if (!m || !ms || ms->n != m->n || !cam || !accum_rgb) return fail(RTNW_ERR_INVALID, "null argument");
+    const int rc = validate_multi_params(params, "rtnw_render_multi");
+    if (rc != RTNW_OK) return rc;
+    return multi_frame(m, ms, cam, params, false, accum_rgb, nullptr, nullptr, nullptr, stats);
+}
+
+int rtnw_render_aov_multi(rtnw_multi* m, const rtnw_multi_scene* ms, const rtnw_camera* cam, const rtnw_render_params* params,
+                          float* accum_rgb, const rtnw_aov* aov, const rtnw_denoise_params* dp, float* denoised_rgb, rtnw_stats* stats) {
+    if (!m || !ms || ms->n != m->n || !cam || (aov && !aov_complete(aov))) return fail(RTNW_ERR_INVALID, "null argument");
+    if (!accum_rgb && !aov && !denoised_rgb) return fail(RTNW_ERR_INVALID, "no output: give accum_rgb, aov or denoised_rgb");
+    if (!dp != !denoised_rgb) return fail(RTNW_ERR_INVALID, "denoise params and denoised_rgb go together");
+    int rc = validate_multi_params(params, "rtnw_render_aov_multi");
+    if (rc != RTNW_OK) return rc;
+    if (dp && (rc = validate_denoise(params->nx, params->ny, params->sample_count, dp)) != RTNW_OK) return rc;
+    return multi_frame(m, ms, cam, params, true, accum_rgb, aov, dp, denoised_rgb, stats);
 }
 
 }  // extern "C"
