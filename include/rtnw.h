@@ -172,6 +172,38 @@ enum rtnw_background { RTNW_BG_BLACK = 0 /* PSC/main.cpp:44 */, RTNW_BG_SKY = 1 
                                     the frame, and for pixel p this call renders the samples s in [0, ns) with
                                     s = (sample_begin - p) mod sample_stride, + k*sample_stride: rank g of G passes
                                     sample_begin = g, sample_stride = G; each pixel gets floor or ceil(ns/G) samples per rank */
+#define RTNW_F_LIGHT_SAMPLING 64u /* same expected image, other noise (DESIGN.md §5 measures where it helps): lambertian and
+                                    isotropic bounces pick their direction from a one-sample mixture of the scene's light table
+                                    and the reference's own scatter density (below).
+                                    Honoured by rtnw_render, rtnw_render_device, rtnw_render_multi and the colour of
+                                    rtnw_render_aov_multi; accepted and ignored by every other entry point.  A bit-for-bit no-op,
+                                    with no extra draw, when the light table is empty or RTNW_F_EMIT is off */
+
+/* Light sampling (RTNW_F_LIGHT_SAMPLING).  The reference's contract is its own image, so the mixture is weighted by the
+ * reference's scatter density, not by a cosine lobe.  lambertian::scatter (PSC/material.h:64-72) picks n + random_in_unit_sphere(),
+ * uniform in the unit ball tangent at p: its solid-angle density is p_ref(w) = (2/pi) cos^3(theta), cos(theta) = w.n > 0 (the
+ * chord through the ball is 2 cos(theta) long), else 0; isotropic::scatter's is p_ref = 1/(4 pi).  All arithmetic is float32.
+ * L = number of lights in the scene's light table (rtnw_scene_inspect table 4).  At a lambertian or isotropic hit, with L > 0
+ * and RTNW_F_EMIT on, the path first draws u:
+ *   u < 0.5 (light branch): light k = min((int)((2u) L), L - 1), then
+ *     rectangle: q = (a0 + draw() (a1 - a0), b0 + draw() (b1 - b0)) on its extent axes (first draw -> a) at plane offset k0;
+ *                direction d = unit(q - p): unit length, so that the scattered ray's t_min (a parameter, not a distance)
+ *                skips the same ~0.001 of distance as the reference's directions of length 0..2 do; q - p itself (hundreds of
+ *                units long in the Cornell scenes) would skip occluders within 0.5 of p and bias the image;
+ *     sphere:    r1 = draw(), r2 = draw(); if |c - p|^2 <= r^2 the path ends.  cmax = sqrtf(1 - r^2 / |c - p|^2),
+ *                z = 1 + r2 (cmax - 1), phi = 2 pi r1, s = sqrtf(1 - z z); w = unit(c - p), a = |w.x| > 0.9 ? (0,1,0) : (1,0,0),
+ *                v = unit(w x a), u = w x v; d = (cosf(phi) s) u + (sinf(phi) s) v + z w;
+ *     scattered.time: r_in.time for lambertian, 0 for isotropic; attenuation value = the material's texture value.
+ *   otherwise (reference branch): material::scatter exactly as without the flag.
+ * Weight, with e = unit(d):  p_ref as above (lambertian: c = e.n; c > 0 else the path ends; p_ref = c c c (2/pi)), and for each
+ * light k in table order, p_k(e) = 0 unless the ray (p, e) meets light k at t > 0:
+ *     rectangle: t = (k0 - p_N) / e_N along its plane axis N, the point inside the bounds by the reference's inclusive test,
+ *                p_k = t t / (|e_N| area);
+ *     sphere:    p outside it and e.w >= cmax: p_k = 1 / (2 pi (1 - cmax)).
+ * p_mix = 0.5 p_ref + 0.5 (sum_k p_k / L), and attenuation = value * (p_ref / p_mix).  p_mix is the density of the directions
+ * that do not end the path, so every pixel's expectation is the reference's; one bounce's weight lies in [0, 2].  Metal and dielectric
+ * keep the reference's scatter.  The sample stream stays keyed by (seed, pixel, sample). */
+#define RTNW_MAX_LIGHTS 16
 
 typedef struct rtnw_render_params {
     int32_t nx, ny;
@@ -261,7 +293,12 @@ int rtnw_prepared_free(rtnw_prepared* p);
  * inspection (the invariants the traversal's exactness rests on are checked on the CPU from these, tests/test_device_tables.py).
  * table: 0 = record stream (32 B each: 8 floats, [6] = tag bits, [7] = int), 1 = per-record leaf id (int32),
  * 2 = gates (2 x int32: first records of the one or two leaves, -1 = none), 3 = gate tree (128 B per 4-wide node:
- * minx[4] miny[4] minz[4] maxx[4] maxy[4] maxz[4] ref[4] pad[4]; ref >= 0 wide node, < 0 ~gate, INT32_MIN absent).
+ * minx[4] miny[4] minz[4] maxx[4] maxy[4] maxz[4] ref[4] pad[4]; ref >= 0 wide node, < 0 ~gate, INT32_MIN absent),
+ * 4 = light table of RTNW_F_LIGHT_SAMPLING (32 B per light, at most RTNW_MAX_LIGHTS): the records, in record order, whose material
+ * is RTNW_MAT_DIFFUSE_LIGHT and that are an xy / xz / yz rectangle or a sphere that does not move, with the identity as their
+ * own and their item's transform chain, and neither a box face nor a medium boundary.  Floats {a0, a1, b0, b1, k, area, kind,
+ * record}: a rectangle's extents and plane offset as in rtnw_prim, area = (a1 - a0) * (b1 - b0); a sphere's {cx, cy, cz, r, 0, 0};
+ * kind = rtnw_prim_kind and record = index into table 0, both as int32 bit patterns.
  * Copies min(cap_bytes, size) bytes into buf (may be NULL) and returns the table's size in bytes, or a negative status. */
 int64_t rtnw_scene_inspect(const rtnw_scene_desc* desc, int32_t table, void* buf, size_t cap_bytes);
 int rtnw_scene_free(rtnw_ctx* ctx, rtnw_scene* scene);

@@ -26,7 +26,7 @@ RTNW_OK = 0
 RTNW_ERR_INVALID, RTNW_ERR_CUDA, RTNW_ERR_UNSUPPORTED, RTNW_ERR_NOMEM = -1, -2, -3, -4
 BG_BLACK, BG_SKY = 0, 1
 TEXF_BILINEAR = 1
-F_DE_NAN, F_EMIT, F_FAST_BVH, F_COUNTERS, F_ACCUMULATE, F_ROTATE_SAMPLES = 1, 2, 4, 8, 16, 32
+F_DE_NAN, F_EMIT, F_FAST_BVH, F_COUNTERS, F_ACCUMULATE, F_ROTATE_SAMPLES, F_LIGHT_SAMPLING = 1, 2, 4, 8, 16, 32, 64
 FLT_MAX = float(np.finfo(np.float32).max)
 
 
@@ -326,10 +326,10 @@ def write_pfm(path, array: np.ndarray) -> None:
 
 def device_tables(desc_ptr) -> dict:
     """The tables rtnw_scene_upload derives from a scene_desc, built on the host (no GPU needed): record stream, leaf ids,
-    gates and the 4-wide gate tree (include/rtnw.h: rtnw_scene_inspect)."""
+    gates, the 4-wide gate tree and the light table of F_LIGHT_SAMPLING (include/rtnw.h: rtnw_scene_inspect)."""
     out = {}
     for table, (name, dtype, width) in enumerate([("recs", np.float32, 8), ("rec_leaf", np.int32, 1), ("gates", np.int32, 2),
-                                                    ("wnodes", np.float32, 32)]):
+                                                    ("wnodes", np.float32, 32), ("lights", np.float32, 8)]):
         n = device_lib().rtnw_scene_inspect(desc_ptr, table, None, 0)
         _check_dev(min(n, 0))
         a = np.empty(n // np.dtype(dtype).itemsize, dtype=dtype)

@@ -36,6 +36,8 @@ struct render_args {
     int chunk_total;              // range c of a pixel with n samples: k in [cum[c]*n/total, cum[c+1]*n/total)
     int chunk_cum[RTNW_MAX_CHUNKS + 1];
     unsigned long long* ctr;      // [0] next pixel, [1] rays, [2] box tests, [3] primitive tests, [4] task stack overflows
+    const float4* lights;         // RTNW_F_LIGHT_SAMPLING: the scene's light table (2 float4 per light), read by k_render<.., true> only
+    int n_lights;
 };
 
 // Partial sums of the sample ranges of a pixel are added in 64-bit fixed point with integer atomics: integer addition
@@ -72,7 +74,8 @@ template <bool FAST> using block_smem = coop_smem<FAST ? 2 : 1>;
 // block-cooperative (coop_closest_hit): list items in lockstep, BVH items as uniform tasks from shared-memory queues.
 // A per-lane traversal state machine was measured at 2-13 active lanes of 32 per instruction (profiles/r1-r3*.txt);
 // this form keeps every phase uniform across the warp.
-template <bool COUNT, bool FAST>
+// LIGHTS: RTNW_F_LIGHT_SAMPLING with a non-empty light table and RTNW_F_EMIT (mixture_scatter); the host selects it.
+template <bool COUNT, bool FAST, bool LIGHTS>
 __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const render_args P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     typedef block_smem<FAST> SM;
@@ -206,7 +209,8 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
                 } else if (depth < P.p.max_depth) {
                     ray_t sc;
                     f3 att;
-                    if (material_scatter(P.S, s.mat, wr, s, g, att, sc)) {
+                    if (LIGHTS ? mixture_scatter(P.S, P.lights, P.n_lights, s.mat, wr, s, g, att, sc)
+                               : material_scatter(P.S, s.mat, wr, s, g, att, sc)) {
                         T = T * att;
                         wr = sc;
                         ++depth;
@@ -995,7 +999,7 @@ struct rtnw_ctx {
     unsigned char* dn_scratch = nullptr;     // the denoiser's planes for rtnw_denoise_device and rtnw_render_aov_multi
     size_t dn_scratch_bytes = 0;
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;  // rtnw_render's total_ms
-    int blocks_per_sm[4] = {0, 0, 0, 0};
+    int blocks_per_sm[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // per k_render instantiation, render_occupancy
     // freed scene slabs are kept for the next upload (cudaMalloc/cudaFree synchronise the device and can take
     // milliseconds to hundreds of milliseconds in a process that also hosts another allocator)
     void* spare_slab[2] = {nullptr, nullptr};
@@ -1004,6 +1008,8 @@ struct rtnw_ctx {
 
 struct rtnw_scene {
     scene_view view;
+    const float4* lights = nullptr;  // light table (2 float4 per light) for k_render's RTNW_F_LIGHT_SAMPLING; kept out of scene_view,
+    int32_t n_lights = 0;            // which every other kernel takes by value
     void* slab = nullptr;  // one allocation holding every table
     size_t slab_bytes = 0;
 };
@@ -1394,7 +1400,25 @@ struct stream_builder {
         if (recs.size() >= (1u << 24) || gates.size() >= (1u << RTNW_IDX_BITS) || wnodes.size() / 8 >= (1u << RTNW_IDX_BITS)) return bad("scene exceeds the record / gate index range");
         if (gate_leaves.empty()) gate_leaves.push_back(make_int2(-1, -1));
         if (wnodes.empty()) wnodes.resize(8, make_float4(0, 0, 0, 0));
+        collect_lights();
         return true;
+    }
+
+    // ---- light table of RTNW_F_LIGHT_SAMPLING (include/rtnw.h, rtnw_scene_inspect table 4) ----------------------------
+    std::vector<float4> lights;  // 2 per light
+    void collect_lights() {
+        for (size_t i = 0; i < recs.size() && lights.size() < 2 * RTNW_MAX_LIGHTS; ++i) {
+            const rec& r = recs[i];
+            const uint32_t tag = as_uint(r.b.z), kind = tag & 15u;
+            if (kind == K_MEDIUM) { i += (size_t)as_int(r.a.z); continue; }  // its boundary records are not lights
+            if (kind != K_SPHERE && (kind < K_RECT_XY || kind > K_RECT_YZ)) continue;  // box faces and moving spheres are not sampled
+            if ((tag >> 8) != 0 || rec_xf[i] != 0) continue;                             // nor anything behind a transform
+            const int32_t mat = as_int(r.b.w);
+            if (d.materials[mat].kind != RTNW_MAT_DIFFUSE_LIGHT) continue;
+            const float area = kind == K_SPHERE ? 0.f : (r.a.y - r.a.x) * (r.a.w - r.a.z);
+            lights.push_back(r.a);
+            lights.push_back(make_float4(kind == K_SPHERE ? 0.f : r.b.x, area, bits((int32_t)kind), bits((int32_t)i)));
+        }
     }
 };
 
@@ -1420,23 +1444,23 @@ int report_stats(rtnw_ctx* ctx, rtnw_stats* stats, rtnw_stats s, bool total) {
     return RTNW_OK;
 }
 
-// resident blocks per SM of k_render<COUNT, FAST> (cached per context)
-template <bool COUNT, bool FAST>
+// resident blocks per SM of k_render<COUNT, FAST, LIGHTS> (cached per context)
+template <bool COUNT, bool FAST, bool LIGHTS>
 int render_occupancy(rtnw_ctx* ctx, int* out) {
-    int& bps = ctx->blocks_per_sm[(COUNT ? 1 : 0) + (FAST ? 2 : 0)];
+    int& bps = ctx->blocks_per_sm[(COUNT ? 1 : 0) + (FAST ? 2 : 0) + (LIGHTS ? 4 : 0)];
     if (bps == 0) {
-        CUDA_TRY(cudaFuncSetAttribute(k_render<COUNT, FAST>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(block_smem<FAST>)));
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_render<COUNT, FAST>, RTNW_BLOCK, sizeof(block_smem<FAST>)));
+        CUDA_TRY(cudaFuncSetAttribute(k_render<COUNT, FAST, LIGHTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(block_smem<FAST>)));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_render<COUNT, FAST, LIGHTS>, RTNW_BLOCK, sizeof(block_smem<FAST>)));
         if (bps < 1) bps = 1;
     }
     *out = bps;
     return RTNW_OK;
 }
 
-template <bool COUNT, bool FAST>
+template <bool COUNT, bool FAST, bool LIGHTS>
 int launch_render(rtnw_ctx* ctx, const render_args& a, cudaStream_t st) {
     int bps = 0;
-    const int rc = render_occupancy<COUNT, FAST>(ctx, &bps);
+    const int rc = render_occupancy<COUNT, FAST, LIGHTS>(ctx, &bps);
     if (rc != RTNW_OK) return rc;
     int blocks = ctx->sm_count * bps;
     const long long warps_needed = ((long long)a.p.pixel_count * a.chunks + 31) / 32;
@@ -1445,7 +1469,7 @@ int launch_render(rtnw_ctx* ctx, const render_args& a, cudaStream_t st) {
 #ifdef RTNW_TUNING  // A/B builds only (scripts/ab_build.sh): the product library reads no environment on the launch path
     if (const char* e = getenv("RTNW_GRID_BLOCKS")) { const int v = atoi(e); if (v > 0) blocks = v; }
 #endif
-    k_render<COUNT, FAST><<<blocks, RTNW_BLOCK, sizeof(block_smem<FAST>), st>>>(a);
+    k_render<COUNT, FAST, LIGHTS><<<blocks, RTNW_BLOCK, sizeof(block_smem<FAST>), st>>>(a);
     CUDA_TRY(cudaGetLastError());
     return RTNW_OK;
 }
@@ -1512,6 +1536,10 @@ int render_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam
     if (a.p.pixel_count == 0) { a.p.pixel_begin = 0; a.p.pixel_stride = 1; a.p.pixel_count = p->nx * p->ny; }
     a.accum = accum_dev;
     a.ctr = ctx->ctr;
+    a.lights = scene->lights;
+    a.n_lights = scene->n_lights;
+    // light sampling changes nothing without a light to sample or without emission: those renders take the plain kernel
+    const bool lights = (p->flags & RTNW_F_LIGHT_SAMPLING) && (p->flags & RTNW_F_EMIT) && scene->n_lights > 0;
     int rc = RTNW_OK;
     pick_chunks(a.p, a);
     a.fixed = nullptr;
@@ -1527,7 +1555,10 @@ int render_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam
     }
     CUDA_TRY(cudaMemsetAsync(ctx->ctr, 0, 8 * sizeof(unsigned long long), st));
     CUDA_TRY(cudaEventRecord(ctx->ev0, st));
-    rc = by_variant(p->flags, [&](auto count, auto fast) { return launch_render<decltype(count)::value, decltype(fast)::value>(ctx, a, st); });
+    rc = by_variant(p->flags, [&](auto count, auto fast) {
+        constexpr bool COUNT = decltype(count)::value, FAST = decltype(fast)::value;
+        return lights ? launch_render<COUNT, FAST, true>(ctx, a, st) : launch_render<COUNT, FAST, false>(ctx, a, st);
+    });
     if (rc != RTNW_OK) return rc;
     if (a.chunks > 1) {
         k_finish_fixed<<<(a.p.pixel_count + 255) / 256, 256, 0, st>>>(a.fixed, a.p.pixel_begin, a.p.pixel_stride, a.p.pixel_count,
@@ -1836,6 +1867,7 @@ int64_t rtnw_scene_inspect(const rtnw_scene_desc* desc, int32_t table, void* buf
         case 1: src = sb.leaf.data(); bytes = sb.leaf.size() * sizeof(int32_t); break;
         case 2: src = sb.gate_leaves.data(); bytes = sb.gate_leaves.size() * sizeof(int2); break;
         case 3: src = sb.wnodes.data(); bytes = sb.wnodes.size() * sizeof(float4); break;
+        case 4: src = sb.lights.data(); bytes = sb.lights.size() * sizeof(float4); break;
         default: return fail(RTNW_ERR_INVALID, "unknown table");
     }
     if (buf && cap_bytes) std::memcpy(buf, src, std::min(cap_bytes, bytes));
@@ -1844,13 +1876,13 @@ int64_t rtnw_scene_inspect(const rtnw_scene_desc* desc, int32_t table, void* buf
 
 // The device image of a scene, built once on the host (no device needed): one slab with every table at a 256-byte
 // aligned offset, in pinned memory when a CUDA driver is present (so an upload is a single asynchronous DMA).
-enum prepared_table { T_RECS, T_LEAF, T_RXF, T_NODES, T_GATES, T_XF, T_MAT, T_TEX, T_RV, T_PERM, T_IMG, N_TABLES };
+enum prepared_table { T_RECS, T_LEAF, T_RXF, T_NODES, T_GATES, T_XF, T_MAT, T_TEX, T_RV, T_PERM, T_IMG, T_LIGHTS, N_TABLES };
 struct rtnw_prepared {
     uint8_t* host = nullptr;
     bool pinned = false;
     size_t bytes = 0;
     size_t off[N_TABLES] = {};  // byte offset of each table in the slab
-    int32_t n_recs = 0, n_materials = 0, n_textures = 0, n_wnodes = 0, fast_node_base = 0;
+    int32_t n_recs = 0, n_materials = 0, n_textures = 0, n_wnodes = 0, fast_node_base = 0, n_lights = 0;
 };
 
 int rtnw_prepared_free(rtnw_prepared* p) {
@@ -1879,11 +1911,12 @@ int rtnw_scene_prepare(const rtnw_scene_desc* desc, rtnw_prepared** out) {
 
     // one slab, every table 256-byte aligned; the image table has 16 bytes of slack after the pool
     const void* src[N_TABLES] = {sb.recs.data(), sb.leaf.data(), sb.rec_xf.data(), sb.wnodes.data(), sb.gate_leaves.data(),
-                                 desc->xforms, desc->materials, desc->textures, ranvec.data(), perm.data(), desc->images};
+                                 desc->xforms, desc->materials, desc->textures, ranvec.data(), perm.data(), desc->images, sb.lights.data()};
     const size_t sz[N_TABLES] = {sb.recs.size() * sizeof(rec), sb.leaf.size() * sizeof(int32_t), sb.rec_xf.size() * sizeof(uint32_t),
                                  sb.wnodes.size() * sizeof(float4), sb.gate_leaves.size() * sizeof(int2),
                                  (size_t)desc->n_xform_ops * sizeof(rtnw_xform_op), (size_t)desc->n_materials * sizeof(rtnw_material),
-                                 (size_t)desc->n_textures * sizeof(rtnw_texture), 256 * sizeof(float4), 768, (size_t)desc->image_bytes + 16};
+                                 (size_t)desc->n_textures * sizeof(rtnw_texture), 256 * sizeof(float4), 768, (size_t)desc->image_bytes + 16,
+                                 sb.lights.size() * sizeof(float4)};
     rtnw_prepared* P = new rtnw_prepared();
     P->bytes = layout256(sz, N_TABLES, P->off);
     void* pin = nullptr;
@@ -1900,6 +1933,7 @@ int rtnw_scene_prepare(const rtnw_scene_desc* desc, rtnw_prepared** out) {
     P->fast_node_base = sb.fast_base;
     P->n_materials = desc->n_materials;
     P->n_textures = desc->n_textures;
+    P->n_lights = (int32_t)(sb.lights.size() / 2);
     *out = P;
     return RTNW_OK;
 }
@@ -1952,6 +1986,8 @@ int rtnw_scene_upload_prepared(rtnw_ctx* ctx, const rtnw_prepared* P, rtnw_scene
     s->view.fast_node_base = P->fast_node_base;
     s->view.n_materials = P->n_materials;
     s->view.n_textures = P->n_textures;
+    s->lights = reinterpret_cast<const float4*>(base + o[T_LIGHTS]);
+    s->n_lights = P->n_lights;
     *out = s;
     return RTNW_OK;
 }

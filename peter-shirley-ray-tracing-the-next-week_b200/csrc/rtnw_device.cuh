@@ -1250,6 +1250,92 @@ __device__ __forceinline__ bool material_scatter(const scene_view& S, int mat, c
     return true;
 }
 
+// ------------------------------------------------------------------------------------------------ light sampling
+// RTNW_F_LIGHT_SAMPLING (include/rtnw.h): a light of the table is two float4, a = {a0, a1, b0, b1} (rectangle) or {cx, cy, cz, r}
+// (sphere), b = {plane offset k, area, kind bits, record bits}.  tests/light_oracle.c restates these functions draw for draw.
+__device__ __forceinline__ f3 cross(f3 a, f3 b) { return mk3(a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x); }
+
+// p_k(e): the solid-angle density with which light k samples the unit direction e from p; 0 where the ray (p, e) misses it
+template <int N, int A, int B>
+__device__ __forceinline__ float rect_pdf(float4 la, float4 lb, f3 p, f3 e) {
+    const float* o = &p.x;
+    const float* d = &e.x;
+    const float t = (lb.x - o[N]) / d[N];
+    if (!(t > 0.f)) return 0.f;
+    const float a = o[A] + t * d[A], b = o[B] + t * d[B];
+    if (a < la.x || a > la.y || b < la.z || b > la.w) return 0.f;
+    return t * t / (fabsf(d[N]) * lb.y);
+}
+__device__ __forceinline__ float light_pdf(const float4* __restrict__ lights, int k, f3 p, f3 e) {
+    const float4 la = __ldg(&lights[2 * k]), lb = __ldg(&lights[2 * k + 1]);
+    switch (__float_as_int(lb.z)) {
+        case RTNW_PRIM_RECT_XY: return rect_pdf<2, 0, 1>(la, lb, p, e);
+        case RTNW_PRIM_RECT_XZ: return rect_pdf<1, 0, 2>(la, lb, p, e);
+        case RTNW_PRIM_RECT_YZ: return rect_pdf<0, 1, 2>(la, lb, p, e);
+        default: {  // sphere: uniform in the cone it subtends
+            const f3 oc = mk3(la.x, la.y, la.z) - p;
+            const float d2 = dot(oc, oc), r2 = la.w * la.w;
+            if (!(d2 > r2)) return 0.f;
+            const float cmax = sqrtf(1.f - r2 / d2);
+            if (!(dot(e, unit_vector(oc)) >= cmax)) return 0.f;
+            return 1.f / (6.28318531f * (1.f - cmax));
+        }
+    }
+}
+// a unit direction towards light k from p; false when p is inside or on a sphere light
+__device__ __forceinline__ bool sample_light(const float4* __restrict__ lights, int k, f3 p, rng_t& g, f3& d) {
+    const float4 la = __ldg(&lights[2 * k]), lb = __ldg(&lights[2 * k + 1]);
+    const float u1 = g.draw(), u2 = g.draw();
+    const int kind = __float_as_int(lb.z);
+    if (kind != RTNW_PRIM_SPHERE) {
+        const float a = la.x + u1 * (la.y - la.x), b = la.z + u2 * (la.w - la.z);
+        const f3 q = kind == RTNW_PRIM_RECT_XY ? mk3(a, b, lb.x) : (kind == RTNW_PRIM_RECT_XZ ? mk3(a, lb.x, b) : mk3(lb.x, a, b));
+        d = unit_vector(q - p);  // unit length like the sphere's: the scattered ray's t_min stays a distance of ~0.001, as in the reference branch
+        return true;
+    }
+    const f3 oc = mk3(la.x, la.y, la.z) - p;
+    const float d2 = dot(oc, oc), r2 = la.w * la.w;
+    if (!(d2 > r2)) return false;
+    const float cmax = sqrtf(1.f - r2 / d2);
+    const float z = 1.f + u2 * (cmax - 1.f), phi = 6.28318531f * u1, s = sqrtf(1.f - z * z);
+    const f3 w = unit_vector(oc);
+    const f3 v = unit_vector(cross(w, fabsf(w.x) > 0.9f ? mk3(0.f, 1.f, 0.f) : mk3(1.f, 0.f, 0.f)));
+    const f3 u = cross(w, v);
+    d = (cosf(phi) * s) * u + (sinf(phi) * s) * v + z * w;
+    return true;
+}
+// material_scatter with the one-sample light mixture for lambertian and isotropic bounces (n_lights > 0, RTNW_F_EMIT on)
+__device__ __forceinline__ bool mixture_scatter(const scene_view& S, const float4* __restrict__ lights, int n_lights, int mat,
+                                                const ray_t& r_in, const surf_t& s, rng_t& g, f3& attenuation, ray_t& scattered) {
+    const float4 m0 = __ldg(reinterpret_cast<const float4*>(S.materials + mat));
+    const uint32_t kind = __float_as_uint(m0.x);
+    const bool mix = kind == RTNW_MAT_LAMBERTIAN || kind == RTNW_MAT_ISOTROPIC;
+    const float u = mix ? g.draw() : 1.f;
+    if (u < 0.5f) {  // light branch
+        const int k = min((int)(2.f * u * (float)n_lights), n_lights - 1);
+        if (!sample_light(lights, k, s.p, g, scattered.d)) return false;
+        scattered.o = s.p;
+        scattered.time = kind == RTNW_MAT_LAMBERTIAN ? r_in.time : 0.f;
+        attenuation = texture_value(S, __float_as_int(m0.y), s.u, s.v, s.p);
+    } else if (!material_scatter(S, mat, r_in, s, g, attenuation, scattered)) {
+        return false;
+    }
+    if (!mix) return true;
+    const f3 e = unit_vector(scattered.d);
+    float p_ref = 0.0795774715f;  // isotropic: 1 / (4 pi)
+    if (kind == RTNW_MAT_LAMBERTIAN) {
+        const float c = dot(e, s.n);
+        if (!(c > 0.f)) return false;
+        p_ref = c * c * c * 0.636619772f;  // (2 / pi) cos^3
+    }
+    float sum = 0.f;
+#pragma unroll 1
+    for (int k = 0; k < n_lights; ++k) sum += light_pdf(lights, k, s.p, e);
+    const float w = p_ref / (0.5f * p_ref + 0.5f * (sum / (float)n_lights));
+    attenuation = w * attenuation;
+    return true;
+}
+
 // ------------------------------------------------------------------------------------------------ camera
 // PSC/main.cpp:305-306 + PSC/camera.h:41-56.  Draw order of the path's sequential stream: jitter u, jitter v,
 // disk (first draw -> y, second -> x, g++ right-to-left), time.
