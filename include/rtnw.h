@@ -233,7 +233,7 @@ typedef struct rtnw_stats {
     float kernel_ms;       /* device time of the render kernel(s), CUDA events */
     float total_ms;        /* including copies done inside the call */
     int32_t kernel_launches; /* k_render, + k_finish_fixed when the samples of a pixel were cut into more than one range */
-    int32_t sample_ranges;   /* (pixel, sample range) work items per pixel of this call; their partial sums are added in 64-bit fixed point (order independent) */
+    int32_t sample_ranges;   /* (pixel, sample range) work items per pixel of this call; their partial sums are added exactly in fixed point (order independent) and rounded once, see rtnw_plan_sample_ranges */
 } rtnw_stats;
 
 typedef struct rtnw_ray {
@@ -320,7 +320,11 @@ int rtnw_render_device(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera
  * (host arithmetic only, no device needed).  Writes n+1 cumulative boundaries cum[0..n] (cum[0] = 0, cum[n] = total,
  * total = the most samples a pixel has in the call) and returns n (<= cap), or a negative status.  Range c of a pixel
  * with m <= total samples covers its samples k in [cum[c]*m/total, cum[c+1]*m/total): the ranges of every pixel are
- * disjoint and cover all of its samples; their partial sums are added exactly, in 64-bit fixed point (rtnw_stats.sample_ranges = n). */
+ * disjoint and cover all of its samples (rtnw_stats.sample_ranges = n).  With n > 1 the float32 partial sums of a pixel's ranges
+ * (each summed in sample order from 0) are reduced exactly: every finite partial is rounded once, to nearest with ties to
+ * even, to a multiple of 2^-54; these are summed exactly (no clamp, no overflow, in any order); the sum is rounded once to
+ * float32, to nearest with ties to even, +-inf beyond FLT_MAX.  A NaN partial, or +inf and -inf partials together, make the
+ * pixel NaN; +inf or -inf partials alone make it that infinity.  With n = 1 the pixel is its float sum. */
 int rtnw_plan_sample_ranges(const rtnw_render_params* params, int32_t* cum, int32_t cap);
 
 /* Output stage on the device, PSC/main.cpp:315-325: col = sums/ns (vec3::operator/=: multiply by float(1.0/ns)), sqrt gamma,

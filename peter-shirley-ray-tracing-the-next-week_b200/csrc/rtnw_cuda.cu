@@ -31,7 +31,7 @@ struct render_args {
     rtnw_camera cam;
     rtnw_render_params p;
     float* accum;                 // nx*ny*3 sums, index (j*nx+i)*3+c
-    unsigned long long* fixed;    // chunks > 1: nx*ny*3 fixed-point sums (add_fixed / k_finish_fixed), all zero between renders
+    unsigned long long* fixed;    // chunks > 1: nx*ny*3 fixed-point sums, RTNW_FIXED_WORDS planes (add_fixed / k_finish_fixed), all zero between renders
     int chunks;                   // each pixel's samples are cut into this many contiguous ranges, one work item each
     int chunk_total;              // range c of a pixel with n samples: k in [cum[c]*n/total, cum[c+1]*n/total)
     int chunk_cum[RTNW_MAX_CHUNKS + 1];
@@ -40,23 +40,94 @@ struct render_args {
     int n_lights;
 };
 
-// Partial sums of the sample ranges of a pixel are added in 64-bit fixed point with integer atomics: integer addition
-// commutes, so the pixel's sum is the same bits whatever order the ranges finish in, with ONE plane of scratch instead of
-// one float plane per range.  Value = round(v * 2^41), always even; bit 0 is a sticky "not a number" flag (a NaN or infinite
-// partial sum — only possible without RTNW_F_DE_NAN — makes the pixel NaN, as `col += temp` does in the reference).
-// Resolution 4.5e-13, range +-2^22 (larger partial sums saturate; radiance sums are < 1e5).
-__device__ __forceinline__ void add_fixed(unsigned long long* dst, float v) {
-    if (v - v == 0.f) {  // finite
-        const float c = fminf(fmaxf(v, -4194303.f), 4194303.f);
-        const long long q = __double2ll_rn((double)c * 1099511627776.0) << 1;  // 2^40, then << 1
-        if (q != 0) atomicAdd(dst, (unsigned long long)q);
+// Partial sums of the sample ranges of a pixel are added in fixed point with integer atomics: integer addition commutes,
+// so the pixel's sum is the same bits whatever order the ranges finish in, with four planes of scratch however many ranges
+// there are.  A finite partial sum v is rounded once (to nearest, ties to even) to an integer q of units 2^-54,
+// |q| < 2^182, and q is cut into four digits with the sign of v: q = a + b 2^14 + c 2^68 + d 2^125, with a < 2^14, b < 2^54,
+// c, d < 2^57.  Each digit has a word of its own, in four planes of nx*ny*3 words: b * 8 (plane 0), a, c, d.  64 digits of
+// < 2^57 sum to less than 2^63, so no word overflows and no carry has to be taken at add time: every add is a
+// fire-and-forget atomic, and only words whose digit is not 0 are touched.  A partial sum in [2^-17, 2^14) has only b, so
+// it costs one atomic on one plane of 8 bytes per channel.  Nothing is clamped: 64 ranges of FLT_MAX fit.  Bits 0-2 of
+// plane 0 are sticky flags for a NaN (1), +inf (2) and -inf (4) partial sum (only possible without RTNW_F_DE_NAN), which
+// from_fixed turns into what a float sum of the partials gives in any order.
+#define RTNW_FIXED_WORDS 4  // per channel
+__device__ __forceinline__ unsigned long long fixed_digit(unsigned m, int sh, int bits) {  // bits [.., bits) of m * 2^sh
+    if (sh >= 64 || sh <= -24) return 0ull;
+    const unsigned long long x = sh >= 0 ? (unsigned long long)m << sh : (unsigned long long)m >> -sh;
+    return x & ((1ull << bits) - 1ull);
+}
+__device__ __noinline__ void add_fixed_wide(unsigned long long* dst, unsigned long long plane, float v) {
+    const unsigned b = __float_as_uint(v), e = (b >> 23) & 255u;
+    if (e == 255u) {  // NaN or infinite
+        atomicOr(dst, (b & 0x7fffffu) ? 1ull : (b >> 31) ? 4ull : 2ull);
+        return;
+    }
+    const unsigned m = e ? (b & 0x7fffffu) | 0x800000u : b & 0x7fffffu;  // |v| = m * 2^(max(e,1) - 150)
+    const int s = (int)max(e, 1u) - 96;                                  // |v| * 2^54 = m * 2^s
+    unsigned long long d[RTNW_FIXED_WORDS];                              // b, a, c, d
+    if (s < 0) {  // round m * 2^s to an integer, ties to even (m < 2^24: 0 from s = -25 down)
+        if (s < -25) return;
+        const unsigned r = (unsigned)-s, q = m >> r, rem = m & ((1u << r) - 1u), half = 1u << (r - 1u);
+        const unsigned long long qr = q + (rem > half || (rem == half && (q & 1u)));
+        d[0] = qr >> 14; d[1] = qr & 0x3fffull; d[2] = 0ull; d[3] = 0ull;
     } else {
-        atomicOr(dst, 1ull);
+        d[0] = fixed_digit(m, s - 14, 54);
+        d[1] = fixed_digit(m, s, 14);
+        d[2] = fixed_digit(m, s - 68, 57);
+        d[3] = fixed_digit(m, s - 125, 57);
+    }
+    d[0] <<= 3;
+#pragma unroll
+    for (int i = 0; i < RTNW_FIXED_WORDS; ++i)
+        if (d[i]) atomicAdd(dst + i * plane, (b >> 31) ? 0ull - d[i] : d[i]);
+}
+__device__ __forceinline__ void add_fixed(unsigned long long* dst, unsigned long long plane, float v) {
+    const unsigned b = __float_as_uint(v), e = (b >> 23) & 255u;
+    if (e - 110u <= 30u) {  // |v| in [2^-17, 2^14): b = m * 2^(e - 110) exactly, a = c = d = 0
+        const unsigned long long d = (unsigned long long)((b & 0x7fffffu) | 0x800000u) << (e - 107u);  // b * 8
+        atomicAdd(dst, (b >> 31) ? 0ull - d : d);
+    } else if (v != 0.f) {
+        add_fixed_wide(dst, plane, v);
     }
 }
-__device__ __forceinline__ float from_fixed(unsigned long long u) {
-    if (u & 1ull) return __int_as_float(0x7fc00000);
-    return (float)((double)(long long)u * (1.0 / 2199023255552.0));  // 2^-41, one rounding
+
+// The four words of one channel as a float: the exact sum rounded once, to nearest even (+-inf beyond FLT_MAX); the flags
+// as a float sum of the partials gives them: NaN, or +inf and -inf together -> NaN; +inf alone -> +inf; -inf alone -> -inf.
+__device__ __forceinline__ float from_fixed(unsigned long long wb, unsigned long long wa, unsigned long long wc, unsigned long long wd) {
+    const unsigned f = (unsigned)wb & 7u;
+    if ((f & 1u) || f == 6u) return __int_as_float(0x7fc00000);
+    if (f) return __int_as_float(f == 2u ? 0x7f800000 : 0xff800000);
+    // carries between the digit sums (each < 2^63 in magnitude): ra, rb, rc >= 0, the sign in td
+    const long long sa = (long long)wa, sb = ((long long)wb >> 3) + (sa >> 14), sc = (long long)wc + (sb >> 54);
+    const long long td = (long long)wd + (sc >> 57);
+    const unsigned long long ra = (unsigned long long)sa & 0x3fffull, rb = (unsigned long long)sb & ((1ull << 54) - 1ull),
+                             rc = (unsigned long long)sc & ((1ull << 57) - 1ull);
+    // one 192-bit two's-complement integer (|sum| < 2^188): ra at bit 0, rb at 14, rc at 68, td at 125
+    unsigned long long w0 = ra | (rb << 14), w1 = (rb >> 50) | (rc << 4) | ((unsigned long long)td << 61),
+                       w2 = (unsigned long long)(td >> 3);
+    const bool neg = td < 0;
+    if (neg) {
+        w0 = ~w0 + 1ull;
+        w1 = ~w1 + (w0 == 0ull);
+        w2 = ~w2 + (w0 == 0ull && w1 == 0ull);
+    }
+    // the top 64 bits of the magnitude, the bits below folded into bit 0: one rounding in __ull2float_rn
+    unsigned long long top = w0;
+    int e = 0;  // magnitude ~ top * 2^e
+    if (w2) {
+        const int z = __clzll((long long)w2);  // >= 4
+        top = (w2 << z) | (w1 >> (64 - z));
+        top |= ((w1 << z) | w0) != 0ull;
+        e = 128 - z;
+    } else if (w1) {
+        const int z = __clzll((long long)w1);
+        top = z ? (w1 << z) | (w0 >> (64 - z)) : w1;
+        top |= (z ? w0 << z : w0) != 0ull;
+        e = 64 - z;
+    }
+    // times 2^(e - 54), e - 54 in [-54, 70]: exact, or +inf when the rounded value reaches 2^128
+    const float v = __ull2float_rn(top) * __int_as_float((e - 54 + 127) << 23);
+    return neg ? -v : v;
 }
 
 // the reference-exact kernels traverse one BVH item at a time; the RTNW_F_FAST_BVH kernels two together (two ray frames)
@@ -66,7 +137,7 @@ template <bool FAST> using block_smem = coop_smem<FAST ? 2 : 1>;
 //
 // One thread owns one work item at a time — a pixel and a contiguous range of its samples (pick_chunks): the samples
 // are traced back to back and summed in sample order like `col += temp` in the reference; the partial sums of a pixel's
-// ranges are added in 64-bit fixed point (add_fixed: integer atomics commute, so a pixel's sum never depends on scheduling).  A
+// ranges are added exactly in fixed point (add_fixed: integer atomics commute, so a pixel's sum never depends on scheduling).  A
 // thread that finishes its item pulls the next one from a global counter (warp-aggregated atomic); a thread whose path
 // ends starts the next sample of its item in the same round (path regeneration, which absorbs the 51-bounce tail).
 //
@@ -120,7 +191,8 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
                 const int4 it = sm.span[me];  // z = pixel, w = sample range
                 if (P.chunks > 1) {  // partial sum of one sample range
                     unsigned long long* dst = P.fixed + 3ull * (unsigned long long)it.z;
-                    add_fixed(dst, acc.x); add_fixed(dst + 1, acc.y); add_fixed(dst + 2, acc.z);
+                    const unsigned long long plane = 3ull * (unsigned long long)nx * (unsigned long long)ny;
+                    add_fixed(dst, plane, acc.x); add_fixed(dst + 1, plane, acc.y); add_fixed(dst + 2, plane, acc.z);
                 } else {
                     float* dst = P.accum + 3ull * (unsigned long long)it.z;
                     if (accumulate) { dst[0] += acc.x; dst[1] += acc.y; dst[2] += acc.z; }
@@ -646,18 +718,19 @@ __global__ void k_quantize(const float* __restrict__ sums, int nx, int ny, float
     }
 }
 
-// chunks > 1: the fixed-point sums of the subset's pixels become float sums (added to accum with RTNW_F_ACCUMULATE) and the
-// plane is cleared for the next render
-__global__ void k_finish_fixed(unsigned long long* __restrict__ fixed, int pixel_begin, int pixel_stride, int pixel_count,
-                               int accumulate, float* __restrict__ accum) {
+// chunks > 1: the fixed-point sums of the subset's pixels (4 planes of nx*ny*3 words) become float sums (added to accum
+// with RTNW_F_ACCUMULATE) and the plane is cleared for the next render
+__global__ void k_finish_fixed(unsigned long long* __restrict__ fixed, unsigned long long plane, int pixel_begin, int pixel_stride,
+                               int pixel_count, int accumulate, float* __restrict__ accum) {
     const int q = blockIdx.x * blockDim.x + threadIdx.x;
     if (q >= pixel_count) return;
-    const unsigned long long at = 3ull * (unsigned long long)(pixel_begin + q * pixel_stride);
+    const unsigned long long pix = (unsigned long long)(pixel_begin + q * pixel_stride);
+    unsigned long long* w = fixed + 3ull * pix;
 #pragma unroll
     for (int c = 0; c < 3; ++c) {
-        const float v = from_fixed(fixed[at + c]);
-        fixed[at + c] = 0ull;
-        if (accumulate) accum[at + c] += v; else accum[at + c] = v;
+        const float v = from_fixed(w[c], w[c + plane], w[c + 2 * plane], w[c + 3 * plane]);
+        w[c] = 0ull; w[c + plane] = 0ull; w[c + 2 * plane] = 0ull; w[c + 3 * plane] = 0ull;
+        if (accumulate) accum[3ull * pix + c] += v; else accum[3ull * pix + c] = v;
     }
 }
 
@@ -1478,7 +1551,7 @@ int launch_render(rtnw_ctx* ctx, const render_args& a, cudaStream_t st) {
 // in a tail as long as the most expensive pixel — at 100 spp about 14 ms of 220, during which most of the device idles —
 // and an image with fewer pixels than the device has resident threads (the reference's own 200x100 default is 20 000)
 // never fills it.  So every pixel's samples are cut into contiguous ranges, handed out range-major; a range's partial
-// sum is added to the pixel's 64-bit fixed-point sum (add_fixed) and k_finish_fixed turns the plane into floats
+// sum is added exactly to the pixel's fixed-point sum (add_fixed) and k_finish_fixed rounds it once to float
 // (reproducible bit for bit; differs from the one-range float sum only by rounding).  Ranges are four samples long (more when
 // there are more than ~110 samples per pixel) and the last ones shrink to 4, 2, 1, 1, because the kernel's tail is as long
 // as the longest item still running when the items run out.  Measured on the bench workload: 453 (1 range) / 477 (2) /
@@ -1543,13 +1616,13 @@ int render_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam
     int rc = RTNW_OK;
     pick_chunks(a.p, a);
     a.fixed = nullptr;
-    const size_t plane = (size_t)p->nx * p->ny * 3;
+    const size_t plane = (size_t)p->nx * p->ny * 3, words = plane * RTNW_FIXED_WORDS;
     if (a.chunks > 1) {
-        if (ctx->fixed_words < plane) {
+        if (ctx->fixed_words < words) {
             CUDA_TRY(cudaStreamSynchronize(st));
-            rc = grow(&ctx->fixed, &ctx->fixed_words, plane, "cudaMalloc of the sample-range accumulation plane failed");
+            rc = grow(&ctx->fixed, &ctx->fixed_words, words, "cudaMalloc of the sample-range accumulation plane failed");
             if (rc != RTNW_OK) return rc;
-            CUDA_TRY(cudaMemsetAsync(ctx->fixed, 0, plane * sizeof(unsigned long long), st));  // k_finish_fixed keeps it zero afterwards
+            CUDA_TRY(cudaMemsetAsync(ctx->fixed, 0, words * sizeof(unsigned long long), st));  // k_finish_fixed keeps it zero afterwards
         }
         a.fixed = ctx->fixed;
     }
@@ -1561,7 +1634,7 @@ int render_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam
     });
     if (rc != RTNW_OK) return rc;
     if (a.chunks > 1) {
-        k_finish_fixed<<<(a.p.pixel_count + 255) / 256, 256, 0, st>>>(a.fixed, a.p.pixel_begin, a.p.pixel_stride, a.p.pixel_count,
+        k_finish_fixed<<<(a.p.pixel_count + 255) / 256, 256, 0, st>>>(a.fixed, plane, a.p.pixel_begin, a.p.pixel_stride, a.p.pixel_count,
                                                                       (p->flags & RTNW_F_ACCUMULATE) ? 1 : 0, accum_dev);
         CUDA_TRY(cudaGetLastError());
     }

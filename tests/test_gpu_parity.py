@@ -374,7 +374,7 @@ def test_rotated_sample_split_is_an_even_partition(rtnw, ctx, ns, world):
 
 def test_small_image_sample_ranges(rtnw, ctx):
     """A pixel with enough samples is rendered as several (sample range, pixel) work items whose partial sums are added
-    in 64-bit fixed point: same paths, same rays, the sums equal up to float rounding, and still bitwise reproducible.
+    exactly in fixed point: same paths, same rays, the sums equal up to float rounding, and still bitwise reproducible.
     rtnw_render_params.sample_ranges forces the number of ranges (1 = one thread per pixel)."""
     import torch
     hs = rtnw.HostScene("cornell_smoke")
@@ -426,7 +426,8 @@ def test_fixed_point_range_sums_keep_nan_and_pixel_subsets(rtnw, ctx):
 
 def test_device_epilogue_equals_host_epilogue(rtnw, ctx):
     """rtnw_quantize_device (gamma + quantise + clamp on the GPU, after the reduce) is bit-identical to the host epilogue
-    rtnw_host_quantize, which restates PSC/main.cpp:315-325; includes values > 1 (light), 0 and NaN-free negatives."""
+    rtnw_host_quantize, which restates PSC/main.cpp:315-325; includes values > 1 (light), 0, and every sum the sample-range
+    reduction can return: negatives, NaN, +-inf, -0 and means so large that 255.99*sqrt(mean) leaves the int range."""
     import torch
     hs = rtnw.HostScene("cornell_box")
     ds = ctx.upload(hs.desc_ptr)
@@ -441,6 +442,15 @@ def test_device_epilogue_equals_host_epilogue(rtnw, ctx):
     t = torch.from_numpy(synth).cuda()
     for n in (1, 3, 100, 1000):
         assert np.array_equal(ctx.quantize_device(t.data_ptr(), nx, ny, n, True), rtnw.quantize(synth, n, True))
+    special = np.float32([np.nan, np.inf, -np.inf, -0.0, -1.0, -1e-30, -3e38, 1e20, 7.0377e13, 7.0379e13, 3.4e38, 1e-45])
+    synth = (rng.standard_normal((ny, nx, 3)) * 10.0 ** rng.integers(-30, 37, (ny, nx, 3))).astype(np.float32)
+    synth.reshape(-1)[:special.size * 50] = np.tile(special, 50)
+    t = torch.from_numpy(synth).cuda()
+    for n in (1, 3, 100, 1000):
+        for clamp in (True, False):
+            want = rtnw.quantize(synth, n, clamp)
+            assert np.array_equal(ctx.quantize_device(t.data_ptr(), nx, ny, n, clamp), want)
+    assert (want == np.int32(-2 ** 31)).any()  # NaN and out-of-range means did reach the x86 conversion result
     ds.close()
 
 
