@@ -205,6 +205,39 @@ enum rtnw_background { RTNW_BG_BLACK = 0 /* PSC/main.cpp:44 */, RTNW_BG_SKY = 1 
  * keep the reference's scatter.  The sample stream stays keyed by (seed, pixel, sample). */
 #define RTNW_MAX_LIGHTS 16
 
+#define RTNW_F_NEXT_EVENT  128u /* same expected image, other noise (DESIGN.md §5 measures it): next-event estimation.  Lambertian
+                                   and isotropic vertices trace a shadow ray to a point sampled on the scene's light table, weighted
+                                   by the balance heuristic against the reference's own scatter density; the path itself is the
+                                   exact mode's, vertex for vertex (below).  Honoured by rtnw_render, rtnw_render_device,
+                                   rtnw_render_multi and the colour of rtnw_render_aov_multi, which reject it together with
+                                   RTNW_F_LIGHT_SAMPLING (RTNW_ERR_INVALID); accepted and ignored by every other entry point.  A
+                                   bit-for-bit no-op when the light table is empty or RTNW_F_EMIT is off */
+
+/* Next-event estimation (RTNW_F_NEXT_EVENT).  L, p_k(e) and p_ref(e) as for light sampling above (p_ref(e) = 0 for a lambertian
+ * vertex where c = e.n <= 0), and
+ *     p_L(e) = (sum_k p_k(e), summed in table order) / L,     W(e) = p_ref(e) / (p_ref(e) + p_L(e)).
+ * The path's rays, draws, scatters and attenuations are the exact mode's, bit for bit: every number the estimator adds is a keyed
+ * Philox number, not a draw of the path's stream.  Only the accounting of radiance changes.  T = the path's throughput: 1 at the
+ * camera ray, T <- T * attenuation at each bounce.  A ray of throughput T that finds a light's emission Le adds (T * Le) * w to
+ * the path's radiance, in the order of the rays, with the weight w below.
+ * At a vertex x that the path's query of depth d finds, when x's material is lambertian or isotropic, d < max_depth, RTNW_F_EMIT
+ * is on and L > 0:
+ *   continuation: material::scatter from the path's stream, unchanged; T <- T * a, a = the texture value at x (the reference's
+ *     attenuation); with e' = unit(scattered.d), w_B = p_L(e') > 0 ? W(e') : 1.
+ *   shadow ray: (u0, u1, u2) = u01 of words x, y, z of Philox(counter = (0xFFFFFFFF, 1 + d, sample, pixel), key = seed); u01(w) =
+ *     (w >> 8) 2^-24.  Light k = min((int)(u0 L), L - 1), and e = the light branch's direction towards light k from x.p with the
+ *     draws (u1, u2) in place of draw(), draw().  No shadow ray when that fails (x.p inside a sphere light) or p_ref(e) = 0.  The
+ *     ray (x.p, e, scattered.time) is one closest-hit query over [t_min, t_max] like the path's own, traced before the
+ *     continuation; its media draw with the depth word 0x80000000 | d, where the path's own queries use 1 + depth <= 2^31.  If
+ *     its closest hit is a record of the light table (any light, not only k), it adds (T * Le) * W(e), T = the updated throughput
+ *     T * a and Le = the emitted texture value at that hit's (u, v, p).
+ * The path's own ray that finds a record of the light table adds its emission with w = the w_B of the vertex it left when that
+ * vertex was one as above, and every other emission (the camera ray's, after a metal or dielectric bounce, emitters outside the
+ * table) and the sky with w = 1.  The weights lie in [0, 1], and W(e) + p_L(e) / (p_ref(e) + p_L(e)) = 1: the shadow ray's
+ * term is (T * a) Le p_ref / p_L times the balance weight p_L / (p_ref + p_L), the path's is (T * a) Le times p_ref / (p_ref + p_L),
+ * so every pixel's expectation is the reference's (DESIGN.md §5).  RTNW_F_DE_NAN applies to the path's total.  rtnw_stats.rays
+ * counts the shadow queries; paths is unchanged. */
+
 typedef struct rtnw_render_params {
     int32_t nx, ny;
     int32_t sample_begin;   /* this call renders samples s = sample_begin + k*sample_stride, k in [0, sample_count) */

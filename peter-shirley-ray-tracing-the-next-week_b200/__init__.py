@@ -27,6 +27,7 @@ RTNW_ERR_INVALID, RTNW_ERR_CUDA, RTNW_ERR_UNSUPPORTED, RTNW_ERR_NOMEM = -1, -2, 
 BG_BLACK, BG_SKY = 0, 1
 TEXF_BILINEAR = 1
 F_DE_NAN, F_EMIT, F_FAST_BVH, F_COUNTERS, F_ACCUMULATE, F_ROTATE_SAMPLES, F_LIGHT_SAMPLING = 1, 2, 4, 8, 16, 32, 64
+F_NEXT_EVENT = 128
 FLT_MAX = float(np.finfo(np.float32).max)
 
 

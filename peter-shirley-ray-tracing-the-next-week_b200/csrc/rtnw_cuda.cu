@@ -36,7 +36,7 @@ struct render_args {
     int chunk_total;              // range c of a pixel with n samples: k in [cum[c]*n/total, cum[c+1]*n/total)
     int chunk_cum[RTNW_MAX_CHUNKS + 1];
     unsigned long long* ctr;      // [0] next pixel, [1] rays, [2] box tests, [3] primitive tests, [4] task stack overflows
-    const float4* lights;         // RTNW_F_LIGHT_SAMPLING: the scene's light table (2 float4 per light), read by k_render<.., true> only
+    const float4* lights;         // the scene's light table (2 float4 per light), read by k_render<.., RENDER_MIXTURE / RENDER_NEE> only
     int n_lights;
 };
 
@@ -133,6 +133,38 @@ __device__ __forceinline__ float from_fixed(unsigned long long wb, unsigned long
 // the reference-exact kernels traverse one BVH item at a time; the RTNW_F_FAST_BVH kernels two together (two ray frames)
 template <bool FAST> using block_smem = coop_smem<FAST ? 2 : 1>;
 
+// k_render's estimator, which the host picks (render_launch): the reference's; the one-sample light mixture of
+// RTNW_F_LIGHT_SAMPLING (mixture_scatter); the next-event estimation of RTNW_F_NEXT_EVENT
+enum render_mode { RENDER_EXACT = 0, RENDER_MIXTURE = 1, RENDER_NEE = 2 };
+
+// RTNW_F_NEXT_EVENT's path state that outlives a round, per thread: 10 KB a block, so two blocks still fit an SM, where
+// the same state would take 8 of the 96 registers the traversal has.  A shadow ray has the origin and time of the path's
+// continuation, so only the continuation's direction is stashed while the shadow ray is traced.
+template <int FRAMES>
+struct nee_smem : coop_smem<FRAMES> {
+    float4 nee_d[RTNW_BLOCK];  // xyz = the stashed continuation's direction; w = w_B, the weight of an emission the path's next ray finds
+    float4 nee_l[RTNW_BLOCK];  // xyz = the path's radiance so far; w = the weight of the shadow ray in flight
+};
+template <bool FAST, int MODE>
+using render_smem = typename std::conditional<MODE == RENDER_NEE, nee_smem<FAST ? 2 : 1>, block_smem<FAST>>::type;
+
+// finish_hit for k_render<.., RENDER_NEE>, with (u,v) only where the hit's texture reads them; returns the first float4 of the
+// hit's material (kind, texture, ...).  The other k_render modes inline the same lines: calling this function there changes
+// their register allocation.
+__device__ __forceinline__ float4 shade_hit(const scene_view& S, const ray_t& wr, hit_t& h, surf_t& s) {
+    // does value(u,v,p) of this hit's texture read u,v?  (only image_texture does, PSC/surface_texture.h:19-30;
+    // a checker forwards u,v to its children, so it is treated as if it did)
+    const int mat_id = __float_as_int(__ldg(&S.recs[h.rec].b).w);
+    const float4 m0 = __ldg(reinterpret_cast<const float4*>(S.materials + mat_id));
+    bool want_uv = false;
+    if (__float_as_int(m0.y) >= 0 && __float_as_uint(m0.x) != RTNW_MAT_METAL && __float_as_uint(m0.x) != RTNW_MAT_DIELECTRIC) {
+        const uint32_t tk = __float_as_uint(__ldg(reinterpret_cast<const float4*>(S.textures + __float_as_int(m0.y))).x);
+        want_uv = tk == RTNW_TEX_IMAGE || tk == RTNW_TEX_CHECKER;
+    }
+    finish_hit(S, wr, h, s, want_uv);
+    return m0;
+}
+
 // The sample loop of PSC/main.cpp:299-313 as ONE persistent megakernel.
 //
 // One thread owns one work item at a time — a pixel and a contiguous range of its samples (pick_chunks): the samples
@@ -145,11 +177,13 @@ template <bool FAST> using block_smem = coop_smem<FAST ? 2 : 1>;
 // block-cooperative (coop_closest_hit): list items in lockstep, BVH items as uniform tasks from shared-memory queues.
 // A per-lane traversal state machine was measured at 2-13 active lanes of 32 per instruction (profiles/r1-r3*.txt);
 // this form keeps every phase uniform across the warp.
-// LIGHTS: RTNW_F_LIGHT_SAMPLING with a non-empty light table and RTNW_F_EMIT (mixture_scatter); the host selects it.
-template <bool COUNT, bool FAST, bool LIGHTS>
+// MODE (render_mode): RENDER_MIXTURE and RENDER_NEE run with a non-empty light table and RTNW_F_EMIT only.
+// RENDER_NEE: a thread's round traces either its path's ray or the shadow ray of the path's last vertex; the path's radiance
+// accumulates over its rays in sm.nee_l.
+template <bool COUNT, bool FAST, int MODE>
 __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const render_args P) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
-    typedef block_smem<FAST> SM;
+    typedef render_smem<FAST, MODE> SM;
     SM& sm = *reinterpret_cast<SM*>(smem_raw);
     constexpr unsigned FULL = 0xffffffffu;
     const unsigned lane = threadIdx.x & 31u;
@@ -173,6 +207,7 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
     int me = threadIdx.x % RTNW_BLOCK;  // index of this thread's work item in sm.acc / sm.span
     bool alive = true, need = true, has_item = false;
     int depth = 0;
+    bool shadow = false;  // RENDER_NEE: this round traces the shadow ray of the path's vertex at `depth`
     f3 T = mk3(0.f, 0.f, 0.f);
     ray_t wr;
     wr.o = T; wr.d = mk3(1.f, 1.f, 1.f); wr.time = 0.f;
@@ -182,6 +217,10 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
     unsigned long long box_total = 0, prim_total = 0;
     trav_counters cnt;
     cnt.box_tests = 0; cnt.prim_tests = 0;
+    if constexpr (MODE == RENDER_NEE) {  // and again whenever a path ends
+        sm.nee_l[me] = make_float4(0.f, 0.f, 0.f, 0.f);
+        sm.nee_d[me].w = 1.f;
+    }
 
     for (;;) {
         // ---- next sample of the pixel, or next pixel, PSC/main.cpp:299-308
@@ -248,6 +287,8 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
         // ---- world->hit(r, t_min, t_max, rec), PSC/main.cpp:27
         medium_key mk;
         mk.k0 = k0; mk.k1 = k1; mk.pixel = (uint32_t)sm.span[me].z; mk.sample = g.sample; mk.depth = (uint32_t)depth;
+        if constexpr (MODE == RENDER_NEE)
+            if (shadow) mk.depth += 0x7fffffffu;  // the shadow ray's media draw with the depth word 1 + mk.depth = 0x80000000 | depth
         const bool tracing = alive && !need;  // a pixel that owns no sample of this call has no ray (RTNW_F_ROTATE_SAMPLES, ns < G)
 #ifdef RTNW_ROUND_STATS
         const long long c0 = clock64();
@@ -258,7 +299,85 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
         const long long c1 = clock64();
 #endif
         // ---- one level of color(), PSC/main.cpp:25-46, in iterative form (DESIGN.md §5)
-        if (tracing) {
+        if constexpr (MODE == RENDER_NEE) {
+            if (tracing) {
+                ++n_rays;
+                const float4 st = sm.nee_l[me];
+                f3 L = mk3(st.x, st.y, st.z);
+                float w_shadow = 0.f;  // the weight of a shadow ray this round sets up
+                hit_t h;
+                key_to_hit(P.S, key, P.p.t_max, h);
+                need = true;
+                if (shadow) {  // the light the shadow ray reaches, if any; then the path goes on with its stashed continuation
+                    if (h.rec >= 0 && is_light_record(P.lights, P.n_lights, h.rec)) {
+                        surf_t s;
+                        const float4 m0 = shade_hit(P.S, wr, h, s);
+                        L = L + st.w * (T * texture_value(P.S, __float_as_int(m0.y), s.u, s.v, s.p));
+                    }
+                    const float4 d = sm.nee_d[me];
+                    wr.d = mk3(d.x, d.y, d.z);
+                    ++depth;
+                    shadow = false;
+                    need = false;
+                } else if (h.rec >= 0) {
+                    surf_t s;
+                    const float4 m0 = shade_hit(P.S, wr, h, s);
+                    const uint32_t kind = __float_as_uint(m0.x);
+                    if (kind == RTNW_MAT_DIFFUSE_LIGHT) {
+                        const float w = is_light_record(P.lights, P.n_lights, h.rec) ? sm.nee_d[me].w : 1.f;
+                        L = L + w * (T * texture_value(P.S, __float_as_int(m0.y), s.u, s.v, s.p));
+                    } else if (depth < P.p.max_depth) {
+                        ray_t sc;
+                        f3 att, e;
+                        if (material_scatter(P.S, s.mat, wr, s, g, att, sc)) {  // the path's own continuation, as without the flag
+                            T = T * att;
+                            wr = sc;
+                            need = false;
+                            float w_b = 1.f;
+                            if (kind == RTNW_MAT_LAMBERTIAN || kind == RTNW_MAT_ISOTROPIC) {
+                                const bool lam = kind == RTNW_MAT_LAMBERTIAN;
+                                const f3 e1 = unit_vector(sc.d);
+                                const float pr1 = ref_density(lam, s.n, e1), pl1 = lights_density(P.lights, P.n_lights, s.p, e1);
+                                if (pl1 > 0.f) w_b = pr1 / (pr1 + pl1);
+                                // the shadow ray: keyed numbers, so that the path's stream is the exact mode's
+                                const uint4 u = philox_block(0xffffffffu, 1u + (uint32_t)depth, g.sample, (uint32_t)sm.span[me].z, k0, k1);
+                                const int k = min((int)(u01(u.x) * (float)P.n_lights), P.n_lights - 1);
+                                if (sample_light(P.lights, k, s.p, u01(u.y), u01(u.z), e)) {
+                                    const float pr = ref_density(lam, s.n, e);
+                                    if (pr > 0.f) {
+                                        w_shadow = pr / (pr + lights_density(P.lights, P.n_lights, s.p, e));
+                                        shadow = true;
+                                    }
+                                }
+                            }
+                            if (shadow) {  // same origin and time as the continuation
+                                sm.nee_d[me] = make_float4(sc.d.x, sc.d.y, sc.d.z, w_b);
+                                wr.d = e;
+                            } else {
+                                sm.nee_d[me].w = w_b;
+                                ++depth;
+                            }
+                        }
+                    }
+                } else if (sky) {
+                    L = L + T * sky_color(wr.d);
+                }
+                if (need) {  // the path ended
+                    if (denan) {
+                        if (!(L.x == L.x)) L.x = 0.f;
+                        if (!(L.y == L.y)) L.y = 0.f;
+                        if (!(L.z == L.z)) L.z = 0.f;
+                    }
+                    float4 acc = sm.acc[me];
+                    acc.x += L.x; acc.y += L.y; acc.z += L.z;
+                    sm.acc[me] = acc;
+                    sm.nee_l[me] = make_float4(0.f, 0.f, 0.f, 0.f);
+                    sm.nee_d[me].w = 1.f;
+                } else {
+                    sm.nee_l[me] = make_float4(L.x, L.y, L.z, w_shadow);
+                }
+            }
+        } else if (tracing) {
             ++n_rays;
             f3 L = mk3(0.f, 0.f, 0.f);  // radiance of this path: only its last ray (a light, or the sky) adds any, so it need not live across rounds
             hit_t h;
@@ -281,7 +400,7 @@ __global__ void __launch_bounds__(RTNW_BLOCK, RTNW_MIN_BLOCKS) k_render(const re
                 } else if (depth < P.p.max_depth) {
                     ray_t sc;
                     f3 att;
-                    if (LIGHTS ? mixture_scatter(P.S, P.lights, P.n_lights, s.mat, wr, s, g, att, sc)
+                    if (MODE == RENDER_MIXTURE ? mixture_scatter(P.S, P.lights, P.n_lights, s.mat, wr, s, g, att, sc)
                                : material_scatter(P.S, s.mat, wr, s, g, att, sc)) {
                         T = T * att;
                         wr = sc;
@@ -1072,7 +1191,7 @@ struct rtnw_ctx {
     unsigned char* dn_scratch = nullptr;     // the denoiser's planes for rtnw_denoise_device and rtnw_render_aov_multi
     size_t dn_scratch_bytes = 0;
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;  // rtnw_render's total_ms
-    int blocks_per_sm[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // per k_render instantiation, render_occupancy
+    int blocks_per_sm[12] = {};  // per k_render instantiation, render_occupancy
     // freed scene slabs are kept for the next upload (cudaMalloc/cudaFree synchronise the device and can take
     // milliseconds to hundreds of milliseconds in a process that also hosts another allocator)
     void* spare_slab[2] = {nullptr, nullptr};
@@ -1517,23 +1636,24 @@ int report_stats(rtnw_ctx* ctx, rtnw_stats* stats, rtnw_stats s, bool total) {
     return RTNW_OK;
 }
 
-// resident blocks per SM of k_render<COUNT, FAST, LIGHTS> (cached per context)
-template <bool COUNT, bool FAST, bool LIGHTS>
+// resident blocks per SM of k_render<COUNT, FAST, MODE> (cached per context)
+template <bool COUNT, bool FAST, int MODE>
 int render_occupancy(rtnw_ctx* ctx, int* out) {
-    int& bps = ctx->blocks_per_sm[(COUNT ? 1 : 0) + (FAST ? 2 : 0) + (LIGHTS ? 4 : 0)];
+    int& bps = ctx->blocks_per_sm[(COUNT ? 1 : 0) + (FAST ? 2 : 0) + 4 * MODE];
     if (bps == 0) {
-        CUDA_TRY(cudaFuncSetAttribute(k_render<COUNT, FAST, LIGHTS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(block_smem<FAST>)));
-        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_render<COUNT, FAST, LIGHTS>, RTNW_BLOCK, sizeof(block_smem<FAST>)));
+        constexpr int smem = (int)sizeof(render_smem<FAST, MODE>);
+        CUDA_TRY(cudaFuncSetAttribute(k_render<COUNT, FAST, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        CUDA_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&bps, k_render<COUNT, FAST, MODE>, RTNW_BLOCK, smem));
         if (bps < 1) bps = 1;
     }
     *out = bps;
     return RTNW_OK;
 }
 
-template <bool COUNT, bool FAST, bool LIGHTS>
+template <bool COUNT, bool FAST, int MODE>
 int launch_render(rtnw_ctx* ctx, const render_args& a, cudaStream_t st) {
     int bps = 0;
-    const int rc = render_occupancy<COUNT, FAST, LIGHTS>(ctx, &bps);
+    const int rc = render_occupancy<COUNT, FAST, MODE>(ctx, &bps);
     if (rc != RTNW_OK) return rc;
     int blocks = ctx->sm_count * bps;
     const long long warps_needed = ((long long)a.p.pixel_count * a.chunks + 31) / 32;
@@ -1542,7 +1662,7 @@ int launch_render(rtnw_ctx* ctx, const render_args& a, cudaStream_t st) {
 #ifdef RTNW_TUNING  // A/B builds only (scripts/ab_build.sh): the product library reads no environment on the launch path
     if (const char* e = getenv("RTNW_GRID_BLOCKS")) { const int v = atoi(e); if (v > 0) blocks = v; }
 #endif
-    k_render<COUNT, FAST, LIGHTS><<<blocks, RTNW_BLOCK, sizeof(block_smem<FAST>), st>>>(a);
+    k_render<COUNT, FAST, MODE><<<blocks, RTNW_BLOCK, sizeof(render_smem<FAST, MODE>), st>>>(a);
     CUDA_TRY(cudaGetLastError());
     return RTNW_OK;
 }
@@ -1592,6 +1712,13 @@ int validate_params(const rtnw_render_params* p) {
     return RTNW_OK;
 }
 
+// the calls that honour RTNW_F_LIGHT_SAMPLING and RTNW_F_NEXT_EVENT take one of the two estimators at a time
+int validate_estimator(const rtnw_render_params* p) {
+    if ((p->flags & RTNW_F_LIGHT_SAMPLING) && (p->flags & RTNW_F_NEXT_EVENT))
+        return fail(RTNW_ERR_INVALID, "RTNW_F_LIGHT_SAMPLING and RTNW_F_NEXT_EVENT exclude each other");
+    return RTNW_OK;
+}
+
 // A render in two halves, so that one host thread can keep several devices busy (rtnw_render_multi): render_launch queues
 // everything on stream st and returns; render_finish waits for it and fills stats (kernel_ms from CUDA events on st).
 struct render_ticket {
@@ -1611,8 +1738,10 @@ int render_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam
     a.ctr = ctx->ctr;
     a.lights = scene->lights;
     a.n_lights = scene->n_lights;
-    // light sampling changes nothing without a light to sample or without emission: those renders take the plain kernel
-    const bool lights = (p->flags & RTNW_F_LIGHT_SAMPLING) && (p->flags & RTNW_F_EMIT) && scene->n_lights > 0;
+    // light sampling and next-event estimation change nothing without a light to sample or without emission: those renders
+    // take the plain kernel
+    const bool lit = (p->flags & RTNW_F_EMIT) && scene->n_lights > 0;
+    const int mode = !lit ? RENDER_EXACT : (p->flags & RTNW_F_LIGHT_SAMPLING) ? RENDER_MIXTURE : (p->flags & RTNW_F_NEXT_EVENT) ? RENDER_NEE : RENDER_EXACT;
     int rc = RTNW_OK;
     pick_chunks(a.p, a);
     a.fixed = nullptr;
@@ -1630,7 +1759,11 @@ int render_launch(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam
     CUDA_TRY(cudaEventRecord(ctx->ev0, st));
     rc = by_variant(p->flags, [&](auto count, auto fast) {
         constexpr bool COUNT = decltype(count)::value, FAST = decltype(fast)::value;
-        return lights ? launch_render<COUNT, FAST, true>(ctx, a, st) : launch_render<COUNT, FAST, false>(ctx, a, st);
+        switch (mode) {
+            case RENDER_MIXTURE: return launch_render<COUNT, FAST, RENDER_MIXTURE>(ctx, a, st);
+            case RENDER_NEE: return launch_render<COUNT, FAST, RENDER_NEE>(ctx, a, st);
+            default: return launch_render<COUNT, FAST, RENDER_EXACT>(ctx, a, st);
+        }
     });
     if (rc != RTNW_OK) return rc;
     if (a.chunks > 1) {
@@ -2099,7 +2232,7 @@ int rtnw_render_device(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera
     int rc = check_ctx(ctx);
     if (rc != RTNW_OK) return rc;
     if (!scene || !cam || !accum_rgb_dev) return fail(RTNW_ERR_INVALID, "null argument");
-    if ((rc = validate_params(params)) != RTNW_OK) return rc;
+    if ((rc = validate_params(params)) != RTNW_OK || (rc = validate_estimator(params)) != RTNW_OK) return rc;
     cudaStream_t st = cuda_stream ? static_cast<cudaStream_t>(cuda_stream) : cudaStreamLegacy;  // NULL = the legacy default stream
     return render_core(ctx, scene, cam, params, accum_rgb_dev, st, stats);
 }
@@ -2109,7 +2242,7 @@ int rtnw_render(rtnw_ctx* ctx, const rtnw_scene* scene, const rtnw_camera* cam, 
     int rc = check_ctx(ctx);
     if (rc != RTNW_OK) return rc;
     if (!scene || !cam || !accum_rgb) return fail(RTNW_ERR_INVALID, "null argument");
-    if ((rc = validate_params(params)) != RTNW_OK) return rc;
+    if ((rc = validate_params(params)) != RTNW_OK || (rc = validate_estimator(params)) != RTNW_OK) return rc;
     if (params->pixel_count != 0 || (params->flags & RTNW_F_ACCUMULATE))
         return fail(RTNW_ERR_INVALID, "pixel subsets / RTNW_F_ACCUMULATE need rtnw_render_device (the host entry point returns whole images)");
     const size_t floats = (size_t)params->nx * params->ny * 3;
@@ -2460,7 +2593,7 @@ int rtnw_scene_upload_multi(rtnw_multi* m, const rtnw_scene_desc* desc, rtnw_mul
 // rtnw_render_multi and rtnw_render_aov_multi accept whole frames only
 static int validate_multi_params(const rtnw_render_params* params, const char* who) {
     int rc = validate_params(params);
-    if (rc != RTNW_OK) return rc;
+    if (rc != RTNW_OK || (rc = validate_estimator(params)) != RTNW_OK) return rc;
     if (params->pixel_count != 0 || params->sample_begin != 0 || params->sample_stride != 1 ||
         (params->flags & (RTNW_F_ACCUMULATE | RTNW_F_ROTATE_SAMPLES)))
         return fail(RTNW_ERR_INVALID, std::string(who) + " renders whole frames: sample_begin 0, sample_stride 1, no pixel subset, no ACCUMULATE / ROTATE flags");

@@ -1282,10 +1282,9 @@ __device__ __forceinline__ float light_pdf(const float4* __restrict__ lights, in
         }
     }
 }
-// a unit direction towards light k from p; false when p is inside or on a sphere light
-__device__ __forceinline__ bool sample_light(const float4* __restrict__ lights, int k, f3 p, rng_t& g, f3& d) {
+// a unit direction towards light k from p for the draws (u1, u2); false when p is inside or on a sphere light
+__device__ __forceinline__ bool sample_light(const float4* __restrict__ lights, int k, f3 p, float u1, float u2, f3& d) {
     const float4 la = __ldg(&lights[2 * k]), lb = __ldg(&lights[2 * k + 1]);
-    const float u1 = g.draw(), u2 = g.draw();
     const int kind = __float_as_int(lb.z);
     if (kind != RTNW_PRIM_SPHERE) {
         const float a = la.x + u1 * (la.y - la.x), b = la.z + u2 * (la.w - la.z);
@@ -1303,6 +1302,11 @@ __device__ __forceinline__ bool sample_light(const float4* __restrict__ lights, 
     const f3 u = cross(w, v);
     d = (cosf(phi) * s) * u + (sinf(phi) * s) * v + z * w;
     return true;
+}
+// the same with the next two draws of the path's stream
+__device__ __forceinline__ bool sample_light(const float4* __restrict__ lights, int k, f3 p, rng_t& g, f3& d) {
+    const float u1 = g.draw(), u2 = g.draw();
+    return sample_light(lights, k, p, u1, u2, d);
 }
 // material_scatter with the one-sample light mixture for lambertian and isotropic bounces (n_lights > 0, RTNW_F_EMIT on)
 __device__ __forceinline__ bool mixture_scatter(const scene_view& S, const float4* __restrict__ lights, int n_lights, int mat,
@@ -1334,6 +1338,29 @@ __device__ __forceinline__ bool mixture_scatter(const scene_view& S, const float
     const float w = p_ref / (0.5f * p_ref + 0.5f * (sum / (float)n_lights));
     attenuation = w * attenuation;
     return true;
+}
+
+// ------------------------------------------------------------------------------------------------ next-event estimation
+// RTNW_F_NEXT_EVENT (include/rtnw.h), restated operation for operation by tests/nee_oracle.c.
+// p_ref(e) of a lambertian (normal n) or isotropic vertex for the unit direction e
+__device__ __forceinline__ float ref_density(bool lambertian, f3 n, f3 e) {
+    if (!lambertian) return 0.0795774715f;  // 1 / (4 pi)
+    const float c = dot(e, n);
+    return c > 0.f ? c * c * c * 0.636619772f : 0.f;  // (2 / pi) cos^3
+}
+// p_L(e): the mean of the lights' densities, summed in table order
+__device__ __forceinline__ float lights_density(const float4* __restrict__ lights, int n_lights, f3 p, f3 e) {
+    float sum = 0.f;
+#pragma unroll 1
+    for (int k = 0; k < n_lights; ++k) sum += light_pdf(lights, k, p, e);
+    return sum / (float)n_lights;
+}
+// is record rec one of the light table's (n_lights <= RTNW_MAX_LIGHTS)
+__device__ __forceinline__ bool is_light_record(const float4* __restrict__ lights, int n_lights, int rec) {
+#pragma unroll 1
+    for (int k = 0; k < n_lights; ++k)
+        if (__float_as_int(__ldg(&lights[2 * k + 1]).w) == rec) return true;
+    return false;
 }
 
 // ------------------------------------------------------------------------------------------------ camera

@@ -1,6 +1,6 @@
 // rtnw_main — the reference's main() (PSC/main.cpp:244-336) with the triple sample loop replaced by the GPU library.
 //
-//   rtnw_main [scene] [nx ny ns] [out.ppm] [--binary] [--seed N] [--device D] [--gpus N] [--fast] [--lights] [--aov PREFIX]
+//   rtnw_main [scene] [nx ny ns] [out.ppm] [--binary] [--seed N] [--device D] [--gpus N] [--fast] [--lights] [--nee] [--aov PREFIX]
 //             [--denoise OUT.ppm]
 //   rtnw_main --selftest-bridge          exercises world->hit / scatter / emitted / value through the reference API
 //
@@ -12,6 +12,7 @@
 // --denoise OUT.ppm also writes the frame denoised from those buffers (rtnw_denoise with RTNW_DENOISE_DEFAULTS) with the same
 // epilogue as the main output; with --aov, PREFIX_denoised.pfm holds the denoised mean colour.  Both need one GPU.
 // --lights renders with RTNW_F_LIGHT_SAMPLING: the same expected image with less noise in scenes lit by small area lights.
+// --nee renders with RTNW_F_NEXT_EVENT: the same expected image, with a shadow ray to the lights at every diffuse vertex.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -64,7 +65,7 @@ static int selftest_bridge() {
 
 int main(int argc, char** argv) {
     std::string scene = "final", out = "Test.ppm", aov, denoise;  // PSC/main.cpp:291,295
-    int nx = 0, ny = 0, ns = 0, binary = 0, device = 0, gpus = 1, fast = 0, lights = 0;
+    int nx = 0, ny = 0, ns = 0, binary = 0, device = 0, gpus = 1, fast = 0, lights = 0, nee = 0;
     unsigned long long seed = 1;
     std::vector<std::string> pos;
     for (int i = 1; i < argc; ++i) {
@@ -76,6 +77,7 @@ int main(int argc, char** argv) {
         else if (a == "--gpus" && i + 1 < argc) gpus = std::atoi(argv[++i]);  // devices device .. device+gpus-1 (rtnw_render_multi)
         else if (a == "--fast") fast = 1;                                       // RTNW_F_FAST_BVH
         else if (a == "--lights") lights = 1;                                   // RTNW_F_LIGHT_SAMPLING
+        else if (a == "--nee") nee = 1;                                         // RTNW_F_NEXT_EVENT
         else if (a == "--aov" && i + 1 < argc) aov = argv[++i];
         else if (a == "--denoise" && i + 1 < argc) denoise = argv[++i];
         else pos.push_back(a);
@@ -102,7 +104,8 @@ int main(int argc, char** argv) {
     rtnw_render_params p;
     std::memset(&p, 0, sizeof p);
     p.nx = nx; p.ny = ny; p.sample_begin = 0; p.sample_count = ns; p.sample_stride = 1; p.max_depth = 50;
-    p.t_min = view.t_min; p.t_max = MAXFLOAT; p.background = view.background; p.flags = view.flags | (fast ? RTNW_F_FAST_BVH : 0u) | (lights ? RTNW_F_LIGHT_SAMPLING : 0u);
+    p.t_min = view.t_min; p.t_max = MAXFLOAT; p.background = view.background; p.flags = view.flags | (fast ? RTNW_F_FAST_BVH : 0u) | (lights ? RTNW_F_LIGHT_SAMPLING : 0u)
+              | (nee ? RTNW_F_NEXT_EVENT : 0u);
     p.seed = seed;
     const size_t npix = (size_t)nx * ny;
     std::vector<float> accum(npix * 3);

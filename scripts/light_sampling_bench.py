@@ -1,17 +1,18 @@
 #!/usr/bin/env python
-"""What RTNW_F_LIGHT_SAMPLING buys on the scenes lit by one small area light: BASELINE configs 3 (cornell_box), 4 (cornell_smoke)
-and 5N (final_northstar), each at its stated size and spp N, on one GPU.
+"""What RTNW_F_LIGHT_SAMPLING and RTNW_F_NEXT_EVENT buy on the scenes lit by one small area light: BASELINE configs 3
+(cornell_box), 4 (cornell_smoke) and 5N (final_northstar), each at its stated size and spp N, on one GPU.  --modes picks the
+estimators from exact (no flag), lights (RTNW_F_LIGHT_SAMPLING) and nee (RTNW_F_NEXT_EVENT); exact is always measured.
 
 Per config:
-  speed     rtnw_render with and without the flag, alternating, after a warm-up of each; Mpaths/s from the kernel time (CUDA
-            events, rtnw_stats.kernel_ms), medians over --reps.
+  speed     rtnw_render in each mode, alternating, after a warm-up of each; Mpaths/s from the kernel time (CUDA events,
+            rtnw_stats.kernel_ms), and closest-hit queries (rtnw_stats.rays) per path, medians over --reps.
   error     RMSE of the per-pixel mean colour against a converged image: the mean of --conv exact-mode frames of N spp each
             (other seeds), i.e. --conv times N spp.  Measured for both modes at N and at N/4 spp, averaged over --seeds frames;
             the exponent of RMSE ~ spp^-e between the two spp values checks the 1/sqrt(spp) scaling the ratio below assumes.
             The converged image still has 1/conv of the exact mode's variance at N: it is included in every RMSE.
-  ratio     equal-error time ratio: the time the exact mode needs to reach the flagged mode's RMSE at N spp,
-            N (rmse_exact / rmse_flag)^2 spp at the exact mode's rate, over the flagged mode's time for N spp.  > 1 means the flag
-            reaches that error sooner.
+  ratio     equal-error time ratio of each flagged mode: the time the exact mode needs to reach the flagged mode's RMSE at N
+            spp, N (rmse_exact / rmse_flag)^2 spp at the exact mode's rate, over the flagged mode's time for N spp.  > 1 means the
+            flag reaches that error sooner.
 Prints one JSON object, with the device name and power limit read in the same run, and writes it to --out when given."""
 import argparse
 import importlib
@@ -33,6 +34,7 @@ ap.add_argument("--configs", default="3,4,5N")
 ap.add_argument("--reps", type=int, default=5)
 ap.add_argument("--seeds", type=int, default=3)
 ap.add_argument("--conv", type=int, default=16)
+ap.add_argument("--modes", default="exact,lights")
 ap.add_argument("--out")
 a = ap.parse_args()
 
@@ -51,14 +53,17 @@ for cfg in a.configs.split(","):
         sums, st = ds.render(cam, hs.params(nx=nx, ny=ny, ns=spp, seed=seed, flags_extra=flags))
         return sums.astype(np.float64) / spp, st
 
-    modes = {"exact": 0, "lights": rtnw.F_LIGHT_SAMPLING}
+    flags = {"exact": 0, "lights": rtnw.F_LIGHT_SAMPLING, "nee": rtnw.F_NEXT_EVENT}
+    modes = {k: flags[k] for k in ["exact"] + [m for m in a.modes.split(",") if m != "exact"]}
     for f in modes.values():
         render(ns, 1, f)  # warm-up
     rate = {k: [] for k in modes}
+    rays = {k: [] for k in modes}
     for r in range(a.reps):
         for k, f in modes.items():
             st = render(ns, 10 + r, f)[1]
             rate[k].append(st.paths / st.kernel_ms / 1e3)
+            rays[k].append(st.rays / st.paths)
     conv = sum(render(ns, 5000 + r, 0)[0] for r in range(a.conv)) / a.conv
     rmse = {}
     for k, f in modes.items():
@@ -67,10 +72,15 @@ for cfg in a.configs.split(","):
             rmse[f"{k}_{spp}"] = float(np.sqrt(np.mean(mse)))
     mp = {k: statistics.median(v) for k, v in rate.items()}
     exponent = {k: float(np.log(rmse[f"{k}_{ns // 4}"] / rmse[f"{k}_{ns}"]) / np.log(4.0)) for k in modes}
-    spp_eq = ns * (rmse[f"exact_{ns}"] / rmse[f"lights_{ns}"]) ** 2
-    ratio = (spp_eq / mp["exact"]) / (ns / mp["lights"])
+    flagged = [k for k in modes if k != "exact"]
+    spp_eq = {k: ns * (rmse[f"exact_{ns}"] / rmse[f"{k}_{ns}"]) ** 2 for k in flagged}
+    ratio = {k: (spp_eq[k] / mp["exact"]) / (ns / mp[k]) for k in flagged}
+    if flagged == ["lights"]:  # the layout of the light-sampling run
+        spp_eq, ratio = spp_eq["lights"], ratio["lights"]
     result["configs"][cfg] = dict(workload=f"{name} {nx}x{ny}, {ns} spp", mpaths_per_s_median=mp, mpaths_per_s=rate, rmse=rmse,
                                   rmse_spp_exponent=exponent, exact_spp_for_equal_rmse=spp_eq, equal_error_time_ratio=ratio)
+    if "nee" in modes:
+        result["configs"][cfg]["rays_per_path_median"] = {k: statistics.median(v) for k, v in rays.items()}
     print(json.dumps({cfg: result["configs"][cfg]}), flush=True)
     ds.close()
     hs.close()
